@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- one PPBO iteration (GP Laplace fit + RFF acquisition over the xi-grids of every query direction).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config ackley20d] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config ackley20d] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one full iteration on synthetic inputs of the named BASELINE.json shape (default: Ackley-20D, 200 queries x
@@ -54,7 +54,12 @@ def parse_args():
     ap.add_argument("--samples", type=int, default=None, help="override S (debug)")
     ap.add_argument("--profile", default=None, choices=[None, "cold", "steady"],
                     help="1 warm-up + --steps resident steps of the named kind, no JSON (for ncu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed resident step returned as DIR/<name>.npy (float64), to compare two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------- clocks
@@ -385,6 +390,34 @@ def parity_gate(prob, gp, rff, sums_full, S, iteration, ops, torch):
     return gate
 
 
+# ------------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_MATRIX_BYTES = 16 << 20        # per matrix: the outputs stay far below 64 MB in all
+DUMP_SEED = 0
+
+
+def dump_outputs(dirname, sums, gp, rff):
+    """What run_iteration returned to its caller, as DIR/<name>.npy in float64: the per-direction sums, the GP mode and
+    alpha, the weight-space mode and its Hessian diagonal in full; of Sigma [N x N] and Phi_X [F x N] a fixed seeded sample of
+    rows (the row numbers in <name>_index.npy).  The inputs and the sample depend only on the arguments, so two builds run
+    with the same arguments can be compared file for file."""
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {"sums": sums}
+    if gp is not None:
+        arrays.update(f_map=gp.f_map, alpha=gp.alpha, Sigma_rows=gp.Sigma)
+    if rff is not None:
+        arrays.update(omega_map=rff.omega_map, hess_diag=rff.hess_diag, Phi_X_rows=rff.Phi_X)
+    for name, t in arrays.items():
+        if t is None:
+            continue
+        a = t.detach().cpu().numpy().astype(np.float64)
+        if name.endswith("_rows"):
+            k = min(a.shape[0], max(1, DUMP_MATRIX_BYTES // (8 * a.shape[1])))
+            idx = np.sort(np.random.RandomState(DUMP_SEED).choice(a.shape[0], k, replace=False))
+            a = a[idx]
+            np.save(os.path.join(dirname, name + "_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------- src/ API leg (configs 1-3)
 def api_leg(torch):
     """BASELINE configs 1-3 through the reference's own API (ppbo_numerical_main.py:102-124): update_feedback_processing_object ->
@@ -617,6 +650,8 @@ def main():
         held[0] = step(resident)           # (a warm-up that drops its products at once leaves the second timed step to
                                            # cudaMalloc a second set of 200 MB buffers: +1 ms on one GPU, up to +10 ms on two)
     ms_dev, launches, out = timed_run(resident)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *out)
     fit_stats = out[1].lap.stats if out[1] is not None else None
     rff_iters = out[2].stats["iterations"] if (out[2] is not None and out[2].stats) else None
     for _ in range(2):
