@@ -139,6 +139,10 @@ int ppbo_evidence_matrix(const double* Sigma, long long lds, int Q, int m, const
 /* C[M x N] = alpha * A[M x K] . B[N x K]^T + beta * C   (row-major, K contiguous in A and B) */
 int ppbo_gemm_nt(const double* A, long long lda, const double* B, long long ldb, double* C, long long ldc,
                  int M, int N, int K, double alpha, double beta, void* stream);
+/* lower tiles of C = alpha A B^T + beta C for a square C[N x N], in the tile configuration of ppbo_gemm_nt (same bits below the
+ * diagonal); tiles above the diagonal are not written */
+int ppbo_gemm_nt_lower(const double* A, long long lda, const double* B, long long ldb, double* C, long long ldc, int N, int K,
+                       double alpha, double beta, void* stream);
 /* tuning entry: ppbo_gemm_nt with an explicit tile configuration index (scripts/ubench_ops.py) */
 int ppbo_gemm_nt_cfg(int cfg, const double* A, long long lda, const double* B, long long ldb, double* C, long long ldc,
                      int M, int N, int K, double alpha, double beta, void* stream);
@@ -175,6 +179,8 @@ long long ppbo_lu_workspace_bytes(int n);
 int ppbo_lu_logdet(double* A, long long lda, int n, void* workspace, long long workspace_bytes, double* result_h, void* stream);
 /* y = A x for row-major A[M x N] */
 int ppbo_gemv(const double* A, long long lda, int M, int N, const double* x, double* y, void* stream);
+/* y = A x for a symmetric A[n x n], reading only its lower triangle; the bits do not depend on the launch grid */
+int ppbo_symv_lower(const double* A, long long lda, int n, const double* x, double* y, void* stream);
 
 /* ---- K4: prediction and exact-GP acquisition ----------------------------------------------------- */
 long long ppbo_predict_workspace_bytes(int N, int Q, int m, int P, int batch);

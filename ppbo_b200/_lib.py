@@ -47,6 +47,7 @@ _SIGNATURES = {
     "ppbo_factor_extend": (_I, [_P, _L, _I, _I, _P, _P, _I, _D, _P, _I, _P]),
     "ppbo_gemm_nt": (_I, [_P, _L, _P, _L, _P, _L, _I, _I, _I, _D, _D, _P]),
     "ppbo_gemm_nt_cfg": (_I, [_I, _P, _L, _P, _L, _P, _L, _I, _I, _I, _D, _D, _P]),
+    "ppbo_gemm_nt_lower": (_I, [_P, _L, _P, _L, _P, _L, _I, _I, _D, _D, _P]),
     "ppbo_potrf_workspace_bytes": (_L, [_I]),
     "ppbo_potrf_lower": (_I, [_P, _L, _I, _P, _L, _PI, _P]),
     "ppbo_trsm_right_lower": (_I, [_P, _L, _I, _P, _L, _I, _I, _P, _L, _P]),
@@ -60,6 +61,7 @@ _SIGNATURES = {
     "ppbo_lu_workspace_bytes": (_L, [_I]),
     "ppbo_lu_logdet": (_I, [_P, _L, _I, _P, _L, _PD, _P]),
     "ppbo_gemv": (_I, [_P, _L, _I, _I, _P, _P, _P]),
+    "ppbo_symv_lower": (_I, [_P, _L, _I, _P, _P, _P]),
     "ppbo_neg_count": (_I, [_P, _I, _PI, _I, _P]),
     "ppbo_neg_corr_doubles": (_L, [_I, _I]),
     "ppbo_neg_corr_build": (_I, [_P, _L, _I, _P, _P, _I, _PI, _I, _P, _P]),

@@ -987,7 +987,7 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
         PPBO_CL rff_psi_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, M);
         {
             GemmOperands g{ws.PsiT, M, 0, ws.PsiT, M, 0, F, F, M};
-            StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 0, 0, 0};
+            StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 2, 0, 0};        // lower tiles only: the factorisation reads no more
             if ((rc = launch_gemm_nt(g, ep, 1, st))) return rc;
         }
         PPBO_CL add_identity_kernel<<<ceil_div(F, 256), 256, 0, st>>>(ws.H, F, F);
@@ -1065,7 +1065,7 @@ extern "C" int ppbo_rff_refactor(const double* Phi_X, long long ld, int F, int Q
     if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega, ws, nullptr, nullptr, true, ws.scal + 24, st))) return rc;
     PPBO_CL rff_psi_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, M);
     GemmOperands g{ws.PsiT, M, 0, ws.PsiT, M, 0, F, F, M};
-    StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 0, 0, 0};
+    StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 2, 0, 0};                // lower tiles only, as in ppbo_rff_fit
     if ((rc = launch_gemm_nt(g, ep, 1, st))) return rc;
     PPBO_CL add_identity_kernel<<<ceil_div(F, 256), 256, 0, st>>>(ws.H, F, F);
     PPBO_LAUNCH_CHECK();

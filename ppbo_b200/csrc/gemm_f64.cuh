@@ -124,7 +124,8 @@ __device__ __forceinline__ void gemm_mainloop(const GemmOperands& g, const doubl
 struct StoreEpilogue {
     double* C; long long ldc; long long strideC;
     double alpha, beta;
-    int lower_only;      // 1: blockIdx.x enumerates tiles (ti >= tj) of a square tiling (BM == BN)
+    int lower_only;      // 1: blockIdx.x enumerates tiles (ti >= tj) of a square tiling (BM == BN); 2: the same in the tile
+                         //    configuration the full product would use (its lower tiles bit-identical to the full product's)
     int vec_ok;          // 1: C rows are 16-byte aligned at even columns (set by the launcher)
     int in_place;        // 1: C aliases A (row-panel update); launcher picks a tile with BN >= N == K
     long long strideC2 = 0;   // outer batch stride (GemmOperands::zinner)

@@ -966,12 +966,13 @@ struct FitWorkspace {
     double *bvec, *sa, *ap, *t, *Sb, *dalpha, *df, *set_part, *scal, *arrow_tmp, *binv, *state, *hist;
     double *bR, *bT, *bC, *bw;           // bordered warm start: R [BORDER_MAX x M], scratch T [BORDER_MAX x M], C [BORDER_MAX^2], w
     double *aaH, *aa, *part0;            // Anderson history [(3 AA_M + 3) x N], its state [8], likelihood sums at the current iterate [Q]
+    double* sym;                         // partials of the symmetric mat-vecs with Sigma (N) and G (M < N): symv_scratch_doubles(N)
     int* info;
     static long long doubles(int Q, int m) {
         const long long N = (long long)Q * (m + 1), M = (long long)Q * m;
         return 4 * N + 3 * M + (M + CHOL_NB) + (long long)NSTEP * Q + 32 + 8 + 64 + CHORD_STATE + 2 * CHORD_BATCH_MAX +
                blockinv_doubles((int)M) + 2LL * BORDER_MAX * (M + 2) + (long long)BORDER_MAX * BORDER_MAX + BORDER_MAX + 8 +
-               (3LL * AA_M + 3) * N + AA_STATE + Q;
+               (3LL * AA_M + 3) * N + AA_STATE + Q + symv_scratch_doubles((int)N);
     }
     void carve(double* base, int Q, int m) {
         const long long N = (long long)Q * (m + 1), M = (long long)Q * m;
@@ -998,7 +999,8 @@ struct FitWorkspace {
         bw = p; p += BORDER_MAX;
         aaH = p; p += (3LL * AA_M + 3) * N;
         aa = p; p += AA_STATE;
-        part0 = p;
+        part0 = p; p += Q;
+        sym = p;
     }
 };
 
@@ -1271,7 +1273,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
         if (!in_diff) return PPBO_OK;
         in_diff = false;
         PPBO_CL from_diff_kernel<<<set_blocks, 256, 0, st>>>(ws.bvec, Q, m, alpha);          // alpha = B gamma
-        return gemv(Sigma, lds, N, N, alpha, f_map, st);                                       // f = Sigma alpha
+        return symv_lower(Sigma, lds, N, alpha, f_map, ws.sym, st);                            // f = Sigma alpha
     };
     while (it < max_iter && !converged) {
         if (!refactor) {
@@ -1311,7 +1313,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
                     if (bordered)
                         PPBO_CL dborder_coeff_kernel<<<ceil_div(nb, 64), 64, 0, st>>>(dv + M_old, nb, sigma, m, ws.sa + M_old, ws.ap + M_old, skip);
                     PPBO_CL dchord_rhs_kernel<<<ceil_div(M, 256), 256, 0, st>>>(dv, ws.ap, M, sigma, m, cv, skip);
-                    if ((rc = gemv(G, ldg, M, M, cv, ws.t, st, skip))) return rc;
+                    if ((rc = symv_lower(G, ldg, M, cv, ws.t, ws.sym, st, skip))) return rc;
                     PPBO_CL dchord_scale_kernel<<<ceil_div(M, 256), 256, 0, st>>>(ws.t, ws.sa, M, skip);
                     if ((rc = chord_solve(skip))) return rc;
                     PPBO_CL dchord_update_kernel<<<ceil_div(M, 256), 256, 0, st>>>(cv, ws.sa, ws.ap, ws.t, gam, dv, M, thr, dgam, ddv, skip);
@@ -1325,11 +1327,11 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
             for (int i = 0; i < kb; ++i) {
                 if (bordered) refresh_border(skip);
                 PPBO_CL lik_terms_kernel<<<set_blocks, 256, 0, st>>>(f_map, Q, m, sigma, nullptr, nullptr, nullptr, nullptr, ws.bvec, ws.ap, nullptr, skip);
-                if ((rc = gemv(Sigma, lds, N, N, ws.bvec, ws.Sb, st, skip))) return rc;
+                if ((rc = symv_lower(Sigma, lds, N, ws.bvec, ws.Sb, ws.sym, st, skip))) return rc;
                 PPBO_CL diff_scale_kernel<<<ceil_div(M, 256), 256, 0, st>>>(ws.Sb, ws.sa, Q, m, ws.t, skip);
                 if ((rc = chord_solve(skip))) return rc;
                 PPBO_CL alpha_update_kernel<<<set_blocks, 256, 0, st>>>(ws.bvec, ws.sa, ws.t, alpha, Q, m, ws.dalpha, skip);
-                if ((rc = gemv(Sigma, lds, N, N, ws.dalpha, ws.df, st, skip))) return rc;
+                if ((rc = symv_lower(Sigma, lds, N, ws.dalpha, ws.df, ws.sym, st, skip))) return rc;
                 PPBO_CL chord_lik_kernel<<<set_blocks, 256, 0, st>>>(f_map, ws.df, Q, m, sigma, ws.state, ws.set_part, anderson ? ws.part0 : nullptr);
                 PPBO_CL chord_decide_kernel<<<1, 1024, 0, st>>>(alpha, ws.dalpha, f_map, ws.df, N, ws.set_part, Q, m, ws.state, ws.hist,
                                                                   (chord_extrapolate && !anderson) ? 1 : 0, anderson ? ws.part0 : nullptr);
@@ -1380,7 +1382,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
             PPBO_CUDA_CHECK(cudaMemsetAsync(ws.aa, 0, sizeof(double) * 8, st));
             rel3_h = INFINITY;
         }
-        if ((rc = gemv(Sigma, lds, N, N, ws.bvec, ws.Sb, st))) return rc;
+        if ((rc = symv_lower(Sigma, lds, N, ws.bvec, ws.Sb, ws.sym, st))) return rc;
         PPBO_CL diff_scale_kernel<<<ceil_div(M, 256), 256, 0, st>>>(ws.Sb, ws.sa, Q, m, ws.t);
         if (!identity_factor) {
             // From the second factorisation on -- and for the first one of a cold fit, which enters the Anderson-mixed chord phase
@@ -1394,7 +1396,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
             if (rc) return rc;
         }
         PPBO_CL alpha_update_kernel<<<set_blocks, 256, 0, st>>>(ws.bvec, ws.sa, ws.t, alpha, Q, m, ws.dalpha);
-        if ((rc = gemv(Sigma, lds, N, N, ws.dalpha, ws.df, st))) return rc;
+        if ((rc = symv_lower(Sigma, lds, N, ws.dalpha, ws.df, ws.sym, st))) return rc;
         PPBO_LAUNCH_CHECK();
         if (!alpha_known) {
             // arbitrary start: alpha_old is unknown (would need Sigma^-1 f); take the full Newton step, which

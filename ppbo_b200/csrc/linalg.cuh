@@ -25,5 +25,10 @@ int potrs_bwd_blockinv(const double* L, long long ldl, int n, double* W, double*
 int trsm_right_blockinv(const double* L, long long ldl, int n, const double* W, double* T, long long ldt, double* R, long long ldr,
                         int nrhs, cudaStream_t st);
 int gemv(const double* A, long long lda, int M, int N, const double* x, double* y, cudaStream_t st, const double* skip = nullptr);
+// y = A x for a symmetric n x n A of which only the lower triangle is read; part: symv_scratch_doubles(n) doubles.  The result
+// does not depend on the launch grid.
+long long symv_scratch_doubles(int n);
+int symv_lower(const double* A, long long lda, int n, const double* x, double* y, double* part, cudaStream_t st,
+               const double* skip = nullptr);
 
 }  // namespace ppbo

@@ -46,11 +46,12 @@ CONCURRENT_FITS = True
 # OVERLAP_RESERVED_SMS(_COLD) SMs to the fit (tuning key 14); a contraction CTA fills its SM, so the two never share one.
 # PPBO_OVERLAP_SAMPLING=0 restores the sequential order (diagnostics).
 import os as _os
-# Reserved SMs: an appended iteration's GP chain is short (it ends ~2 ms before the contraction on 16 SMs); a cold fit has 13
-# chord steps with two 216 MB mat-vecs each and is the longer chain, so it gets more (sweeps in DESIGN.md 5.1).
+# Reserved SMs: an appended iteration's GP chain is short (it still ends before the contraction on 8 SMs); a cold fit has 13
+# chord steps with one 100 MB half-triangle mat-vec of G each plus the factorisation and is the longer chain, so it gets more
+# (sweeps in DESIGN.md 5.1).
 _RESERVE_ENV = _os.environ.get("PPBO_OVERLAP_RESERVE")
-OVERLAP_RESERVED_SMS = int(_RESERVE_ENV) if _RESERVE_ENV else 16            # appended iterations
-OVERLAP_RESERVED_SMS_COLD = int(_RESERVE_ENV) if _RESERVE_ENV else 32       # cold iterations
+OVERLAP_RESERVED_SMS = int(_RESERVE_ENV) if _RESERVE_ENV else 12            # appended iterations
+OVERLAP_RESERVED_SMS_COLD = int(_RESERVE_ENV) if _RESERVE_ENV else 24       # cold iterations
 # Steady state of the overlapped pipeline, opt-in: refresh the weight-space Hessian factor at each new optimum while the contraction
 # runs (RFFState.refresh_factor).  The next fit then needs 10 chord steps and never a mid-fit refactorisation (13 steps and a
 # refactorisation every ~4th iteration with the stale factor), but the refresh (10 GFLOP of Hessian GEMM + a Cholesky) shares

@@ -268,6 +268,14 @@ def gemm_nt(A, B, C=None, alpha=1.0, beta=0.0):
     return C
 
 
+def gemm_nt_lower(A, B, C, alpha=1.0, beta=0.0):
+    """lower tiles of C = alpha A B^T + beta C (square C); the lower triangle has the bits of gemm_nt"""
+    N, K = A.shape
+    check(_lib.load().ppbo_gemm_nt_lower(_p(A), A.stride(0), _p(B), B.stride(0), _p(C), C.stride(0), N, K, float(alpha),
+                                         float(beta), _stream()), "ppbo_gemm_nt_lower")
+    return C
+
+
 def gemm_nt_cfg(cfg, A, B, C, alpha=1.0, beta=0.0):
     M, K = A.shape
     N = B.shape[0]
@@ -369,6 +377,14 @@ def shrink_inplace(K, shrinkage):
 def gemv(A, x, out=None):
     y = torch.empty(A.shape[0], dtype=F64, device=A.device) if out is None else out
     check(_lib.load().ppbo_gemv(_p(A), A.stride(0), A.shape[0], A.shape[1], _p(x), _p(y), _stream()), "ppbo_gemv")
+    return y
+
+
+def symv_lower(A, x, out=None):
+    """y = A x for a symmetric A, reading only its lower triangle"""
+    n = A.shape[0]
+    y = torch.empty(n, dtype=F64, device=A.device) if out is None else out
+    check(_lib.load().ppbo_symv_lower(_p(A), A.stride(0), n, _p(x), _p(y), _stream()), "ppbo_symv_lower")
     return y
 
 
