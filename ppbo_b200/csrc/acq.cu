@@ -283,12 +283,14 @@ __global__ void rff_maximize_select_kernel(const double* __restrict__ xall, cons
 }
 
 // y[i] = sum_f Phi[f][i] omega[f]   (feature-major Phi: coalesced over i).  HBM-bound (8 F N bytes): the feature range is cut
-// into FV_SLICES slices so that ~8 x N/128 CTAs stream concurrently; slice partials are combined in a fixed order.
+// into FV_SLICES slices so that ~8 x N/128 CTAs stream concurrently; slice partials are combined in a fixed order by the last CTA
+// of each column block to finish (count[blockIdx.x] counts the finished slices and is back at 0 when the kernel ends).
 constexpr int FV_SLICES = 8, FV_COLS = 128;
-__global__ void __launch_bounds__(256) rff_fvals_partial_kernel(const double* __restrict__ Phi, long long ld, int F, int N,
-                                                                const double* __restrict__ omega, double* __restrict__ part,
-                                                                const double* __restrict__ skip) {
+__global__ void __launch_bounds__(256) rff_fvals_kernel(const double* __restrict__ Phi, long long ld, int F, int N,
+                                                        const double* __restrict__ omega, double* part, double* __restrict__ y,
+                                                        unsigned* __restrict__ count, const double* __restrict__ skip) {
     __shared__ double red[FV_COLS];
+    __shared__ bool last;
     if (skip && *skip != 0.0) return;          // queued chord step behind the one that stopped the batch (see ppbo_rff_fit)
     const int c = threadIdx.x & (FV_COLS - 1), half = threadIdx.x >> 7;          // 128 columns x 2 row phases
     const int i = blockIdx.x * FV_COLS + c;
@@ -306,20 +308,25 @@ __global__ void __launch_bounds__(256) rff_fvals_partial_kernel(const double* __
     if (half == 1) red[c] = s0 + s1;
     __syncthreads();
     if (half == 0 && i < N) part[(long long)blockIdx.y * N + i] = (s0 + s1) + red[c];
-}
-__global__ void __launch_bounds__(256) rff_fvals_combine_kernel(const double* __restrict__ part, int N, double* __restrict__ y) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= N) return;
-    double s = 0.0;
+    __threadfence();                           // this slice's partials are visible before it is counted
+    __syncthreads();
+    if (threadIdx.x == 0) last = atomicAdd(count + blockIdx.x, 1u) == FV_SLICES - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    if (half == 0 && i < N) {
+        double s = 0.0;
 #pragma unroll
-    for (int k = 0; k < FV_SLICES; ++k) s += part[(long long)k * N + i];
-    y[i] = s;
+        for (int k = 0; k < FV_SLICES; ++k) s += __ldcg(part + (long long)k * N + i);
+        y[i] = s;
+    }
+    if (threadIdx.x == 0) count[blockIdx.x] = 0u;
 }
-// part: FV_SLICES * N doubles of scratch
+// part: FV_SLICES * N doubles of scratch; count: fvals_count_words(N) zeroed words (left zeroed)
+static int fvals_count_words(int N) { return ceil_div(N, FV_COLS); }
 static int launch_rff_fvals(const double* Phi, long long ld, int F, int N, const double* omega, double* part, double* y,
-                            cudaStream_t st, const double* skip = nullptr) {
-    PPBO_CL rff_fvals_partial_kernel<<<dim3(ceil_div(N, FV_COLS), FV_SLICES), 256, 0, st>>>(Phi, ld, F, N, omega, part, skip);
-    PPBO_CL rff_fvals_combine_kernel<<<ceil_div(N, 256), 256, 0, st>>>(part, N, y);
+                            unsigned* count, cudaStream_t st, const double* skip = nullptr) {
+    PPBO_CL rff_fvals_kernel<<<dim3(ceil_div(N, FV_COLS), FV_SLICES), 256, 0, st>>>(Phi, ld, F, N, omega, part, y, count, skip);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
 }
@@ -435,9 +442,11 @@ int launch_linesearch_lik(const double* f, const double* df, int Q, int m, doubl
 constexpr int LS_STEPS = 8;      // == NSTEP of laplace.cu: step sizes 1, 1/2, ..., 2^-7
 
 // scal[0..2] = omega.omega, omega.step, step.step ; scal[3] = max|step| ; scal[4] = max|omega| ; scal[8 + c] = sum_q part[c][q]
-__global__ void __launch_bounds__(1024) rff_ls_scalars_kernel(const double* __restrict__ omega, const double* __restrict__ step,
-                                                              int F, const double* __restrict__ part, int Q,
-                                                              double* __restrict__ scal) {
+// (1024 threads)
+// (rff_chord_tail_kernel writes omega and scal later on: no __restrict__ on them, so that no read goes through the non-coherent
+// read-only path)
+__device__ __forceinline__ void rff_ls_scalars(const double* omega, const double* __restrict__ step, int F,
+                                               const double* __restrict__ part, int Q, double* scal) {
     __shared__ double red_multi[32 * (3 + LS_STEPS)];
     __shared__ double mx[2][32];
     double m0 = 0, m1 = 0;
@@ -469,6 +478,11 @@ __global__ void __launch_bounds__(1024) rff_ls_scalars_kernel(const double* __re
         for (int c = 0; c < LS_STEPS; ++c) scal[8 + c] = sums[3 + c];
     }
 }
+__global__ void __launch_bounds__(1024) rff_ls_scalars_kernel(const double* __restrict__ omega, const double* __restrict__ step,
+                                                              int F, const double* __restrict__ part, int Q,
+                                                              double* __restrict__ scal) {
+    rff_ls_scalars(omega, step, F, part, Q, scal);
+}
 
 // Device-side acceptance test of one weight-space chord step (same scheme as chord_decide_kernel of laplace.cu): the full step is
 // taken when S does not fall, convergence and contraction are tested here, and the host synchronises once per batch.
@@ -480,11 +494,10 @@ __global__ void __launch_bounds__(1024) rff_ls_scalars_kernel(const double* __re
 // the current iterate is recomputed every step (the iterate may have been mixed since the last accepted step).
 // anderson: the steps of this batch are mixed (rff_anderson_kernel); mixed steps are not monotone step by step, so the contraction
 // is judged over three steps (a chord step costs ~1/10 of a refactorisation: three steps must gain a factor 5).
-__global__ void __launch_bounds__(256) rff_chord_decide_kernel(double* __restrict__ omega, const double* __restrict__ step, int F,
-                                                               const double* __restrict__ scal, int m, double* __restrict__ state,
-                                                               double* __restrict__ hist, int anderson) {
+// Returns whether the step was taken (the same value in every thread).
+__device__ __forceinline__ bool rff_chord_decide(double* omega, const double* __restrict__ step, int F, const double* scal, int m,
+                                                 double* state, double* hist, int anderson) {
     __shared__ int accept_s;
-    if (state[4] != 0.0) return;
     if (threadIdx.x == 0) {
         const double oo = scal[0], od = scal[1], dd = scal[2], max_step = scal[3], max_om = fmax(scal[4], 1e-300);
         const double S_cur = -0.5 * oo - scal[24] / m;
@@ -510,22 +523,23 @@ __global__ void __launch_bounds__(256) rff_chord_decide_kernel(double* __restric
         }
     }
     __syncthreads();
-    if (!accept_s) return;
+    if (!accept_s) return false;
     for (int i = threadIdx.x; i < F; i += blockDim.x) omega[i] += step[i];
+    return true;
 }
 
 // Anderson acceleration of the weight-space chord iteration omega <- g(omega) = omega + (-H0)^-1 grad S(omega) (depth RAA_M; same
 // scheme as chord_anderson_kernel of laplace.cu).  With the clamped Hessian the iteration matrix differs from the true Hessian by the
 // negative curvature coefficients, so even a factor built next to the optimum contracts only linearly (0.3 .. 0.45 per step on the
 // bench problem, 0.55 for the factor of the previous PPBO iteration); mixing the last residual differences gains about
-// rho / (1 + sqrt(1 - rho^2)) per step instead.  Called after rff_chord_decide_kernel has taken a full step: omega = g(omega_k),
-// residual r_k = step still in memory.  The history is dropped when a step was rejected or the residual grew.  One CTA, fixed order.
+// rho / (1 + sqrt(1 - rho^2)) per step instead.  Called after rff_chord_decide has taken a full step: omega = g(omega_k),
+// residual r_k = step still in memory.  The history is dropped when a step was rejected or the residual grew.  One CTA of 1024
+// threads, fixed order.
 //   aa: [0] history length, [1] next slot, [2] residual norm seen by the previous call, [3] 1 = (prev r, prev g) valid
 //   Hh: [2 RAA_M + 2][F]: dR[RAA_M], dG[RAA_M], prev r, prev g
 constexpr int RAA_M = 5;
-__global__ void __launch_bounds__(1024) rff_anderson_kernel(double* __restrict__ omega, const double* __restrict__ step, int F,
-                                                            const double* __restrict__ state, double* __restrict__ aa,
-                                                            double* __restrict__ Hh) {
+__device__ __forceinline__ void rff_anderson(double* omega, const double* __restrict__ step, int F, const double* state, double* aa,
+                                             double* Hh) {
     __shared__ double gam[RAA_M];
     __shared__ int nh_s;
     if (state[4] != 0.0) return;                                         // converged, rejected or about to refactor: nothing to mix
@@ -626,6 +640,26 @@ __global__ void __launch_bounds__(1024) rff_anderson_kernel(double* __restrict__
         for (int j = 0; j < nm; ++j) c = fma(gam[j], dG[(long long)j * F + i], c);
         omega[i] -= c;
     }
+}
+
+// End of one weight-space chord step in one CTA: the likelihood sum at the current iterate (scal[24], the reduction of sum_kernel),
+// the line-search scalars, the acceptance test and the Anderson mixing, each with the reductions of its former kernel.  What one
+// part writes the next reads after a barrier, through plain (coherent) loads: only step, setlik and part are read-only here.
+__global__ void __launch_bounds__(1024) rff_chord_tail_kernel(double* omega, const double* __restrict__ step, int F,
+                                                              const double* __restrict__ setlik, const double* __restrict__ part,
+                                                              int Q, int m, double* scal, double* state, double* hist, int anderson,
+                                                              double* aa, double* Hh) {
+    __shared__ double red[33];
+    if (state[4] != 0.0) return;               // queued step behind the one that stopped the batch
+    double s = 0.0;
+    for (int i = threadIdx.x; i < Q; i += 1024) s += setlik[i];
+    s = block_sum(s, red);
+    if (threadIdx.x == 0) scal[24] = s;
+    rff_ls_scalars(omega, step, F, part, Q, scal);
+    __syncthreads();
+    if (!rff_chord_decide(omega, step, F, scal, m, state, hist, anderson) || !anderson) return;
+    __syncthreads();
+    rff_anderson(omega, step, F, state, aa, Hh);
 }
 
 }  // namespace ppbo
@@ -830,12 +864,14 @@ extern "C" int ppbo_rff_maximize(const double* W, const double* b, int F, int D,
 
 extern "C" long long ppbo_rff_workspace_bytes(int F, int Q, int m) {
     const long long N = (long long)Q * (m + 1), M = (long long)Q * m;
-    return ((3 + FV_SLICES) * N + 2 * M + Q * 9 + 64 + (long long)F * M + ppbo_factor_doubles(F) + 4 * (long long)F + 2 * CHOL_NB +
-            blockinv_doubles(F) + (2LL * RAA_M + 2) * F + 8) * 8;
+    return ((3 + FV_SLICES) * N + 2 * M + Q * 9 + 64 + (long long)F * M + ppbo_factor_doubles(F) + 3 * (long long)F + 2 * CHOL_NB +
+            blockinv_doubles(F) + (2LL * RAA_M + 2) * F + 8 + (fvals_count_words((int)N) + 1) / 2) * 8;
 }
 
 struct RffWs {
-    double *fvals, *dfv, *fpart, *beta, *arrow, *setlik, *scal, *PsiT, *H, *grad, *step, *trial, *tmp, *binv, *aaH, *aa;
+    double *fvals, *dfv, *fpart, *beta, *arrow, *setlik, *scal, *PsiT, *H, *step, *trial, *tmp, *binv, *aaH, *aa;
+    unsigned* fv_count;        // slice counters of rff_fvals_kernel: zero them once per call (zero_counters)
+    int nfv_count;
     void carve(double* p, int F, int Q, int m) {
         const long long N = (long long)Q * (m + 1), M = (long long)Q * m;
         fvals = p; p += N;
@@ -847,22 +883,25 @@ struct RffWs {
         scal = p; p += 64;
         PsiT = p; p += (long long)F * M;
         H = p; p += ppbo_factor_doubles(F);
-        grad = p; p += F;
         step = p; p += F + CHOL_NB;
         trial = p; p += F;
         tmp = p; p += F;
         aaH = p; p += (2LL * RAA_M + 2) * F;
         aa = p; p += 8;
-        binv = p;
+        binv = p; p += blockinv_doubles(F);
+        fv_count = reinterpret_cast<unsigned*>(p);
+        nfv_count = fvals_count_words((int)N);
     }
+    cudaError_t zero_counters(cudaStream_t st) { return cudaMemsetAsync(fv_count, 0, sizeof(unsigned) * nfv_count, st); }
 };
 
+// lik_sum_dev == nullptr: the likelihood sum is left to the caller (the chord steps take it in rff_chord_tail_kernel)
 static int rff_eval(const double* Phi, long long ld, int F, int Q, int m, double sigma, const double* omega, RffWs& ws,
                     double* grad, double* hdiag, bool want_arrow, double* lik_sum_dev, cudaStream_t st, const double* skip = nullptr) {
     const int N = Q * (m + 1);
-    launch_rff_fvals(Phi, ld, F, N, omega, ws.fpart, ws.fvals, st, skip);
+    launch_rff_fvals(Phi, ld, F, N, omega, ws.fpart, ws.fvals, ws.fv_count, st, skip);
     launch_lik_terms(ws.fvals, Q, m, sigma, ws.setlik, ws.beta, want_arrow ? ws.arrow : nullptr, nullptr, nullptr, st);
-    launch_sum(ws.setlik, Q, lik_sum_dev, st);
+    if (lik_sum_dev) launch_sum(ws.setlik, Q, lik_sum_dev, st);
     if (grad && !hdiag)
         PPBO_CL rff_grad_kernel<<<ceil_div(F, 2), 256, 0, st>>>(Phi, ld, F, N, omega, ws.beta, grad, skip);
     else if (grad || hdiag)
@@ -879,6 +918,7 @@ extern "C" int ppbo_rff_objective(const double* Phi_X, long long ld, int F, int 
     cudaStream_t st = (cudaStream_t)stream;
     RffWs ws;
     ws.carve((double*)workspace, F, Q, m);
+    PPBO_CUDA_CHECK(ws.zero_counters(st));
     int rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega, ws, grad, hess_diag, true, ws.scal + 8, st);
     if (rc) return rc;
     if (S_out) {
@@ -912,6 +952,7 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
     double* Hdinv = ws.H + (long long)F * F;
     int* info_d = reinterpret_cast<int*>(ws.scal + 32);
     PPBO_CUDA_CHECK(cudaMemsetAsync(info_d, 0, sizeof(int), st));       // (a warm fit may never factorise)
+    PPBO_CUDA_CHECK(ws.zero_counters(st));
     if (omega0) PPBO_CUDA_CHECK(cudaMemcpyAsync(omega_map, omega0, sizeof(double) * F, cudaMemcpyDeviceToDevice, st));
     else PPBO_CUDA_CHECK(cudaMemsetAsync(omega_map, 0, sizeof(double) * F, st));
     int rc, it = 0, info = 0, n_factor = 0, n_chord = 0;
@@ -949,15 +990,13 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
             double state_h[8] = {S_cur, last_rel, prev_rel_h, rel3_h, 0.0, 0.0, tol, 0.0}, hist_h[2 * RFF_BATCH_MAX];
             PPBO_CUDA_CHECK(cudaMemcpyAsync(state_d, state_h, sizeof(state_h), cudaMemcpyHostToDevice, st));
             const double* skip = state_d + 4;
-            for (int i = 0; i < kb; ++i) {
-                if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega_map, ws, ws.grad, nullptr, false, ws.scal + 24, st, skip))) return rc;
-                PPBO_CUDA_CHECK(cudaMemcpyAsync(ws.step, ws.grad, sizeof(double) * F, cudaMemcpyDeviceToDevice, st));
+            for (int i = 0; i < kb; ++i) {     // the gradient goes straight into the step vector, which the solve overwrites
+                if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega_map, ws, ws.step, nullptr, false, nullptr, st, skip))) return rc;
                 if ((rc = potrs_vec_blockinv(ws.H, F, F, ws.binv, ws.step, st, skip))) return rc;
-                launch_rff_fvals(Phi_X, ld, F, N, ws.step, ws.fpart, ws.dfv, st, skip);
+                launch_rff_fvals(Phi_X, ld, F, N, ws.step, ws.fpart, ws.dfv, ws.fv_count, st, skip);
                 if ((rc = launch_linesearch_lik(ws.fvals, ws.dfv, Q, m, sigma, part, st))) return rc;
-                PPBO_CL rff_ls_scalars_kernel<<<1, 1024, 0, st>>>(omega_map, ws.step, F, part, Q, ws.scal);
-                PPBO_CL rff_chord_decide_kernel<<<1, 256, 0, st>>>(omega_map, ws.step, F, ws.scal, m, state_d, hist_d, anderson ? 1 : 0);
-                if (anderson) PPBO_CL rff_anderson_kernel<<<1, 1024, 0, st>>>(omega_map, ws.step, F, state_d, ws.aa, ws.aaH);
+                PPBO_CL rff_chord_tail_kernel<<<1, 1024, 0, st>>>(omega_map, ws.step, F, ws.setlik, part, Q, m, ws.scal, state_d, hist_d,
+                                                                 anderson ? 1 : 0, ws.aa, ws.aaH);
             }
             PPBO_LAUNCH_CHECK();
             PPBO_CUDA_CHECK(readback().add(state_h, state_d, sizeof(state_h), st));
@@ -982,25 +1021,30 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
             continue;
         }
         // ---- Newton step: gradient and clamped Hessian at omega, fresh factor (chord steps with a kept factor all go through the
-        // batches above)
-        if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega_map, ws, ws.grad, nullptr, true, ws.scal + 24, st))) return rc;
-        PPBO_CL rff_psi_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, M);
-        {
-            GemmOperands g{ws.PsiT, M, 0, ws.PsiT, M, 0, F, F, M};
-            StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 2, 0, 0};        // lower tiles only: the factorisation reads no more
-            if ((rc = launch_gemm_nt(g, ep, 1, st))) return rc;
+        // batches above).  A null omega0 starts at omega = 0: every difference is 0, so a+ = 0 and the Hessian I + Psi' a+ Psi is
+        // the identity.  That first step is the gradient itself (the same bits the solve with the factor of I gives), and nothing is
+        // factorised: the factor in ws.H stays invalid and the next step factorises.
+        const bool identity_step = it == 0 && omega0 == nullptr;
+        // the gradient goes straight into the step vector, which the solve overwrites
+        if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega_map, ws, ws.step, nullptr, !identity_step, ws.scal + 24, st))) return rc;
+        if (!identity_step) {
+            PPBO_CL rff_psi_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, M);
+            {
+                GemmOperands g{ws.PsiT, M, 0, ws.PsiT, M, 0, F, F, M};
+                StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 2, 0, 0};        // lower tiles only: the factorisation reads no more
+                if ((rc = launch_gemm_nt(g, ep, 1, st))) return rc;
+            }
+            PPBO_CL add_identity_kernel<<<ceil_div(F, 256), 256, 0, st>>>(ws.H, F, F);
+            if ((rc = potrf_lower(ws.H, F, F, Hdinv, info_d, st))) return rc;
+            ++n_factor;
+            binv_valid = false;
+            PPBO_CUDA_CHECK(cudaMemsetAsync(ws.aa, 0, sizeof(double) * 8, st));     // new iteration matrix: forget the mixing history
+            rel3_h = INFINITY;
+            // step = (-Hessian)^-1 grad  (ascent direction)
+            if ((rc = potrs_vec(ws.H, F, F, Hdinv, ws.step, st))) return rc;
         }
-        PPBO_CL add_identity_kernel<<<ceil_div(F, 256), 256, 0, st>>>(ws.H, F, F);
-        if ((rc = potrf_lower(ws.H, F, F, Hdinv, info_d, st))) return rc;
-        ++n_factor;
-        binv_valid = false;
-        PPBO_CUDA_CHECK(cudaMemsetAsync(ws.aa, 0, sizeof(double) * 8, st));     // new iteration matrix: forget the mixing history
-        rel3_h = INFINITY;
-        PPBO_CUDA_CHECK(cudaMemcpyAsync(ws.step, ws.grad, sizeof(double) * F, cudaMemcpyDeviceToDevice, st));
-        // step = (-Hessian)^-1 grad  (ascent direction)
-        if ((rc = potrs_vec(ws.H, F, F, Hdinv, ws.step, st))) return rc;
         // line search, all LS_STEPS step sizes in one pass: f(omega + s step) = f0 + s df, |omega + s step|^2 in closed form
-        launch_rff_fvals(Phi_X, ld, F, N, ws.step, ws.fpart, ws.dfv, st);
+        launch_rff_fvals(Phi_X, ld, F, N, ws.step, ws.fpart, ws.dfv, ws.fv_count, st);
         if ((rc = launch_linesearch_lik(ws.fvals, ws.dfv, Q, m, sigma, part, st))) return rc;
         PPBO_CL rff_ls_scalars_kernel<<<1, 1024, 0, st>>>(omega_map, ws.step, F, part, Q, ws.scal);
         PPBO_LAUNCH_CHECK();
@@ -1025,7 +1069,7 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
         last_rel = s * max_step / max_om;
         if (trace) fprintf(stderr, "[ppbo_rff_fit] it %d newton step %.3g rel %.3e S %.12g\n", it, s, last_rel, S_cur);
         if (c == 0 && last_rel <= tol) { ++it; break; }
-        refactor = !(c == 0 && last_rel <= CHORD_REL);       // chord steps once a full Newton step is in the contraction region
+        refactor = identity_step || !(c == 0 && last_rel <= CHORD_REL);   // chord steps once a full Newton step is in the contraction region
     }
     if (std::isnan(S_cur)) {                             // last step left S unevaluated: evaluate at the final point
         if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega_map, ws, nullptr, nullptr, false, ws.scal + 24, st))) return rc;
@@ -1061,6 +1105,7 @@ extern "C" int ppbo_rff_refactor(const double* Phi_X, long long ld, int F, int Q
     ws.binv = factor_cache + ppbo_factor_doubles(F);
     double* Hdinv = ws.H + (long long)F * F;
     int* info_d = reinterpret_cast<int*>(ws.scal + 32);
+    PPBO_CUDA_CHECK(ws.zero_counters(st));
     int rc;
     if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega, ws, nullptr, nullptr, true, ws.scal + 24, st))) return rc;
     PPBO_CL rff_psi_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, M);
