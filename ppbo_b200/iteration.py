@@ -53,8 +53,8 @@ _RESERVE_ENV = _os.environ.get("PPBO_OVERLAP_RESERVE")
 OVERLAP_RESERVED_SMS = int(_RESERVE_ENV) if _RESERVE_ENV else 12            # appended iterations
 OVERLAP_RESERVED_SMS_COLD = int(_RESERVE_ENV) if _RESERVE_ENV else 24       # cold iterations
 # Steady state of the overlapped pipeline, opt-in: refresh the weight-space Hessian factor at each new optimum while the contraction
-# runs (RFFState.refresh_factor).  The next fit then needs 10 chord steps and never a mid-fit refactorisation (13 steps and a
-# refactorisation every ~4th iteration with the stale factor), but the refresh (10 GFLOP of Hessian GEMM + a Cholesky) shares
+# runs (RFFState.refresh_factor).  The next fit then needs 10 chord steps and never a mid-fit refactorisation (7-13 steps and a
+# refactorisation in 6 of 13 iterations with the stale factor, tests/test_steady_state.py), but the refresh (10 GFLOP of Hessian GEMM + a Cholesky) shares
 # the reserved SMs with the GP chain, which then ends AFTER the contraction: 14.05 ms per appended iteration against 13.09 without
 # (measured), so it is off.
 REFRESH_RFF_FACTOR = _os.environ.get("PPBO_RFF_REFRESH", "0") != "0"
