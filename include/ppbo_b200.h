@@ -21,6 +21,8 @@ extern "C" {
 #define PPBO_KERNEL_RQ 1       /* src/kernels.py:27-34 (alpha = 2)                                     */
 #define PPBO_KERNEL_CAMPHOR 2  /* src/kernels.py:36-53                                                 */
 #define PPBO_KERNEL_SQDIST 3   /* internal: squared Euclidean distance (ppbo_sqdist)                   */
+#define PPBO_KERNEL_MATERN32 4 /* sf^2 (1 + sqrt3 r) exp(-sqrt3 r), r = |(x - y) / l| (ARD as for SE)   */
+#define PPBO_KERNEL_MATERN52 5 /* sf^2 (1 + sqrt5 r + 5 r^2 / 3) exp(-sqrt5 r)                          */
 
 int ppbo_version(void);
 const char* ppbo_last_error(void);

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libppbo_b200.so")
 
 FIT_G_READY, FIT_FACTOR_WARM, FIT_FACTOR_AT_MODE = 1, 2, 4
-KERNEL_KINDS = {"SE_kernel": 0, "RQ_kernel": 1, "camphor_copper_kernel": 2}
+KERNEL_KINDS = {"SE_kernel": 0, "RQ_kernel": 1, "camphor_copper_kernel": 2, "Matern32_kernel": 4, "Matern52_kernel": 5}
 
 
 class PPBOError(RuntimeError):

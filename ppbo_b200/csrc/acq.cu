@@ -724,7 +724,8 @@ extern "C" long long ppbo_predict_workspace_bytes(int N, int Q, int m, int P, in
 /* workspace of a mean-only call (Sigma_p == NULL): the tensor-pipe kernels never materialise the cross-covariance */
 extern "C" long long ppbo_predict_mean_workspace_bytes(int kind, int N, int P, int batch) {
     const long long PT = (long long)P * batch;
-    if (kind == PPBO_KERNEL_SE || kind == PPBO_KERNEL_RQ) return (PT * ((N + 63) / 64) + 64) * 8;
+    if (kind == PPBO_KERNEL_SE || kind == PPBO_KERNEL_RQ || kind == PPBO_KERNEL_MATERN32 || kind == PPBO_KERNEL_MATERN52)
+        return (PT * ((N + 63) / 64) + 64) * 8;
     return (PT * N + 64) * 8;
 }
 

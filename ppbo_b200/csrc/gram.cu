@@ -25,10 +25,12 @@ struct KernelParams {
 constexpr int KT_M = 64, KT_N = 128, KT_THREADS = 256;
 
 __device__ __forceinline__ double kernel_from_sums(int kind, double r2, double sf2) {
-    // r2: scaled squared distance (SE / RQ) or the summed exponent (camphor)
+    // r2: scaled squared distance (SE / RQ / Matern) or the summed exponent (camphor)
     if (kind == PPBO_KERNEL_SE) return sf2 * exp(-0.5 * r2);
     if (kind == PPBO_KERNEL_RQ) { const double t = 1.0 + 0.25 * r2; return sf2 / (t * t); }   // alpha = 2
     if (kind == PPBO_KERNEL_SQDIST) return r2;                                                // kernels.dist: the distance itself
+    if (kind == PPBO_KERNEL_MATERN32) { const double a = sqrt(3.0 * r2); return sf2 * (1.0 + a) * exp(-a); }
+    if (kind == PPBO_KERNEL_MATERN52) { const double a = sqrt(5.0 * r2); return sf2 * (1.0 + a + 5.0 * r2 / 3.0) * exp(-a); }
     return sf2 * exp(-r2);
 }
 
@@ -106,7 +108,7 @@ __global__ void __launch_bounds__(KT_THREADS) kernel_matrix_kernel(const double*
 }
 
 
-// SE / RQ kernels: register-tiled version.  Thread tile 8 rows x 4 columns; the 4 column points' coordinates are cached in
+// SE / RQ / Matern kernels: register-tiled version.  Thread tile 8 rows x 4 columns; the 4 column points' coordinates are cached in
 // registers 4 dimensions at a time, the row coordinates arrive as warp-broadcast shared-memory loads, so the inner loop
 // issues 0.31 shared loads per FMA (the plain version above issues 1.0 and is LDS-bound at D = 20).  Stores: 32 B per thread,
 // 1 KB contiguous per warp and row.
@@ -182,7 +184,7 @@ __global__ void __launch_bounds__(KT_THREADS, 2) kernel_matrix_tiled_kernel(cons
     }
 }
 
-// ---- SE / RQ kernels on the FP64 tensor pipe ------------------------------------------------------------------------------
+// ---- SE / RQ / Matern kernels on the FP64 tensor pipe -----------------------------------------------------------------------
 // The scaled squared distance is formed the way the reference's kernels.dist does (src/kernels.py:3-11),
 //   r2 = |x|^2 + |y|^2 - 2 x.y   clipped at 0,
 // with the cross term as a DMMA product (D FMAs per pair instead of the 2 D of the difference form, 0.03 shared-memory loads per
@@ -215,7 +217,7 @@ __host__ __device__ inline int km_ldx(int D) { const int Dp = (D + 3) / 4 * 4; r
 // Coefficients live in constant memory and enter the FMAs as constant-bank operands: FP64 literals have no immediate form, and
 // under the 64-register budget of this kernel the compiler otherwise re-materialises every coefficient with two moves per use
 // (253 IMAD.MOV next to 256 DFMA per 16 entries in the first version).  Horner form: one constant per FMA.
-__constant__ double KM_EXP[20] = {
+__constant__ double KM_EXP[23] = {
     1.4426950408889634,          // [0] log2(e)
     6755399441055744.0,          // [1] 2^52 + 2^51
     -6.93147180369123816490e-01, // [2] -ln2 (high part)
@@ -223,16 +225,12 @@ __constant__ double KM_EXP[20] = {
     1.0, 1.0, 0.5, 1.6666666666666666e-01, 4.1666666666666664e-02, 8.3333333333333332e-03, 1.3888888888888889e-03,      // [4..] 1/k!
     1.9841269841269841e-04, 2.4801587301587302e-05, 2.7557319223985893e-06, 2.7557319223985888e-07, 2.5052108385441720e-08,
     2.0876756987868100e-09, 1.6059043836821613e-10,
-    -708.0, -0.25};
-// SE entry from v = |x|^2 + |y|^2 - 2 x.y (may be slightly negative by cancellation):  sf2' exp(-max(v, 0) / 2), straight-line.
-//   w = v + |v| = 2 max(v, 0) exactly (|.| is an operand modifier), its high word clamped at that of 2832 (exp(-708) = 3e-308: the
-//   result stays a normal number whatever the inputs; one integer min instead of the ~8 instructions of a NaN-aware fmax);
-//   x = -w / 4 = n ln2 + r with |r| <= ln2 / 2 (rint by the 2^52 + 2^51 trick, ln2 in two pieces); exp(r) by its degree-13 Taylor
-//   polynomial in Horner form (truncation 4e-18); 2^n by an integer add to the exponent field.  23 FP64 + 2 integer instructions.
-__device__ __forceinline__ double se_entry(double v, double scale_c) {
-    double w = v + fabs(v);
-    w = __hiloint2double(min(__double2hiint(w), 0x40A62000), __double2loint(w));          // high word of 2832.0
-    const double x = w * KM_EXP[19];
+    -708.0, -0.25,
+    1.5, 2.5, 3.3333333333333331e-01};                                                                                // [20..22] Matern
+// exp(x) for x in [-708, 0] (a little beyond -708 is fine: 2^n stays normal down to x = -708.39), straight-line:
+//   x = n ln2 + r with |r| <= ln2 / 2 (rint by the 2^52 + 2^51 trick, ln2 in two pieces); exp(r) by its degree-13 Taylor polynomial
+//   in Horner form (truncation 4e-18); 2^n by an integer add to the exponent field.  17 FP64 + 2 integer instructions.
+__device__ __forceinline__ double km_exp(double x) {
     const double t = fma(x, KM_EXP[0], KM_EXP[1]);
     const int n = __double2loint(t);
     const double nf = t - KM_EXP[1];
@@ -241,11 +239,36 @@ __device__ __forceinline__ double se_entry(double v, double scale_c) {
     double pv = KM_EXP[17];
 #pragma unroll
     for (int k = 16; k >= 4; --k) pv = fma(pv, r, KM_EXP[k]);
-    return scale_c * __hiloint2double(__double2hiint(pv) + (n << 20), __double2loint(pv));
+    return __hiloint2double(__double2hiint(pv) + (n << 20), __double2loint(pv));
+}
+// SE entry from v = |x|^2 + |y|^2 - 2 x.y (may be slightly negative by cancellation):  sf2' exp(-max(v, 0) / 2), straight-line.
+//   w = v + |v| = 2 max(v, 0) exactly (|.| is an operand modifier), its high word clamped at that of 2832 (exp(-708) = 3e-308: the
+//   result stays a normal number whatever the inputs; one integer min instead of the ~8 instructions of a NaN-aware fmax);
+//   then exp(-w / 4) by km_exp.  23 FP64 + 2 integer instructions.
+__device__ __forceinline__ double se_entry(double v, double scale_c) {
+    double w = v + fabs(v);
+    w = __hiloint2double(min(__double2hiint(w), 0x40A62000), __double2loint(w));          // high word of 2832.0
+    return scale_c * km_exp(w * KM_EXP[19]);
+}
+// Matern-nu entry (nu = 3/2, 5/2) from the same v, straight-line.  With a = sqrt(2 nu) r (r^2 = max(v, 0)):
+//   q = nu (v + |v|) = a^2, its high word clamped to [that of 2^-1000, that of 708^2]: rsqrt_nr needs a normal operand, and
+//   a <= 708 (+3e-7 relative: the low word is kept) keeps exp(-a) normal as in se_entry.  At v <= 0 the entry is sf2' exactly
+//   (a = 2^-500 rounds away).  a = q rsqrt_nr(q) (one MUFU + 9 FP64); e = sf2' exp(-a) by km_exp;
+//   nu = 3/2: (1 + a) e,  nu = 5/2: (1 + a + a^2 / 3) e, the prefactor folded into the last FMA(s).  The coefficients (nu, 1/3)
+//   are constant-bank operands like the exp's.
+template <int KIND>
+__device__ __forceinline__ double matern_entry(double v, double scale_c) {
+    double q = (v + fabs(v)) * KM_EXP[KIND == PPBO_KERNEL_MATERN32 ? 20 : 21];
+    q = __hiloint2double(max(min(__double2hiint(q), 0x411E9840), 0x01700000), __double2loint(q));     // [2^-1000, 708^2]
+    const double a = q * rsqrt_nr(q);
+    const double pf = (KIND == PPBO_KERNEL_MATERN32) ? a : fma(q, KM_EXP[22], a);                        // prefactor - 1
+    const double e = scale_c * km_exp(-a);
+    return fma(pf, e, e);
 }
 template <int KIND>
 __device__ __forceinline__ double km_entry(double v, double scale_c, double sf2, double diag_scale) {
     if (KIND == PPBO_KERNEL_SE) return se_entry(v, scale_c);
+    if (KIND == PPBO_KERNEL_MATERN32 || KIND == PPBO_KERNEL_MATERN52) return matern_entry<KIND>(v, scale_c);
     return diag_scale * kernel_from_sums(KIND, fmax(v, 0.0), sf2);
 }
 
@@ -490,8 +513,24 @@ static int launch_kernel_matrix_mma(const KernelParams& p, const double* X1, int
     return PPBO_OK;
 }
 
+static bool km_has_mma(int kind) {
+    return kind == PPBO_KERNEL_SE || kind == PPBO_KERNEL_RQ || kind == PPBO_KERNEL_MATERN32 || kind == PPBO_KERNEL_MATERN52;
+}
+static int launch_kernel_matrix_mma_kind(const KernelParams& p, const double* X1, int n1, const double* X2, int n2, double* out,
+                                         long long ld, int mode, const double* alpha, cudaStream_t st, int* groups_out = nullptr) {
+    switch (p.kind) {
+        case PPBO_KERNEL_SE: return launch_kernel_matrix_mma<PPBO_KERNEL_SE>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
+        case PPBO_KERNEL_RQ: return launch_kernel_matrix_mma<PPBO_KERNEL_RQ>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
+        case PPBO_KERNEL_MATERN32:
+            return launch_kernel_matrix_mma<PPBO_KERNEL_MATERN32>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
+        case PPBO_KERNEL_MATERN52:
+            return launch_kernel_matrix_mma<PPBO_KERNEL_MATERN52>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
+    }
+    PPBO_REQUIRE(false, "kernel kind has no tensor-pipe version");
+}
+
 static int fill_params(KernelParams& p, int kind, int D, const double* ls_h, double sigma_f) {
-    PPBO_REQUIRE(kind >= 0 && kind <= 3, "unknown kernel kind");
+    PPBO_REQUIRE(kind >= 0 && kind <= PPBO_KERNEL_MATERN52, "unknown kernel kind");
     PPBO_REQUIRE(D >= 1 && D <= PPBO_MAX_D, "D must be in [1, 64]");
     PPBO_REQUIRE(kind != PPBO_KERNEL_CAMPHOR || D == 6, "camphor_copper_kernel is defined for D = 6 only");
     PPBO_REQUIRE(ls_h != nullptr && sigma_f > 0, "hyper-parameters");
@@ -523,6 +562,8 @@ int kernel_matrix(const KernelParams& p, const double* X1, int n1, const double*
         PPBO_CUDA_CHECK(cudaFuncSetAttribute(kernel_matrix_tiled_kernel<PPBO_KERNEL_SE>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
         PPBO_CUDA_CHECK(cudaFuncSetAttribute(kernel_matrix_tiled_kernel<PPBO_KERNEL_RQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
         PPBO_CUDA_CHECK(cudaFuncSetAttribute(kernel_matrix_tiled_kernel<PPBO_KERNEL_SQDIST>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+        PPBO_CUDA_CHECK(cudaFuncSetAttribute(kernel_matrix_tiled_kernel<PPBO_KERNEL_MATERN32>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+        PPBO_CUDA_CHECK(cudaFuncSetAttribute(kernel_matrix_tiled_kernel<PPBO_KERNEL_MATERN52>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
         attr_done = true;
     }
     if (p.kind == PPBO_KERNEL_SQDIST) {         // squared distances: difference form (no cancellation), no tensor-pipe variant
@@ -532,13 +573,12 @@ int kernel_matrix(const KernelParams& p, const double* X1, int n1, const double*
         PPBO_LAUNCH_CHECK();
         return PPBO_OK;
     }
-    if (g_tuning[11] == 0 && (p.kind == PPBO_KERNEL_SE || p.kind == PPBO_KERNEL_RQ)) {     // tuning key 11 = 1: difference-form kernels
+    if (g_tuning[11] == 0 && km_has_mma(p.kind)) {     // tuning key 11 = 1: difference-form kernels
         const int mode = (symmetric_diag && X1 == X2 && n1 == n2) ? KM_SYMMETRIC : KM_STORE;
         KernelParams q = p;
         if (mode != KM_SYMMETRIC) q.diag_add = 0.0;
         if (symmetric_diag && mode != KM_SYMMETRIC) goto general;       // diagonal term on a non-aliased pair: keep the old path
-        return p.kind == PPBO_KERNEL_SE ? launch_kernel_matrix_mma<PPBO_KERNEL_SE>(q, X1, n1, X2, n2, out, ld, mode, nullptr, st)
-                                        : launch_kernel_matrix_mma<PPBO_KERNEL_RQ>(q, X1, n1, X2, n2, out, ld, mode, nullptr, st);
+        return launch_kernel_matrix_mma_kind(q, X1, n1, X2, n2, out, ld, mode, nullptr, st);
     }
 general:
     const int Dp = (p.D + KR_DC - 1) / KR_DC * KR_DC;
@@ -550,8 +590,17 @@ general:
         case PPBO_KERNEL_RQ:
             PPBO_CL kernel_matrix_tiled_kernel<PPBO_KERNEL_RQ><<<grid, KT_THREADS, smem_t, st>>>(X1, n1, X2, n2, p, out, ld, symmetric_diag);
             break;
-        default:
+        case PPBO_KERNEL_MATERN32:
+            PPBO_CL kernel_matrix_tiled_kernel<PPBO_KERNEL_MATERN32><<<grid, KT_THREADS, smem_t, st>>>(X1, n1, X2, n2, p, out, ld, symmetric_diag);
+            break;
+        case PPBO_KERNEL_MATERN52:
+            PPBO_CL kernel_matrix_tiled_kernel<PPBO_KERNEL_MATERN52><<<grid, KT_THREADS, smem_t, st>>>(X1, n1, X2, n2, p, out, ld, symmetric_diag);
+            break;
+        case PPBO_KERNEL_CAMPHOR:
             PPBO_CL kernel_matrix_kernel<PPBO_KERNEL_CAMPHOR><<<grid, KT_THREADS, smem, st>>>(X1, n1, X2, n2, p, out, ld, symmetric_diag);
+            break;
+        default:
+            PPBO_REQUIRE(false, "unknown kernel kind");
     }
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
@@ -572,14 +621,13 @@ int kernel_matrix_raw(int kind, const double* X1, int n1, const double* X2, int 
 // partial: n1 * ceil(n2 / 64) doubles of scratch.  Returns 1 when done, 0 when the kernel kind has no tensor-pipe version.
 int kernel_matvec(int kind, const double* X1, int n1, const double* X2, int n2, int D, const double* ls_h, double sigma_f,
                   const double* alpha, double* mu, double* partial, cudaStream_t st) {
-    if (g_tuning[11] != 0 || !(kind == PPBO_KERNEL_SE || kind == PPBO_KERNEL_RQ)) return 0;
+    if (g_tuning[11] != 0 || !km_has_mma(kind)) return 0;
     KernelParams p;
     int rc = fill_params(p, kind, D, ls_h, sigma_f);
     if (rc) return rc;
     if (n1 <= 0) return 1;
     int G = 1;
-    rc = kind == PPBO_KERNEL_SE ? launch_kernel_matrix_mma<PPBO_KERNEL_SE>(p, X1, n1, X2, n2, partial, 0, KM_MATVEC, alpha, st, &G)
-                                : launch_kernel_matrix_mma<PPBO_KERNEL_RQ>(p, X1, n1, X2, n2, partial, 0, KM_MATVEC, alpha, st, &G);
+    rc = launch_kernel_matrix_mma_kind(p, X1, n1, X2, n2, partial, 0, KM_MATVEC, alpha, st, &G);
     if (rc) return rc;
     PPBO_CL km_rowsum_kernel<<<ceil_div(n1, 256), 256, 0, st>>>(partial, n1, G, mu);
     PPBO_LAUNCH_CHECK();
@@ -843,7 +891,14 @@ extern "C" int ppbo_mu_pred_point(int kind, const double* X, int N, int D, const
     switch (kind) {
         case PPBO_KERNEL_SE: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_SE><<<1, 1024, 0, st>>>(X, N, p, alpha, g_point.dev, out); break;
         case PPBO_KERNEL_RQ: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_RQ><<<1, 1024, 0, st>>>(X, N, p, alpha, g_point.dev, out); break;
-        default: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_CAMPHOR><<<1, 1024, 0, st>>>(X, N, p, alpha, g_point.dev, out);
+        case PPBO_KERNEL_MATERN32:
+            PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_MATERN32><<<1, 1024, 0, st>>>(X, N, p, alpha, g_point.dev, out);
+            break;
+        case PPBO_KERNEL_MATERN52:
+            PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_MATERN52><<<1, 1024, 0, st>>>(X, N, p, alpha, g_point.dev, out);
+            break;
+        case PPBO_KERNEL_CAMPHOR: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_CAMPHOR><<<1, 1024, 0, st>>>(X, N, p, alpha, g_point.dev, out); break;
+        default: PPBO_REQUIRE(false, "kernel kind has no posterior-mean kernel");
     }
     PPBO_LAUNCH_CHECK();
     PPBO_CUDA_CHECK(cudaStreamSynchronize(st));
@@ -866,7 +921,14 @@ extern "C" int ppbo_mu_pred_points(int kind, const double* X, int N, int D, cons
     switch (kind) {
         case PPBO_KERNEL_SE: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_SE><<<B, 1024, 0, st>>>(X, N, p, alpha, g_batch.dev, out); break;
         case PPBO_KERNEL_RQ: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_RQ><<<B, 1024, 0, st>>>(X, N, p, alpha, g_batch.dev, out); break;
-        default: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_CAMPHOR><<<B, 1024, 0, st>>>(X, N, p, alpha, g_batch.dev, out);
+        case PPBO_KERNEL_MATERN32:
+            PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_MATERN32><<<B, 1024, 0, st>>>(X, N, p, alpha, g_batch.dev, out);
+            break;
+        case PPBO_KERNEL_MATERN52:
+            PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_MATERN52><<<B, 1024, 0, st>>>(X, N, p, alpha, g_batch.dev, out);
+            break;
+        case PPBO_KERNEL_CAMPHOR: PPBO_CL mu_pred_point_kernel<PPBO_KERNEL_CAMPHOR><<<B, 1024, 0, st>>>(X, N, p, alpha, g_batch.dev, out); break;
+        default: PPBO_REQUIRE(false, "kernel kind has no posterior-mean kernel");
     }
     PPBO_LAUNCH_CHECK();
     PPBO_CUDA_CHECK(cudaStreamSynchronize(st));

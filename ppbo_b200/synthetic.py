@@ -7,6 +7,8 @@ point first, then the m pseudo-observations alpha_k xi + x on a jittered equispa
 """
 import numpy as np
 
+from .spectral import draw_rff_basis
+
 # name: D, Q, m, kernel, theta=[sigma, l, sigma_f], S (MC samples), P (grid points per direction), F (RFF features)
 CONFIGS = {
     "camel2d": dict(D=2, Q=39, m=25, kernel="SE_kernel", theta=[0.01, 0.26, 0.1], S=150, P=70, F=1000),
@@ -59,10 +61,12 @@ def make_design(D, Q, m, seed=0, answer_noise=1e-3):
     return np.clip(X, 0, 1), log, centre
 
 
-def make_problem(name, seed=0, Q=None, S=None, P=None, F=None):
-    """All host inputs of one iteration for config `name` (sizes overridable for small parity cases)."""
+def make_problem(name, seed=0, Q=None, S=None, P=None, F=None, kernel=None):
+    """All host inputs of one iteration for config `name` (sizes overridable for small parity cases).  `kernel` overrides the
+    config's covariance function; the RFF basis is then drawn from that kernel's spectral density (draw_rff_basis).  The design,
+    the grids and, for the configs' own kernels, every draw are the same as without the override."""
     cfg = dict(CONFIGS[name])
-    for k, v in (("Q", Q), ("S", S), ("P", P), ("F", F)):
+    for k, v in (("Q", Q), ("S", S), ("P", P), ("F", F), ("kernel", kernel)):
         if v is not None:
             cfg[k] = v
     D, Qn, m = cfg["D"], cfg["Q"], cfg["m"]
@@ -78,7 +82,9 @@ def make_problem(name, seed=0, Q=None, S=None, P=None, F=None):
     alphas = np.stack([jittered_alphas(rng, cfg["P"]) for _ in range(D)])
     prob.update(xis=xis, xs=xs, alphas=alphas, grids=alphas[:, :, None] * xis[:, None, :] + xs[:, None, :])
     if cfg["F"]:
-        prob["W"] = rng.randn(cfg["F"], D) / cfg["theta"][1]            # src/random_fourier_sampler.py:42
-        prob["b"] = rng.uniform(0, 2 * np.pi, cfg["F"])                 # :43
+        W, b = draw_rff_basis(cfg["kernel"], cfg["F"], D, cfg["theta"][1], rng)       # src/random_fourier_sampler.py:42-43
+        if W is None:
+            raise ValueError("random Fourier basis exists for the SE and Matern kernels only, not %s (use F=0)" % cfg["kernel"])
+        prob["W"], prob["b"] = W, b
         prob["omega0"] = np.zeros(cfg["F"])
     return prob

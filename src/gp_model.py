@@ -23,12 +23,13 @@ if _ROOT not in sys.path:
     sys.path.insert(0, _ROOT)
 
 from feedback_processing import FeedbackProcessing  # noqa: E402
-from kernels import SE_kernel, RQ_kernel, camphor_copper_kernel  # noqa: E402,F401
+from kernels import SE_kernel, RQ_kernel, camphor_copper_kernel, Matern32_kernel, Matern52_kernel  # noqa: E402,F401
 from misc import pd_inverse, regularize_covariance, var2_normal_pdf  # noqa: E402,F401
 from ppbo_b200 import ops  # noqa: E402
 from ppbo_b200 import device_linalg as _dl  # noqa: E402
 
-_KERNELS = {"SE_kernel": SE_kernel, "RQ_kernel": RQ_kernel, "camphor_copper_kernel": camphor_copper_kernel}
+_KERNELS = {"SE_kernel": SE_kernel, "RQ_kernel": RQ_kernel, "camphor_copper_kernel": camphor_copper_kernel,
+            "Matern32_kernel": Matern32_kernel, "Matern52_kernel": Matern52_kernel}
 
 
 class _Lazy:

@@ -3,7 +3,8 @@ numpy arrays, theta = (sigma, l, sigma_f), returning a host float64 matrix.  The
 (ppbo_kernel_matrix, ppbo_b200/csrc/gram.cu); there is no CPU implementation behind these names.
 
 `theta[1]` may also be a length-D sequence of per-dimension length-scales (ARD) -- a strict generalisation of the
-reference, whose SE kernel is isotropic."""
+reference, whose SE kernel is isotropic.  The Matern kernels (nu = 3/2, 5/2, GPy's parametrisation) are additions beyond the
+reference, with the same theta and the same ARD rule."""
 import os
 import sys
 
@@ -54,3 +55,13 @@ def RQ_kernel(X1, X2, theta):
 def camphor_copper_kernel(X1, X2, theta):
     """period-1 periodic kernel on coordinates 0,1,3,4,5 times an SE kernel with l + 0.05 on coordinate 2 (src/kernels.py:36-53)"""
     return _evaluate("camphor_copper_kernel", X1, X2, theta)
+
+
+def Matern32_kernel(X1, X2, theta):
+    """sigma_f^2 (1 + sqrt(3) r) exp(-sqrt(3) r),  r = |(x - y) / l|   (Matern nu = 3/2; not in the reference)"""
+    return _evaluate("Matern32_kernel", X1, X2, theta)
+
+
+def Matern52_kernel(X1, X2, theta):
+    """sigma_f^2 (1 + sqrt(5) r + 5 r^2 / 3) exp(-sqrt(5) r),  r = |(x - y) / l|   (Matern nu = 5/2; not in the reference)"""
+    return _evaluate("Matern52_kernel", X1, X2, theta)

@@ -7,7 +7,7 @@ evaluated on B projected xi-grids as one dense contraction Omega[S x F] . Phi_gr
 max / arg-max, optionally sharded over the GPUs of a box.
 
 Random numbers: every draw comes from the global legacy numpy RNG on the host, in the reference's order (generate_basis:
-W then b; update_omega_MAP: omega0; sample_omega: F normals through numpy's SVD-factor rule, which for the diagonal Laplace
+W then b -- for the Matern kernels, an addition, W's normals, its chi-square draws, then b; update_omega_MAP: omega0; sample_omega: F normals through numpy's SVD-factor rule, which for the diagonal Laplace
 covariance is a permutation by decreasing variance).
 """
 import os
@@ -24,6 +24,7 @@ if _ROOT not in sys.path:
 from misc import pd_inverse, var2_normal_pdf  # noqa: E402,F401
 from ppbo_b200 import ops  # noqa: E402
 from ppbo_b200 import iteration as _it  # noqa: E402
+from ppbo_b200.spectral import draw_rff_basis  # noqa: E402
 
 
 class Hsampler:
@@ -51,9 +52,9 @@ class Hsampler:
 
     # ------------------------------------------------------------------ basis and feature maps (:38-58)
     def generate_basis(self):
-        if self.kernel == "SE_kernel":
-            self.W = np.random.randn(self.nFeatures, self.D) / self.theta[1]
-        self.b = np.random.uniform(low=0, high=2 * np.pi, size=self.nFeatures)[:, None]
+        # SE: the reference's draws; Matern: z, u, b (ppbo_b200/spectral.py); RQ / camphor: b only, no W
+        self.W, b = draw_rff_basis(self.kernel, self.nFeatures, self.D, self.theta[1], np.random)
+        self.b = b[:, None]
         self._dev.clear()
 
     def _d(self, name):
