@@ -300,6 +300,16 @@ int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int m, double 
  * at every one of its iterations, src/random_fourier_sampler.py:124-132.) */
 int ppbo_rff_refactor(const double* Phi_X, long long ld, int F, int Q, int m, double sigma, const double* omega,
                       double* factor_cache, void* workspace, long long workspace_bytes, void* stream);
+/* Full Laplace covariance of the weight-space posterior (opt-in; the reference's covariance is diagonal,
+ * src/random_fourier_sampler.py:134-137, and so is the default path above).  L[F x ldl] (followed by the inverted 128-blocks the
+ * solves read: ppbo_rff_hessian_factor_doubles(F, ldl) doubles in all) receives the Cholesky factor of the EXACT Hessian
+ * -grad^2 S(omega) = I + Psi' diag(a) Psi with the signed likelihood coefficients a at omega -- the precision of the Laplace
+ * approximation, whose diagonal is -hess_diag.  A caller buffer: the fit's factor_cache (clamped chord matrix) is not touched.
+ * info_h (host, may be NULL = no synchronisation): 0 or the first non-positive pivot, also the return value; no fall-back. */
+long long ppbo_rff_hessian_factor_workspace_bytes(int F, int Q, int m);
+long long ppbo_rff_hessian_factor_doubles(int F, long long ldl);
+int ppbo_rff_hessian_factor(const double* Phi_X, long long ld, int F, int Q, int m, double sigma, const double* omega, double* L,
+                            long long ldl, void* workspace, long long workspace_bytes, int* info_h, void* stream);
 /* out[i] = standard normal number (offset + i) of Philox4x32-10 stream `stream_id` under `seed` (Box-Muller on 53-bit uniforms).
  * Counter-based: the value of a given index does not depend on launch shape or on which GPU draws it.  Replaces the host
  * np.random draws of the reference where the caller does not inject its own (oracle: oracle/ppbo_oracle.py philox_normals). */
@@ -311,6 +321,14 @@ int ppbo_normal_fill(unsigned long long seed, unsigned int stream_id, long long 
 int ppbo_rff_sample_omega(const double* omega_map, const double* hess_diag, const double* Z, long long ldz,
                           unsigned long long seed, unsigned int stream_id, long long sample0, int S, int F, double* Omega,
                           long long ldo, void* stream);
+/* Omega = 1 omega_map' + Z L^-1: S draws from N(omega_map, H^-1) for the factor L of ppbo_rff_hessian_factor (the full-covariance
+ * Hsampler.sample_omega, src/random_fourier_sampler.py:207-213, numpy's multivariate_normal with the dense covariance).  Z as in
+ * ppbo_rff_sample_omega (injected, or Philox numbers (sample0 + s) F + f).  S <= 65535 per call.
+ * workspace: ppbo_rff_sample_omega_full_workspace_bytes(S, F) bytes. */
+long long ppbo_rff_sample_omega_full_workspace_bytes(int S, int F);
+int ppbo_rff_sample_omega_full(const double* omega_map, const double* L, long long ldl, const double* Z, long long ldz,
+                               unsigned long long seed, unsigned int stream_id, long long sample0, int S, int F, double* Omega,
+                               long long ldo, void* workspace, long long workspace_bytes, void* stream);
 /* Fs = Omega[S x F] . PhiT_grid[P x F]^T per batch entry (grid), fused per-sample max / first arg-max over P
  * (batched form of the objective in Hsampler.return_xstar, src/random_fourier_sampler.py:166,170).
  * Fs_full (optional, tests only): dense [batch][S x P]. */
@@ -339,6 +357,11 @@ int ppbo_ozaki_slice(const double* X, long long ldx, long long strideX, int rows
  * (Hsampler.sample_omega, src/random_fourier_sampler.py:207-213, batched over S samples.) */
 int ppbo_ozaki_sample_slice(const double* omega_map, const double* hess_diag, unsigned long long seed, unsigned int stream_id,
                             long long sample0, int S, int F, int slices, double* scale, signed char* planes, void* stream);
+/* The standard normals z[s][f] = Philox number (sample0 + s) F + f themselves as A-operand digit planes (no mean, no scale): the
+ * draws of the full-covariance contraction max_p (mu_p + z_s . Phi~_p), which do not depend on the fit.  Bit-identical to
+ * ppbo_normal_fill followed by ppbo_ozaki_slice. */
+int ppbo_ozaki_normal_slice(unsigned long long seed, unsigned int stream_id, long long sample0, int S, int F, int slices,
+                            double* scale, signed char* planes, void* stream);
 /* fmax[batch][S], arg[batch][S] = per-sample max / first arg-max over the P grid points of A . B_b^T from digit planes
  * (A sliced with tile_rows(0), batch 1; B with tile_rows(1), `batch` grids).  Fs_full (optional, tests): dense [batch][S x P].
  * workspace: ppbo_ozaki_rowmax_workspace_bytes(S, P, batch) bytes (partial maxima of the column-tile groups).
@@ -347,6 +370,12 @@ long long ppbo_ozaki_rowmax_workspace_bytes(int S, int P, int batch);
 int ppbo_ozaki_rowmax(const signed char* Aplanes, const double* ascale, int S, const signed char* Bplanes, const double* bscale,
                       int P, int batch, int K, int slices, double* fmax, int* arg, double* Fs_full, void* workspace,
                       long long workspace_bytes, int* err_flag, void* stream);
+/* The same with a column offset: fmax[b][s] = max_p (bias[b][p] + (A . B_b^T)[s][p]), each element formed as ONE fma of the exact
+ * scaled product and the offset (so equal to ozaki_matmul + bias, bit for bit); first arg-max on ties as above.  The posterior
+ * mean mu_p = phi(x_p)' omega_MAP of the full-covariance draws f_s(x_p) = mu_p + z_s . (L^-1 phi(x_p)).  bias: [batch][P]. */
+int ppbo_ozaki_rowmax_bias(const signed char* Aplanes, const double* ascale, int S, const signed char* Bplanes, const double* bscale,
+                           const double* bias, int P, int batch, int K, int slices, double* fmax, int* arg, double* Fs_full,
+                           void* workspace, long long workspace_bytes, int* err_flag, void* stream);
 /* diagnostic: SM clocks for `iters` back-to-back 128 x N x 32 INT8 MMAs on `blocks` SMs, rotating over `nacc` accumulators
  * (mode 0: A, B from shared memory; 1: A from TMEM; 2: B plane re-used); clocks_out[blocks] device int64.
  * Used by scripts/ozaki_probe.py --ubench. */

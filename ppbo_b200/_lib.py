@@ -86,17 +86,24 @@ _SIGNATURES = {
     "ppbo_rff_factor_cache_doubles": (_L, [_I]),
     "ppbo_rff_fit": (_I, [_P, _L, _I, _I, _I, _D, _P, _I, _D, _P, _I, _P, _P, _P, _L, _PD, _P]),
     "ppbo_rff_refactor": (_I, [_P, _L, _I, _I, _I, _D, _P, _P, _P, _L, _P]),
+    "ppbo_rff_hessian_factor_workspace_bytes": (_L, [_I, _I, _I]),
+    "ppbo_rff_hessian_factor_doubles": (_L, [_I, _L]),
+    "ppbo_rff_hessian_factor": (_I, [_P, _L, _I, _I, _I, _D, _P, _P, _L, _P, _L, _PI, _P]),
     "ppbo_normal_fill": (_I, [c_ulonglong, c_uint, _L, _P, _L, _P]),
     "ppbo_rff_sample_omega": (_I, [_P, _P, _P, _L, c_ulonglong, c_uint, _L, _I, _I, _P, _L, _P]),
+    "ppbo_rff_sample_omega_full_workspace_bytes": (_L, [_I, _I]),
+    "ppbo_rff_sample_omega_full": (_I, [_P, _P, _L, _P, _L, c_ulonglong, c_uint, _L, _I, _I, _P, _L, _P, _L, _P]),
     "ppbo_rff_eval_argmax": (_I, [_P, _L, _I, _I, _P, _L, _L, _I, _I, _P, _P, _P, _P]),
     "ppbo_ozaki_tile_rows": (_I, [_I]),
     "ppbo_ozaki_plane_bytes": (_L, [_I, _I, _I, _I, _I]),
     "ppbo_ozaki_scale_doubles": (_L, [_I, _I, _I]),
     "ppbo_ozaki_slice": (_I, [_P, _L, _L, _I, _I, _I, _I, _I, _P, _P, _P]),
     "ppbo_ozaki_sample_slice": (_I, [_P, _P, c_ulonglong, c_uint, _L, _I, _I, _I, _P, _P, _P]),
+    "ppbo_ozaki_normal_slice": (_I, [c_ulonglong, c_uint, _L, _I, _I, _I, _P, _P, _P]),
     "ppbo_ozaki_mma_rate": (_I, [_I, _I, _I, _I, _I, _P, _P]),
     "ppbo_ozaki_rowmax_workspace_bytes": (_L, [_I, _I, _I]),
     "ppbo_ozaki_rowmax": (_I, [_P, _P, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _L, _P, _P]),
+    "ppbo_ozaki_rowmax_bias": (_I, [_P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _L, _P, _P]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

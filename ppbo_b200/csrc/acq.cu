@@ -398,6 +398,20 @@ __global__ void __launch_bounds__(256) rff_psi_kernel(const double* __restrict__
     const double a = arrow[u];
     PsiT[(long long)f * ldp + u] = a > 0.0 ? sqrt(a) * (ph[(long long)q * (m + 1) + 1 + j] - ph[(long long)q * (m + 1)]) : 0.0;
 }
+// Signed form for the exact Hessian I + Psi' diag(a) Psi (ppbo_rff_hessian_factor): PsiA[f][u] = sqrt|a_u| d_u(f) and
+// PsiB[f][u] = sign(a_u) sqrt|a_u| d_u(f), d_u = Phi[f][r(u)] - Phi[f][w(u)], so that PsiA . PsiB^T = sum_u a_u d_u d_u'.
+__global__ void __launch_bounds__(256) rff_psi_signed_kernel(const double* __restrict__ Phi, long long ld, int Q, int m,
+                                                             const double* __restrict__ arrow, double* __restrict__ PsiA,
+                                                             double* __restrict__ PsiB, long long ldp) {
+    const int u = blockIdx.x * blockDim.x + threadIdx.x, f = blockIdx.y;
+    if (u >= Q * m) return;
+    const int q = u / m, j = u % m;
+    const double* ph = Phi + (long long)f * ld;
+    const double a = arrow[u];
+    const double v = sqrt(fabs(a)) * (ph[(long long)q * (m + 1) + 1 + j] - ph[(long long)q * (m + 1)]);
+    PsiA[(long long)f * ldp + u] = v;
+    PsiB[(long long)f * ldp + u] = a < 0.0 ? -v : v;
+}
 __global__ void add_identity_kernel(double* __restrict__ A, long long ld, int n) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) A[(long long)i * ld + i] += 1.0;
@@ -1119,6 +1133,47 @@ extern "C" int ppbo_rff_refactor(const double* Phi_X, long long ld, int F, int Q
     return blockinv_build(ws.H, F, F, Hdinv, ws.binv, st);
 }
 
+/* The exact weight-space Hessian -grad^2 S(omega) = I + Psi' diag(a) Psi with the SIGNED coefficients a (the fit factors the clamped
+ * I + Psi' a+ Psi, which is the right chord matrix but not the Laplace precision), factorised into the caller's L: the full
+ * covariance of the weight-space posterior is its inverse.  Nothing of the fit's factor cache is touched. */
+extern "C" long long ppbo_rff_hessian_factor_workspace_bytes(int F, int Q, int m) {
+    return ppbo_rff_workspace_bytes(F, Q, m) + (long long)F * Q * m * 8;
+}
+extern "C" long long ppbo_rff_hessian_factor_doubles(int F, long long ldl) {
+    return (long long)F * ldl + potrf_dinv_doubles(F) + 2;
+}
+
+extern "C" int ppbo_rff_hessian_factor(const double* Phi_X, long long ld, int F, int Q, int m, double sigma, const double* omega,
+                                       double* L, long long ldl, void* workspace, long long workspace_bytes, int* info_h,
+                                       void* stream) {
+    PPBO_REQUIRE(F >= 1 && Q >= 1 && m >= 1 && ldl >= F && L != nullptr, "shape");
+    PPBO_REQUIRE(workspace_bytes >= ppbo_rff_hessian_factor_workspace_bytes(F, Q, m), "workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int M = Q * m;
+    RffWs ws;
+    ws.carve((double*)workspace, F, Q, m);
+    double* PsiB = (double*)workspace + ppbo_rff_workspace_bytes(F, Q, m) / 8;
+    double* dinv = L + (long long)F * ldl;
+    int* info_d = reinterpret_cast<int*>(dinv + potrf_dinv_doubles(F));
+    PPBO_CUDA_CHECK(ws.zero_counters(st));
+    int rc;
+    if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega, ws, nullptr, nullptr, true, ws.scal + 24, st))) return rc;
+    PPBO_CL rff_psi_signed_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, PsiB, M);
+    GemmOperands g{ws.PsiT, M, 0, PsiB, M, 0, F, F, M};
+    StoreEpilogue ep{L, ldl, 0, 1.0, 0.0, 2, 0, 0};                  // lower tiles only: the factorisation reads no more
+    if ((rc = launch_gemm_nt(g, ep, 1, st))) return rc;
+    PPBO_CL add_identity_kernel<<<ceil_div(F, 256), 256, 0, st>>>(L, ldl, F);
+    PPBO_LAUNCH_CHECK();
+    if ((rc = potrf_lower(L, ldl, F, dinv, info_d, st))) return rc;
+    if (!info_h) return PPBO_OK;
+    int info = 0;
+    PPBO_CUDA_CHECK(readback().add(&info, info_d, sizeof(int), st));
+    PPBO_CUDA_CHECK(readback().finish(st));
+    *info_h = info;
+    if (info) set_error("exact weight-space Hessian not positive definite (pivot %d)", info);
+    return info;
+}
+
 extern "C" int ppbo_rff_eval_argmax(const double* Omega, long long ldo, int S, int F, const double* PhiT_grid, long long ldp,
                                     long long stridePhi, int P, int batch, double* fmax, int* arg, double* Fs_full,
                                     void* stream) {
@@ -1177,6 +1232,14 @@ __global__ void __launch_bounds__(256) sample_omega_kernel(const double* __restr
     if (f0 + 1 < F) o[f0 + 1] = omega_map[f0 + 1] + z1 * rsqrt(-hess_diag[f0 + 1]);
 }
 
+// Omega[s][:] = omega_map (the mean the full-covariance draw adds to Z L^-1)
+__global__ void __launch_bounds__(256) rows_fill_kernel(const double* __restrict__ v, int F, double* __restrict__ Out, long long ld) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f < F) Out[(long long)blockIdx.y * ld + f] = v[f];
+}
+
+int set_identity(double* A, long long ld, int n, cudaStream_t st);   // gram.cu
+
 }  // namespace ppbo
 
 extern "C" int ppbo_normal_fill(unsigned long long seed, unsigned int stream_id, long long offset, double* out, long long n,
@@ -1206,4 +1269,35 @@ extern "C" int ppbo_rff_sample_omega(const double* omega_map, const double* hess
     }
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
+}
+
+/* Omega = 1 omega_map' + Z L^-1 with H = L L' the factor of ppbo_rff_hessian_factor: draws from N(omega_map, H^-1).  L^-1 is applied as
+ * (L^-T)' with L^-T formed once (the triangular solve of the identity of ppbo_potri_lower), then one GEMM over the S rows. */
+extern "C" long long ppbo_rff_sample_omega_full_workspace_bytes(int S, int F) {
+    return ((long long)F * F + (long long)S * F) * 8;
+}
+
+extern "C" int ppbo_rff_sample_omega_full(const double* omega_map, const double* L, long long ldl, const double* Z, long long ldz,
+                                          unsigned long long seed, unsigned int stream_id, long long sample0, int S, int F,
+                                          double* Omega, long long ldo, void* workspace, long long workspace_bytes, void* stream) {
+    PPBO_REQUIRE(S >= 0 && F >= 1 && ldl >= F && ldo >= F && (Z == nullptr || ldz >= F), "shape");
+    PPBO_REQUIRE(S <= 65535, "at most 65535 samples per call");
+    PPBO_REQUIRE(workspace_bytes >= ppbo_rff_sample_omega_full_workspace_bytes(S, F), "workspace too small");
+    if (S == 0) return PPBO_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    double* LinvT = (double*)workspace;
+    int rc;
+    if ((rc = set_identity(LinvT, F, F, st))) return rc;
+    if ((rc = trsm_right_lower_t(L, ldl, F, L + (long long)F * ldl, LinvT, F, F, st))) return rc;     // L^-T (upper)
+    if (!Z) {
+        double* Zw = LinvT + (long long)F * F;
+        if ((rc = ppbo_normal_fill(seed, stream_id, sample0 * F, Zw, (long long)S * F, stream))) return rc;
+        Z = Zw;
+        ldz = F;
+    }
+    PPBO_CL rows_fill_kernel<<<dim3(ceil_div(F, 256), S), 256, 0, st>>>(omega_map, F, Omega, ldo);
+    PPBO_LAUNCH_CHECK();
+    GemmOperands g{Z, ldz, 0, LinvT, F, 0, S, F, F};
+    StoreEpilogue ep{Omega, ldo, 0, 1.0, 1.0, 0, 0, 0};              // Omega = Z (L^-T)' + 1 omega'
+    return launch_gemm_nt(g, ep, 1, st);
 }

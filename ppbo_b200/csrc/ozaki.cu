@@ -130,7 +130,9 @@ __global__ void __launch_bounds__(256) ozaki_slice_kernel(const double* __restri
 // CTA), its row scale is taken there, and the planes are cut from shared memory exactly as ozaki_slice_kernel does from HBM.  The
 // S x F matrix of draws (262 MB at S = 32768, F = 1000) never exists: 8 B written + 16 B read per element become 0.
 // Bit-identical to sample_omega_kernel -> ozaki_rowscale_kernel -> ozaki_slice_kernel (same expressions, same rounding).
-template <int KS>
+// RAW: the planes of z itself (no omega_map / hess_diag applied): the draws of the full-covariance contraction, whose covariance
+// sits in the grid operand instead (ppbo_ozaki_normal_slice); bit-identical to ppbo_normal_fill -> ppbo_ozaki_slice.
+template <int KS, bool RAW = false>
 __global__ void __launch_bounds__(256) ozaki_sample_slice_kernel(const double* __restrict__ omega_map, const double* __restrict__ hess_diag,
                                                                  unsigned long long seed, uint32_t stream_id, long long sample0, int S,
                                                                  int rows_pad, int F, int KBLK, double* __restrict__ scale,
@@ -158,12 +160,12 @@ __global__ void __launch_bounds__(256) ozaki_sample_slice_kernel(const double* _
                     philox_normal2(seed, (unsigned long long)((e + 1) >> 1), stream_id, a, b);
                     z1 = a;
                 }
-                const double v0 = omega_map[f0] + z0 * rsqrt(-hess_diag[f0]);
+                const double v0 = RAW ? z0 : omega_map[f0] + z0 * rsqrt(-hess_diag[f0]);
                 x[f0] = v0;
                 double v = fabs(v0);
                 amax = (v > amax || v != v) ? v : amax;
                 if (f0 + 1 < F) {
-                    const double v1 = omega_map[f0 + 1] + z1 * rsqrt(-hess_diag[f0 + 1]);
+                    const double v1 = RAW ? z1 : omega_map[f0 + 1] + z1 * rsqrt(-hess_diag[f0 + 1]);
                     x[f0 + 1] = v1;
                     v = fabs(v1);
                     amax = (v > amax || v != v) ? v : amax;
@@ -350,6 +352,15 @@ struct Params {
     int* err;
     int diag;      // timing experiments only (tuning key 2): bit 0 = epilogue skips the TMEM reads, bit 1 = producer skips the copies
 };
+// The biased instantiations take the offsets in a derived parameter block: a field added to Params itself changes the code ptxas
+// emits for the unbiased kernels (same arithmetic, other registers and layout).
+struct BiasParams : Params {
+    const double* bias;                                        // [batch][P] column offsets
+};
+template <bool BIAS> struct ParamsOf { using T = Params; };
+template <> struct ParamsOf<true> { using T = BiasParams; };
+__device__ __forceinline__ const double* bias_row(const Params&, int, int) { return nullptr; }
+__device__ __forceinline__ const double* bias_row(const BiasParams& p, int b, int P) { return p.bias + (long long)b * P; }
 
 // Work order.  item -> (grid b, row tile mt, column-tile group ng):  grids in blocks of GB; inside a block the row tiles; inside a
 // row tile the GB grids of the block; inside a grid the NG column groups (fastest).  The ~SM-count items in flight then cover
@@ -375,9 +386,12 @@ __device__ __forceinline__ void decode_item(const Params& p, int item, int& b, i
 // v = (hi + lo 2^-8(KS-G1)) * bs;  the common factor 2^-8(G1+1) and the row scale are applied once per row by the caller.
 // For KS <= 6 both words stay below 2^44 and are converted by adding them to the bit pattern of 2^52 + 2^51 (exact; the
 // INT64 -> FP64 convert instruction is a quarter-rate op and was a third of the epilogue's issue slots).
-template <int KS, int G1, bool CHECKED, int NC>
+// BIAS: every element gets its column's offset, e = fma(v, as2, brow[col]) (one rounding: v as2 is exact, a power-of-two scale), so
+// the row scale is applied per element and the max runs over e; without it the scale is applied once per row after the max.
+template <int KS, int G1, bool CHECKED, int NC, bool BIAS = false>
 __device__ __forceinline__ void epi_columns(const uint32_t (&acc)[KS][NC], const double* __restrict__ bs, int col0, int P,
-                                            double* __restrict__ full_row, double as2, double& best, int& best_arg) {
+                                            double* __restrict__ full_row, double as2, double& best, int& best_arg,
+                                            const double* __restrict__ brow = nullptr) {
     constexpr long long MAGIC = 0x4338000000000000LL;             // bits of 2^52 + 2^51
     const double magic_d = 6755399441055744.0, lo_w = 1.0 / (double)(1ull << (8 * (KS - G1)));
 #pragma unroll
@@ -399,18 +413,22 @@ __device__ __forceinline__ void epi_columns(const uint32_t (&acc)[KS][NC], const
         const int col = col0 + c;
         if (CHECKED) {
             if (col < P) {
-                if (full_row) full_row[col] = v * as2;
-                if (v > best) { best = v; best_arg = col; }
+                const double e = BIAS ? fma(v, as2, __ldg(brow + col)) : v;
+                if (full_row) full_row[col] = BIAS ? e : v * as2;
+                if (e > best) { best = e; best_arg = col; }
             }
-        } else if (v > best) {
-            best = v;
-            best_arg = col;
+        } else {
+            const double e = BIAS ? fma(v, as2, __ldg(brow + col)) : v;
+            if (e > best) {
+                best = e;
+                best_arg = col;
+            }
         }
     }
 }
 
-template <int KS, int BN, bool TS>
-__global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const Params p) {
+template <int KS, int BN, bool TS, bool BIAS = false>
+__global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename ParamsOf<BIAS>::T p) {
     using C = Cfg<KS, BN, TS>;
     extern __shared__ __align__(1024) uint8_t smem[];
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::STAGES * C::STAGE_BYTES);
@@ -551,6 +569,7 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const Params p
             const int nt0 = ng * p.ntg, nt1 = min(p.NT, nt0 + p.ntg);
             const int row = mt * BM + q * 32 + lane;
             const double as2 = ((row < p.S) ? p.ascale[row] : 1.0) * c_hi;     // row scale and the weight of the high word
+            const double* brow = bias_row(p, b, p.P);
             double best = -INFINITY;
             int best_arg = 0;
             for (int nt = nt0; nt < nt1; ++nt, ++tile) {
@@ -573,8 +592,8 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const Params p
                             for (int d = 0; d < KS; ++d) tc_ld8(lane_addr + (uint32_t)(d * BN + cbase + (k + 1) * 8), acc[(k + 1) & 1][d]);
                         }
                         const int col0 = nt * BN + cbase + k * 8;
-                        if (checked) epi_columns<KS, C::G1, true, 8>(acc[k & 1], bs + k * 8, col0, p.P, full_row, as2, best, best_arg);
-                        else epi_columns<KS, C::G1, false, 8>(acc[k & 1], bs + k * 8, col0, p.P, nullptr, as2, best, best_arg);
+                        if (checked) epi_columns<KS, C::G1, true, 8, BIAS>(acc[k & 1], bs + k * 8, col0, p.P, full_row, as2, best, best_arg, brow);
+                        else epi_columns<KS, C::G1, false, 8, BIAS>(acc[k & 1], bs + k * 8, col0, p.P, nullptr, as2, best, best_arg, brow);
                     }
                 }
                 tc_fence_before();
@@ -595,7 +614,7 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const Params p
                 const int a1 = ma[q * 32 + lane];
                 if (v1 > best || (v1 == best && a1 < best_arg)) { best = v1; best_arg = a1; }
                 if (row < p.S) {
-                    p.fmax[((long long)b * p.NG + ng) * p.S + row] = best * as2;
+                    p.fmax[((long long)b * p.NG + ng) * p.S + row] = BIAS ? best : best * as2;
                     p.arg[((long long)b * p.NG + ng) * p.S + row] = best_arg;
                 }
             }
@@ -669,13 +688,13 @@ static int slice_launch(const double* X, long long ldx, long long strideX, int r
     return PPBO_OK;
 }
 
-template <int KS, int BN, bool TS>
-static int rowmax_launch(const Params& p, cudaStream_t st) {
+template <int KS, int BN, bool TS, bool BIAS = false>
+static int rowmax_launch(const typename ParamsOf<BIAS>::T& p, cudaStream_t st) {
     using C = Cfg<KS, BN, TS>;
     static std::once_flag once;
     static cudaError_t err = cudaSuccess;
     std::call_once(once, [] {
-        err = cudaFuncSetAttribute(ozaki_rowmax_kernel<KS, BN, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
+        err = cudaFuncSetAttribute(ozaki_rowmax_kernel<KS, BN, TS, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
     });
     PPBO_CUDA_CHECK(err);
     int dev = 0, sms = PPBO_SM_COUNT;
@@ -690,7 +709,7 @@ static int rowmax_launch(const Params& p, cudaStream_t st) {
     // collect their SMs one by one as ~120 us work items end and the GP fit stretches from 10.6 to 15.3 ms.
     const int reserve = g_tuning[14];
     const int grid = reserve < 0 ? items : min(items, max(sms - reserve, 1));
-    PPBO_CL ozaki_rowmax_kernel<KS, BN, TS><<<grid, THREADS, C::SMEM, st>>>(p);
+    PPBO_CL ozaki_rowmax_kernel<KS, BN, TS, BIAS><<<grid, THREADS, C::SMEM, st>>>(p);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
 }
@@ -819,18 +838,18 @@ extern "C" int ppbo_ozaki_slice(const double* X, long long ldx, long long stride
 }
 
 namespace ppbo { namespace oz {
-template <int KS>
+template <int KS, bool RAW = false>
 static int sample_slice_launch(const double* omega_map, const double* hess_diag, unsigned long long seed, unsigned int stream_id,
                                long long sample0, int S, int F, double* scale, int8_t* planes, cudaStream_t st) {
     const Shape s = shape_of(S, F, BM, 1, KS);
     const int smem = 8 * s.KBLK * KB * (int)sizeof(double);
     static std::once_flag once;
     static cudaError_t err = cudaSuccess;
-    std::call_once(once, [] { err = cudaFuncSetAttribute(ozaki_sample_slice_kernel<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
+    std::call_once(once, [] { err = cudaFuncSetAttribute(ozaki_sample_slice_kernel<KS, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
     PPBO_CUDA_CHECK(err);
     PPBO_REQUIRE(smem <= 200 * 1024, "F too large for the fused draw (8 rows of F doubles must fit shared memory)");
-    PPBO_CL ozaki_sample_slice_kernel<KS><<<s.rows_pad / 8, 256, smem, st>>>(omega_map, hess_diag, seed, stream_id, sample0, S, s.rows_pad, F,
-                                                                              s.KBLK, scale, planes);
+    PPBO_CL ozaki_sample_slice_kernel<KS, RAW><<<s.rows_pad / 8, 256, smem, st>>>(omega_map, hess_diag, seed, stream_id, sample0, S,
+                                                                                   s.rows_pad, F, s.KBLK, scale, planes);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
 }
@@ -851,22 +870,37 @@ extern "C" int ppbo_ozaki_sample_slice(const double* omega_map, const double* he
     }
 }
 
+extern "C" int ppbo_ozaki_normal_slice(unsigned long long seed, unsigned int stream_id, long long sample0, int S, int F, int slices,
+                                       double* scale, signed char* planes, void* stream) {
+    PPBO_REQUIRE(S >= 0 && F >= 1, "shape");
+    PPBO_REQUIRE(slices >= 5 && slices <= oz::MAX_KS, "slices in [5, 7]");
+    PPBO_REQUIRE((reinterpret_cast<uintptr_t>(planes) & 15) == 0, "planes must be 16-byte aligned");
+    if (S == 0) return PPBO_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    int8_t* pl = reinterpret_cast<int8_t*>(planes);
+    switch (slices) {
+        case 5: return oz::sample_slice_launch<5, true>(nullptr, nullptr, seed, stream_id, sample0, S, F, scale, pl, st);
+        case 6: return oz::sample_slice_launch<6, true>(nullptr, nullptr, seed, stream_id, sample0, S, F, scale, pl, st);
+        default: return oz::sample_slice_launch<7, true>(nullptr, nullptr, seed, stream_id, sample0, S, F, scale, pl, st);
+    }
+}
+
 extern "C" long long ppbo_ozaki_rowmax_workspace_bytes(int S, int P, int batch) {
     if (S < 0 || P < 1 || batch < 1) return -1;
     const int NT = ceil_div(P, oz::BN_DEFAULT);               // room for any grouping
     return NT > 1 ? (long long)batch * NT * S * 12 + 16 : 0;
 }
 
-extern "C" int ppbo_ozaki_rowmax(const signed char* Aplanes, const double* ascale, int S, const signed char* Bplanes,
-                                 const double* bscale, int P, int batch, int K, int slices, double* fmax, int* arg,
-                                 double* Fs_full, void* workspace, long long workspace_bytes, int* err_flag, void* stream) {
+static int ozaki_rowmax_impl(const signed char* Aplanes, const double* ascale, int S, const signed char* Bplanes,
+                             const double* bscale, const double* bias, int P, int batch, int K, int slices, double* fmax, int* arg,
+                             double* Fs_full, void* workspace, long long workspace_bytes, int* err_flag, void* stream) {
     PPBO_REQUIRE(S >= 0 && P >= 1 && batch >= 1 && K >= 1, "shape");
     PPBO_REQUIRE(slices >= 5 && slices <= oz::MAX_KS, "slices in [5, 7]");
     PPBO_REQUIRE(ceil_div(K, oz::KB) * oz::KB <= 16384, "K <= 16384 (INT32 accumulator range)");
     PPBO_REQUIRE((reinterpret_cast<uintptr_t>(Aplanes) & 15) == 0 && (reinterpret_cast<uintptr_t>(Bplanes) & 15) == 0,
                  "digit planes must be 16-byte aligned");
     if (S == 0) return PPBO_OK;
-    oz::Params p;
+    oz::BiasParams p;
     p.A = reinterpret_cast<const int8_t*>(Aplanes); p.ascale = ascale; p.S = S; p.MT = ceil_div(S, oz::BM);
     p.B = reinterpret_cast<const int8_t*>(Bplanes); p.bscale = bscale; p.P = P; p.NT = ceil_div(P, oz::BN_DEFAULT); p.batch = batch;
     p.KBLK = ceil_div(K, oz::KB);
@@ -886,13 +920,21 @@ extern "C" int ppbo_ozaki_rowmax(const signed char* Aplanes, const double* ascal
     int* parg = reinterpret_cast<int*>(pmax + (long long)batch * p.NG * S);
     p.fmax = p.NG > 1 ? pmax : fmax; p.arg = p.NG > 1 ? parg : arg; p.full = Fs_full; p.ld_full = P; p.stride_full = (long long)S * P; p.err = err_flag;
     p.diag = g_tuning[2];
+    p.bias = bias;
+    const oz::Params& p0 = p;                  // the unbiased kernels take the base block
     cudaStream_t st = (cudaStream_t)stream;
     const bool ts = g_tuning[1] == 1;          // tuning key 1: 1 = A planes staged in TMEM (comparison variant, slower)
     int rc;
-    switch (slices) {
-        case 5: rc = ts ? oz::rowmax_launch<5, oz::BN_DEFAULT, true>(p, st) : oz::rowmax_launch<5, oz::BN_DEFAULT, false>(p, st); break;
-        case 6: rc = ts ? oz::rowmax_launch<6, oz::BN_DEFAULT, true>(p, st) : oz::rowmax_launch<6, oz::BN_DEFAULT, false>(p, st); break;
-        default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT, false>(p, st); break;   // 7 x 64 + 7 x 16 columns exceed TMEM
+    if (bias) {                                // (no TMEM-staged variant of the biased epilogue)
+        switch (slices) {
+            case 5: rc = oz::rowmax_launch<5, oz::BN_DEFAULT, false, true>(p, st); break;
+            case 6: rc = oz::rowmax_launch<6, oz::BN_DEFAULT, false, true>(p, st); break;
+            default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT, false, true>(p, st); break;
+        }
+    } else switch (slices) {
+        case 5: rc = ts ? oz::rowmax_launch<5, oz::BN_DEFAULT, true>(p0, st) : oz::rowmax_launch<5, oz::BN_DEFAULT, false>(p0, st); break;
+        case 6: rc = ts ? oz::rowmax_launch<6, oz::BN_DEFAULT, true>(p0, st) : oz::rowmax_launch<6, oz::BN_DEFAULT, false>(p0, st); break;
+        default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT, false>(p0, st); break;   // 7 x 64 + 7 x 16 columns exceed TMEM
     }
     if (rc) return rc;
     if (p.NG > 1) {
@@ -900,4 +942,20 @@ extern "C" int ppbo_ozaki_rowmax(const signed char* Aplanes, const double* ascal
         PPBO_LAUNCH_CHECK();
     }
     return PPBO_OK;
+}
+
+extern "C" int ppbo_ozaki_rowmax(const signed char* Aplanes, const double* ascale, int S, const signed char* Bplanes,
+                                 const double* bscale, int P, int batch, int K, int slices, double* fmax, int* arg,
+                                 double* Fs_full, void* workspace, long long workspace_bytes, int* err_flag, void* stream) {
+    return ozaki_rowmax_impl(Aplanes, ascale, S, Bplanes, bscale, nullptr, P, batch, K, slices, fmax, arg, Fs_full, workspace,
+                             workspace_bytes, err_flag, stream);
+}
+
+extern "C" int ppbo_ozaki_rowmax_bias(const signed char* Aplanes, const double* ascale, int S, const signed char* Bplanes,
+                                      const double* bscale, const double* bias, int P, int batch, int K, int slices, double* fmax,
+                                      int* arg, double* Fs_full, void* workspace, long long workspace_bytes, int* err_flag,
+                                      void* stream) {
+    PPBO_REQUIRE(bias != nullptr, "bias missing");
+    return ozaki_rowmax_impl(Aplanes, ascale, S, Bplanes, bscale, bias, P, batch, K, slices, fmax, arg, Fs_full, workspace,
+                             workspace_bytes, err_flag, stream);
 }

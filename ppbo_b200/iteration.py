@@ -33,6 +33,11 @@ SHRINKAGE = 1e-6          # GPModel.COVARIANCE_SHRINKAGE, src/gp_model.py:26
 SAMPLING_ENGINE = "i8"
 SAMPLING_SLICES = 6
 I8_MIN_WORK = 1 << 24     # S * P * F below which the FP64 kernel is used
+# Covariance of the weight-space Laplace posterior the draws come from: "diag" = the reference's 1 / -hess_diag
+# (src/random_fourier_sampler.py:134-137), "full" = the inverse of the exact Hessian I + Psi' diag(a) Psi (opt-in).  With "full" the
+# draws stay standard normals z_s and the covariance moves into the grid operand: f_s(x_p) = mu_p + z_s . Phi~_p with
+# mu_p = phi(x_p)' omega_MAP and Phi~ = Phi L^-T, H = L L'.
+WEIGHT_COVARIANCES = ("diag", "full")
 
 
 # The GP fit and the weight-space (RFF) fit only share their input X: both are chains of small, latency-bound launches with one
@@ -277,8 +282,23 @@ def mustar_over_candidates(g, candidates=None):
 
 
 class RFFFit:
-    """Device-resident state of Hsampler after update_phi_X / update_omega_MAP / update_covariancematrix."""
-    __slots__ = ("W", "b", "sigma_f", "Phi_X", "omega_map", "hess_diag", "stats")
+    """Device-resident state of Hsampler after update_phi_X / update_omega_MAP / update_covariancematrix.  L: buffer of the exact
+    Hessian factor (ops.rff_hessian_factor_buffer) for the full covariance, None for the diagonal one."""
+    __slots__ = ("W", "b", "sigma_f", "Phi_X", "omega_map", "hess_diag", "stats", "L")
+
+    def __init__(self):
+        self.L = None
+
+
+def rff_full_factor(r, Q, m, sigma, out=None):
+    """r.L <- factor of the exact weight-space Hessian at r.omega_map (into `out`, a rff_hessian_factor_buffer, or a new one)"""
+    Fdim = r.omega_map.shape[0]
+    out = ops.rff_hessian_factor_buffer(Fdim, r.omega_map.device) if out is None else out
+    info = ops.rff_hessian_factor(r.Phi_X, Q, m, sigma, r.omega_map, out)
+    if info != 0:
+        raise PPBOError("exact weight-space Hessian not positive definite (pivot %d)" % info)
+    r.L = out
+    return r
 
 
 def rff_fit(X, W, b, theta, Q, m, omega0=None, max_iter=100, tol=1e-10, f_map=None):
@@ -303,6 +323,7 @@ class RFFState:
         self.max_iter, self.tol = max_iter, tol
         self.Phi_cap = torch.empty((W.shape[0], Q_cap * (m + 1)), dtype=F64, device=W.device)
         self.factor_cache = ops.rff_factor_cache(W.shape[0], W.device)
+        self.L_buf = None            # exact-Hessian factor of the full covariance: its own buffer, never the fit's factor_cache
         self.fit = None
         self.pending = None          # stream of an asynchronous refresh of the factor (refresh_factor): the next fit waits for it
 
@@ -316,6 +337,12 @@ class RFFState:
             raise PPBOError("RFF fit: weight-space Hessian not positive definite (info=%d)" % r.stats["info"])
         self.Q, self.fit = Q, r
         return r
+
+    def hessian_factor(self):
+        """exact-Hessian factor of the current fit (full covariance) into this model's own buffer"""
+        if self.L_buf is None:
+            self.L_buf = ops.rff_hessian_factor_buffer(self.W.shape[0], self.W.device)
+        return rff_full_factor(self.fit, self.Q, self.m, self.theta[0], out=self.L_buf)
 
     def _wait_refresh(self):
         if self.pending is not None:
@@ -392,12 +419,42 @@ class SlicedSamples:
             self.planes, self.scale = ops.ozaki_slice(Omega, 0, self.slices)
 
 
-def rff_prepare_samples(r, lo, hi, P, Z=None, seed=0, stream_id=0):
+def rff_prepare_normals(Fdim, lo, hi, P, dev, Z=None, seed=0, stream_id=0):
+    """Standard normals [lo, hi) of the sample stream (the draws of the full covariance) in the form the contraction consumes: digit
+    planes for the INT8 engine, the FP64 matrix otherwise.  Independent of every fit."""
+    if hi <= lo:
+        return None
+    i8 = sampling_engine(hi - lo, P, Fdim) == "i8"
+    if Z is None and i8 and Fdim * 64 <= 200 * 1024:
+        return SlicedSamples(drawn=ops.ozaki_normal_slice(hi - lo, Fdim, dev, seed=seed, stream_id=stream_id, sample0=lo,
+                                                          slices=SAMPLING_SLICES), count=hi - lo)
+    Zloc = Z[lo:hi] if Z is not None else ops.normal_fill(seed, stream_id, lo * Fdim, (hi - lo) * Fdim, dev).view(hi - lo, Fdim)
+    return SlicedSamples(Zloc) if i8 else Zloc
+
+
+def rff_transform_grids(r, PhiT, slices=None):
+    """(mu [B, P], Phi~): the posterior mean phi(x_p)' omega_MAP and the grid features Phi L^-T of the full covariance, Phi~ cut
+    into `slices` digit planes (SlicedGrids) when given.  The triangular solve treats all B P rows in one call: same bits on
+    every rank."""
+    G = PhiT.PhiT if isinstance(PhiT, SlicedGrids) else PhiT
+    B, P, Fdim = G.shape
+    mu = ops.gemv(G.reshape(B * P, Fdim), r.omega_map).view(B, P)
+    L, ws = ops.hessian_factor_views(r.L, Fdim)
+    Gt = G.reshape(B * P, Fdim).clone()
+    ops.trsm_right_lower(L, ws, Gt)                    # rows phi_p' L^-T = (L^-1 phi_p)'
+    Gt = Gt.view(B, P, Fdim)
+    return mu, (SlicedGrids(Gt, slices) if slices is not None else Gt)
+
+
+def rff_prepare_samples(r, lo, hi, P, Z=None, seed=0, stream_id=0, covariance="diag"):
     """Draws [lo, hi) of the sample stream, already in the form the contraction consumes (digit planes for the INT8 engine, the
-    FP64 matrix otherwise).  Needs the weight-space fit only, so run_iteration does this while the GP fit is still running."""
+    FP64 matrix otherwise).  Needs the weight-space fit only, so run_iteration does this while the GP fit is still running.
+    covariance="full": the standard normals themselves (rff_prepare_normals)."""
     if hi <= lo:
         return None
     Fdim = r.omega_map.shape[0]
+    if covariance == "full":
+        return rff_prepare_normals(Fdim, lo, hi, P, r.omega_map.device, Z=Z, seed=seed, stream_id=stream_id)
     if Z is None and sampling_engine(hi - lo, P, Fdim) == "i8" and Fdim * 64 <= 200 * 1024:
         # draws and digit planes in one kernel: the S x F matrix of draws never reaches HBM
         return SlicedSamples(drawn=ops.ozaki_sample_slice(r.omega_map, r.hess_diag, hi - lo, seed=seed, stream_id=stream_id, sample0=lo,
@@ -407,12 +464,15 @@ def rff_prepare_samples(r, lo, hi, P, Z=None, seed=0, stream_id=0):
     return SlicedSamples(Omega) if sampling_engine(hi - lo, P, Fdim) == "i8" else Omega
 
 
-def rff_sampled_maxima(r, PhiT, lo, hi, Z=None, seed=0, stream_id=0, prepared=None):
+def rff_sampled_maxima(r, PhiT, lo, hi, Z=None, seed=0, stream_id=0, prepared=None, covariance="diag", transformed=None):
     """Posterior weight draws [lo, hi) of the sample stream evaluated on every grid: per-sample max and first arg-max over the grid
     points, (fmax [B, hi-lo], arg [B, hi-lo]); (None, None) for an empty slice.  Needs the weight-space fit only -- not mu*.
-    prepared: the result of rff_prepare_samples for the same slice."""
+    prepared: the result of rff_prepare_samples for the same slice.  covariance="full" (r.L set): max_p (mu_p + z_s . Phi~_p);
+    transformed: rff_transform_grids(r, PhiT) when the caller has it already."""
     if hi <= lo:
         return None, None
+    if covariance == "full":
+        return _sampled_maxima_full(r, PhiT, lo, hi, Z, seed, stream_id, prepared, transformed)
     sliced = PhiT if isinstance(PhiT, SlicedGrids) else None
     PhiT = sliced.PhiT if sliced is not None else PhiT
     B, P, Fdim = PhiT.shape
@@ -427,6 +487,23 @@ def rff_sampled_maxima(r, PhiT, lo, hi, Z=None, seed=0, stream_id=0, prepared=No
     return fmax, arg
 
 
+def _sampled_maxima_full(r, PhiT, lo, hi, Z, seed, stream_id, prepared, transformed):
+    G = PhiT.PhiT if isinstance(PhiT, SlicedGrids) else PhiT
+    B, P, Fdim = G.shape
+    if prepared is None:
+        prepared = rff_prepare_normals(Fdim, lo, hi, P, G.device, Z=Z, seed=seed, stream_id=stream_id)
+    if transformed is None:
+        transformed = rff_transform_grids(r, G, slices=prepared.slices if isinstance(prepared, SlicedSamples) else None)
+    mu, Gt = transformed
+    if isinstance(prepared, SlicedSamples):
+        err = torch.zeros(1, dtype=torch.int32, device=G.device)
+        fmax, arg, _ = ops.ozaki_rowmax(prepared.planes, prepared.scale, prepared.count, Gt.planes, Gt.scale, P, B, Fdim, prepared.slices,
+                                        err=err, bias=mu)
+    else:                                              # FP64 engine: the mean-offset row max of the exact-GP sampler
+        fmax, arg = ops.mvn_rowmax(prepared.unsqueeze(0).expand(B, -1, -1), Gt, mu)
+    return fmax, arg
+
+
 def rff_reduce(fmax, mustar_dev, n_grids, shard=None):
     """sums [B, 3] over all ranks' samples of max(fmax - mu*, 0), fmax, fmax^2 (one all-reduce of 3 B doubles)"""
     shard = shard or Shard()
@@ -438,13 +515,14 @@ def rff_reduce(fmax, mustar_dev, n_grids, shard=None):
     return sums
 
 
-def rff_acquisition(r, PhiT, S, mustar_dev, shard=None, Z=None, seed=0, stream_id=0, bounds=None, prepared=None, n_grids=None):
+def rff_acquisition(r, PhiT, S, mustar_dev, shard=None, Z=None, seed=0, stream_id=0, bounds=None, prepared=None, n_grids=None,
+                    covariance="diag"):
     """Sampled acquisition on B grids: per grid b the sums over the S samples of max(fmax - mu*, 0), fmax and fmax^2
     (acquisition.EI / varmax, src/acquisition.py:78-81,176-178, with RFF posterior draws in place of the exact-GP MVN).
     Returns (sums [B,3] reduced over all ranks, fmax [B,S_loc], arg [B,S_loc]); bounds: this rank's samples (default: even split)."""
     shard = shard or Shard()
     lo, hi = bounds if bounds is not None else shard.bounds(S)
-    fmax, arg = rff_sampled_maxima(r, PhiT, lo, hi, Z=Z, seed=seed, stream_id=stream_id, prepared=prepared)
+    fmax, arg = rff_sampled_maxima(r, PhiT, lo, hi, Z=Z, seed=seed, stream_id=stream_id, prepared=prepared, covariance=covariance)
     if n_grids is None:                 # (a rank without samples has no grid features: the caller passes the count)
         n_grids = (PhiT.PhiT if isinstance(PhiT, SlicedGrids) else PhiT).shape[0]
     return rff_reduce(fmax, mustar_dev, n_grids, shard), fmax, arg
@@ -523,7 +601,7 @@ class IterationState:
 
 
 def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, tol=1e-8, timers=None, state=None, shares=None,
-                  factor_at_mode=False, shard_mustar=None):
+                  factor_at_mode=False, shard_mustar=None, weight_covariance="diag"):
     """d: dict of device tensors (IterationInputs.to_device).  Returns (sums [B,3] device, gp, rff).
     Rank 0 fits; the others receive (omega_MAP, hess_diag, mu*) by broadcast while they compute the grid features.
     tol: both Newton iterations stop when the last full step is below tol relative to the iterate.  The chord steps contract
@@ -535,7 +613,13 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     factor_at_mode: also produce the Cholesky factor at the GP mode (only prediction with covariance needs it).
     shard_mustar: split the mu* candidates over the ranks (alpha by broadcast, one all-reduce(max)).  Pays when the other ranks are
     idle by the time the GP fit ends (default: 3 or more ranks and a cold fit); when they are still sampling, rank 0 would wait for
-    them inside the collective."""
+    them inside the collective.
+    weight_covariance: "diag" (the reference's) or "full" (WEIGHT_COVARIANCES): the rank that fits the weight space also factors the
+    exact Hessian at omega_MAP and sends the factor with (omega_MAP, hess_diag); the draws are standard normals and every sampling
+    rank transforms its grid features once (rff_transform_grids)."""
+    if weight_covariance not in WEIGHT_COVARIANCES:
+        raise PPBOError("weight_covariance must be one of %s" % (WEIGHT_COVARIANCES,))
+    full = weight_covariance == "full"
     shard = shard or Shard()
     W, b, grids = d["W"], d["b"], d["grids"]
     dev = W.device
@@ -567,10 +651,10 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
 
     def fit_rff():
         if state is None:
-            return rff_fit(X, W, b, theta, Q, m, omega0=d.get("omega0"), max_iter=fit_iters, tol=tol)
-        if warm:
-            return state.rff.append(block)
-        return state.rff.cold(X, omega0=d.get("omega0"))
+            r = rff_fit(X, W, b, theta, Q, m, omega0=d.get("omega0"), max_iter=fit_iters, tol=tol)
+            return rff_full_factor(r, Q, m, theta[0]) if full else r
+        r = state.rff.append(block) if warm else state.rff.cold(X, omega0=d.get("omega0"))
+        return state.rff.hessian_factor() if full else r
 
     def mu_star(gp, cand):
         """max posterior mean over the design rows and the candidate points; with >= 3 ranks every rank takes a slice of the
@@ -600,18 +684,33 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     grid_stream = _side_stream(dev, tag="grid") if shard.rank == 0 else main
     if grid_stream is not main:
         grid_stream.wait_stream(main)
-    PhiT = None
+    PhiT = normals = None
+    i8 = hi > lo and sampling_engine(hi - lo, P, Fdim) == "i8"
     with torch.cuda.stream(grid_stream):
         if hi > lo:                                           # a rank without samples (rank 0 of several) needs no grid features
             PhiT = rff_grid_features(W, b, theta[2], grids)
-            if sampling_engine(hi - lo, P, Fdim) == "i8":
+            if full:
+                # the draws of the full covariance are plain standard normals: cut into digit planes before any fit ends; the grid
+                # features are sliced after their transform by the Hessian factor
+                normals = rff_prepare_normals(Fdim, lo, hi, P, dev, seed=seed)
+            elif i8:
                 PhiT = SlicedGrids(PhiT)                      # digit planes of the grid features
     mark("grid_features")
+
+    def grid_tensors():
+        if PhiT is None:
+            return ()
+        out = (PhiT.PhiT, PhiT.planes, PhiT.scale) if isinstance(PhiT, SlicedGrids) else (PhiT,)
+        if isinstance(normals, SlicedSamples):
+            out += (normals.planes, normals.scale)
+        elif normals is not None:
+            out += (normals,)
+        return out
     pack = torch.empty(2 * Fdim + 1, dtype=F64, device=dev)
     gp = rff = prepared = None
     cand = grids.reshape(B * P, D)
     rff_rank = 1 if (CONCURRENT_FITS and shard.world > 1) else 0      # with more than one GPU the two fits run on two of them
-    if shard.rank == 0 and CONCURRENT_FITS and shard.world == 1 and OVERLAP_SAMPLING and isinstance(PhiT, SlicedGrids):
+    if shard.rank == 0 and CONCURRENT_FITS and shard.world == 1 and OVERLAP_SAMPLING and i8:
         # One GPU, INT8 engine.  Two chains that only share X:
         #   A  GP fit -> mu*                                   latency-bound, short (8.7 ms cold / 5 ms appended when alone)
         #   B  weight-space fit -> draws -> contraction        the contraction alone keeps every tensor pipe busy for ~9 ms
@@ -639,13 +738,23 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
                 mark("rff_fit")
                 fit_done = torch.cuda.Event()
                 fit_done.record(fg)
-                prepared = rff_prepare_samples(rff, lo, hi, P, seed=seed)
-                fg.wait_stream(grid_stream)
-                for t in (PhiT.PhiT, PhiT.planes, PhiT.scale):
-                    t.record_stream(fg)
+                transformed = None
+                if full:
+                    fg.wait_stream(grid_stream)
+                    for t in grid_tensors():
+                        t.record_stream(fg)
+                    prepared = normals
+                    transformed = rff_transform_grids(rff, PhiT, slices=SAMPLING_SLICES)
+                    mark("grid_transform")
+                else:
+                    prepared = rff_prepare_samples(rff, lo, hi, P, seed=seed)
+                    fg.wait_stream(grid_stream)
+                    for t in grid_tensors():
+                        t.record_stream(fg)
                 lib.ppbo_set_tuning(14, OVERLAP_RESERVED_SMS if warm else OVERLAP_RESERVED_SMS_COLD)
                 try:
-                    fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=prepared)
+                    fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=prepared, covariance=weight_covariance,
+                                                 transformed=transformed)
                 finally:
                     lib.ppbo_set_tuning(14, 0)
                 mark("sampling")
@@ -664,7 +773,7 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
             t.record_stream(main)
         if fg is not main:
             main.wait_stream(fg)
-            for t in (rff.omega_map, rff.hess_diag, rff.Phi_X, fmax):
+            for t in (rff.omega_map, rff.hess_diag, rff.Phi_X, fmax) + ((rff.L,) if full else ()):
                 t.record_stream(main)
         mark("gp_tail")                        # what is left of the GP fit + mu* after the contraction has finished
         sums = rff_reduce(fmax, mustar, B, shard)
@@ -686,8 +795,9 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
             torch.cuda.set_device(dev)
             with torch.cuda.stream(side):
                 fit = fit_rff()
-                # the draws and their digit planes need this fit only: done here, behind the GP fit
-                return fit, rff_prepare_samples(fit, lo, hi, P, seed=seed)
+                # the draws and their digit planes need this fit only: done here, behind the GP fit (the standard normals of the
+                # full covariance are already on the grid stream)
+                return fit, (normals if full else rff_prepare_samples(fit, lo, hi, P, seed=seed))
         fut = _background_worker().submit(weight_space_fit)
         try:
             with torch.cuda.stream(gp_stream):
@@ -703,7 +813,8 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
                 t.record_stream(main)
         main.wait_stream(side)
         for t in (rff.omega_map, rff.hess_diag, rff.Phi_X) + ((prepared.planes, prepared.scale) if isinstance(prepared, SlicedSamples)
-                                                              else ((prepared,) if prepared is not None else ())):
+                                                              else ((prepared,) if prepared is not None else ())) + \
+                ((rff.L,) if full else ()):
             t.record_stream(main)
         mark("rff_fit")                        # what is left of the weight-space fit after the GP fit has finished
     elif shard.world > 1 and CONCURRENT_FITS:
@@ -712,12 +823,16 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
         # rank 0 after its GP fit; when mu* is known only the reduction and the all-reduce of 3 B doubles are left.
         pack_rff, mu_t = pack[:2 * Fdim], pack[2 * Fdim:]
         fmax = None
+        Lbuf = ops.rff_hessian_factor_buffer(Fdim, dev) if full and shard.rank != rff_rank else None
         if shard.rank == 0:
             bstream = _side_stream(dev, tag="bcast")     # rank 0 joins the first broadcast off its critical path
             bstream.wait_stream(main)
             pack.record_stream(bstream)
             with torch.cuda.stream(bstream):
                 shard.broadcast(pack_rff, src=rff_rank)
+                if full:
+                    Lbuf.record_stream(bstream)
+                    shard.broadcast(Lbuf, src=rff_rank)
             gp = fit_gp()
             mark("gp_fit")
             main.wait_stream(bstream)
@@ -727,14 +842,17 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
                 mark("rff_fit")
                 pack_rff[:Fdim].copy_(rff.omega_map)
                 pack_rff[Fdim:].copy_(rff.hess_diag)
+                Lbuf = rff.L
             shard.broadcast(pack_rff, src=rff_rank)
+            if full:
+                shard.broadcast(Lbuf, src=rff_rank)
             mark("rff_received")
         if rff is None:
             rff = RFFFit()
             rff.W, rff.b, rff.sigma_f, rff.Phi_X, rff.stats = W, b, float(theta[2]), None, None
-        rff.omega_map, rff.hess_diag = pack_rff[:Fdim], pack_rff[Fdim:]
+        rff.omega_map, rff.hess_diag, rff.L = pack_rff[:Fdim], pack_rff[Fdim:], Lbuf
         if shard.rank != 0 and hi > lo:
-            fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed)
+            fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=normals, covariance=weight_covariance)
             mark("sampling")
         if shard_mustar:
             mustar = mu_star(gp, cand)
@@ -747,9 +865,9 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
         if shard.rank == 0 and hi > lo:
             if grid_stream is not main:
                 main.wait_stream(grid_stream)
-                for t in ((PhiT.PhiT, PhiT.planes, PhiT.scale) if isinstance(PhiT, SlicedGrids) else (PhiT,)):
+                for t in grid_tensors():
                     t.record_stream(main)
-            fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed)
+            fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=normals, covariance=weight_covariance)
             mark("sampling")
         sums = rff_reduce(fmax, mu_t, B, shard)
         mark("acquisition")
@@ -775,17 +893,21 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     else:
         shard.broadcast(pack[:2 * Fdim], src=rff_rank)
         shard.broadcast(pack[2 * Fdim:], src=0)
+    Lbuf = None
+    if full:
+        Lbuf = rff.L if shard.rank == rff_rank else ops.rff_hessian_factor_buffer(Fdim, dev)
+        shard.broadcast(Lbuf, src=rff_rank)
+        prepared = normals
     if rff is None:
         rff = RFFFit()
         rff.W, rff.b, rff.sigma_f, rff.Phi_X, rff.stats = W, b, float(theta[2]), None, None
-    rff.omega_map, rff.hess_diag = pack[:Fdim], pack[Fdim:2 * Fdim]
+    rff.omega_map, rff.hess_diag, rff.L = pack[:Fdim], pack[Fdim:2 * Fdim], Lbuf
     if grid_stream is not main:
         main.wait_stream(grid_stream)
-        if PhiT is not None:
-            for t in ((PhiT.PhiT, PhiT.planes, PhiT.scale) if isinstance(PhiT, SlicedGrids) else (PhiT,)):
-                t.record_stream(main)
+        for t in grid_tensors():
+            t.record_stream(main)
     sums, fmax, arg = rff_acquisition(rff, PhiT, S, pack[2 * Fdim:], shard=shard, seed=seed, bounds=(lo, hi), prepared=prepared,
-                                      n_grids=B)
+                                      n_grids=B, covariance=weight_covariance)
     mark("acquisition")
     if state is not None:
         state.Q = Q

@@ -657,6 +657,43 @@ def rff_refactor(Phi_X, Q, m, sigma, omega, factor_cache):
                                         _stream()), "ppbo_rff_refactor")
 
 
+def rff_hessian_factor_buffer(F, dev):
+    """flat buffer for rff_hessian_factor: the F x F factor followed by the inverted 128-blocks its solves read"""
+    return torch.empty(_lib.load().ppbo_rff_hessian_factor_doubles(F, F), dtype=F64, device=dev)
+
+
+def hessian_factor_views(Lbuf, F):
+    """(L [F x F] view, the solve workspace behind it) of a rff_hessian_factor buffer, as potrf_lower returns them"""
+    return Lbuf[:F * F].view(F, F), Lbuf[F * F:]
+
+
+def rff_hessian_factor(Phi_X, Q, m, sigma, omega, out, sync=True):
+    """Cholesky factor of the exact weight-space Hessian I + Psi' diag(a) Psi (signed a at omega) into `out`
+    (rff_hessian_factor_buffer); returns info (0, or the first non-positive pivot; sync=False: no host synchronisation, 0)"""
+    lib = _lib.load()
+    F = Phi_X.shape[0]
+    wbytes = lib.ppbo_rff_hessian_factor_workspace_bytes(F, Q, m)
+    ws = _scratch("rff_hessian", wbytes, Phi_X.device)
+    info = ctypes.c_int(0)
+    return check(lib.ppbo_rff_hessian_factor(_p(Phi_X), Phi_X.stride(0), F, Q, m, float(sigma), _p(omega), _p(out), F, _p(ws), wbytes,
+                                             ctypes.byref(info) if sync else None, _stream()), "ppbo_rff_hessian_factor")
+
+
+def rff_sample_omega_full(omega_map, Lbuf, S, Z=None, seed=0, stream_id=0, sample0=0):
+    """Omega [S,F] ~ N(omega_map, H^-1) with H = L L' from rff_hessian_factor: omega_map + Z L^-1 (Z injected or Philox)"""
+    lib = _lib.load()
+    Fdim = omega_map.shape[0]
+    Om = torch.empty((S, Fdim), dtype=F64, device=omega_map.device)
+    for s0 in range(0, S, 65535):
+        n = min(65535, S - s0)
+        wbytes = lib.ppbo_rff_sample_omega_full_workspace_bytes(n, Fdim)
+        ws = _scratch("rff_sample_full", wbytes, omega_map.device)
+        check(lib.ppbo_rff_sample_omega_full(_p(omega_map), _p(Lbuf), Fdim, _p(None if Z is None else Z[s0:s0 + n]),
+                                             Z.stride(0) if Z is not None else 0, int(seed), int(stream_id), int(sample0) + s0, n, Fdim,
+                                             _p(Om[s0:s0 + n]), Fdim, _p(ws), wbytes, _stream()), "ppbo_rff_sample_omega_full")
+    return Om
+
+
 def rff_eval_argmax(Omega, PhiT_grid, want_full=False):
     """Omega [S,F]; PhiT_grid [B,P,F] -> fmax [B,S], arg [B,S], optional dense Fs [B,S,P]"""
     S, F = Omega.shape
@@ -699,8 +736,20 @@ def ozaki_sample_slice(omega_map, hess_diag, S, seed=0, stream_id=0, sample0=0, 
     return planes, scale
 
 
-def ozaki_rowmax(ap, asc, S, bp, bsc, P, B, F, slices, fmax=None, arg=None, want_full=False, err=None):
-    """fused INT8 GEMM + per-sample max / first arg-max from digit planes (ppbo_ozaki_rowmax)"""
+def ozaki_normal_slice(S, Fdim, dev, seed=0, stream_id=0, sample0=0, slices=6):
+    """(digit planes, row scales) of the standard normals z[s][f] = Philox number (sample0 + s) F + f (ppbo_ozaki_normal_slice)"""
+    lib = _lib.load()
+    tr = lib.ppbo_ozaki_tile_rows(0)
+    planes = torch.empty(lib.ppbo_ozaki_plane_bytes(S, Fdim, tr, 1, slices), dtype=torch.int8, device=dev)
+    scale = torch.empty(lib.ppbo_ozaki_scale_doubles(S, tr, 1), dtype=F64, device=dev)
+    check(lib.ppbo_ozaki_normal_slice(int(seed), int(stream_id), int(sample0), S, Fdim, slices, _p(scale), _p(planes), _stream()),
+          "ppbo_ozaki_normal_slice")
+    return planes, scale
+
+
+def ozaki_rowmax(ap, asc, S, bp, bsc, P, B, F, slices, fmax=None, arg=None, want_full=False, err=None, bias=None):
+    """fused INT8 GEMM + per-sample max / first arg-max from digit planes (ppbo_ozaki_rowmax); bias [B, P]: max over
+    bias[b][p] + product (ppbo_ozaki_rowmax_bias)"""
     lib = _lib.load()
     dev = ap.device
     fmax = torch.empty((B, S), dtype=F64, device=dev) if fmax is None else fmax
@@ -708,8 +757,14 @@ def ozaki_rowmax(ap, asc, S, bp, bsc, P, B, F, slices, fmax=None, arg=None, want
     full = torch.empty((B, S, P), dtype=F64, device=dev) if want_full else None
     wbytes = lib.ppbo_ozaki_rowmax_workspace_bytes(S, P, B)
     ws = _scratch("ozaki_rowmax", wbytes, dev) if wbytes > 0 else None
-    check(lib.ppbo_ozaki_rowmax(_p(ap), _p(asc), S, _p(bp), _p(bsc), P, B, F, slices, _p(fmax), _p(arg), _p(full), _p(ws), wbytes,
-                                _p(err), _stream()), "ppbo_ozaki_rowmax")
+    if bias is None:
+        check(lib.ppbo_ozaki_rowmax(_p(ap), _p(asc), S, _p(bp), _p(bsc), P, B, F, slices, _p(fmax), _p(arg), _p(full), _p(ws), wbytes,
+                                    _p(err), _stream()), "ppbo_ozaki_rowmax")
+    else:
+        if tuple(bias.shape) != (B, P) or not bias.is_contiguous():
+            raise PPBOError("bias must be a contiguous [B, P] tensor")
+        check(lib.ppbo_ozaki_rowmax_bias(_p(ap), _p(asc), S, _p(bp), _p(bsc), _p(bias), P, B, F, slices, _p(fmax), _p(arg), _p(full),
+                                         _p(ws), wbytes, _p(err), _stream()), "ppbo_ozaki_rowmax_bias")
     return fmax, arg, full
 
 

@@ -27,6 +27,17 @@ from ppbo_b200 import iteration as _it  # noqa: E402
 from ppbo_b200.spectral import draw_rff_basis  # noqa: E402
 
 
+def legacy_mvn_draw(mean, cov, n, rng=np.random):
+    """n draws of numpy's legacy multivariate_normal(mean, cov) for a dense covariance, computed as numpy computes them: n F
+    standard normals from `rng` in row order, times the SVD factor sqrt(s) V, plus the mean (same values, same generator state)."""
+    mean = np.asarray(mean, dtype=np.float64)
+    x = rng.standard_normal((n, mean.shape[0]))
+    (_, s, v) = np.linalg.svd(cov)
+    x = np.dot(x, np.sqrt(s)[:, None] * v)
+    x += mean
+    return x
+
+
 class Hsampler:
     def __init__(self, gp_model, nFeatures=1000):
         self.nFeatures = nFeatures
@@ -45,6 +56,9 @@ class Hsampler:
         self.omega_MAP = None
         self.covariance = None
         self.covariance_inv = None
+        # Laplace covariance of the weight posterior: "diag" = the reference's 1 / -hess_diag; "full" = the inverse of the exact
+        # Hessian I + Psi' diag(a) Psi (opt-in addition; iteration.WEIGHT_COVARIANCES)
+        self.covariance_form = "diag"
         self.verbose = False
         self.newton_max_iter, self.newton_tol = 100, 1e-10
         self.fit_stats = None
@@ -152,6 +166,21 @@ class Hsampler:
             _, _, hd = self._objective(self.omega_MAP, self.theta, want_hess=True)
             self._dev["hess_diag"] = hd
             self._dev["omega_MAP"] = ops.to_dev(self.omega_MAP)
+        if self.covariance_form == "full":
+            F = self.nFeatures
+            Lbuf = ops.rff_hessian_factor_buffer(F, self._dev["omega_MAP"].device)
+            info = ops.rff_hessian_factor(self._d("phi_X"), self._Q(), self.m, self.theta[0], self._dev["omega_MAP"], Lbuf)
+            if info != 0:
+                print('---!!!--- Posterior covariance matrix is not PSD ---!!!---')
+                return
+            L, ws = ops.hessian_factor_views(Lbuf, F)
+            self._dev["L"] = Lbuf
+            Lh = np.tril(L.cpu().numpy())
+            self.covariance_inv = Lh @ Lh.T
+            self.covariance = ops.potri_lower(L, ws).cpu().numpy()
+            return
+        if self.covariance_form != "diag":
+            raise ValueError("covariance_form must be 'diag' or 'full'")
         h = -self._dev["hess_diag"].cpu().numpy()
         if not np.all(h > 0):
             print('---!!!--- Posterior covariance matrix is not PSD ---!!!---')
@@ -181,6 +210,12 @@ class Hsampler:
         """n draws omega ~ N(omega_MAP, covariance).  seed=None: host RNG in reference order; seed=int: counter-based device RNG"""
         if self.covariance is None:
             raise ValueError("update_covariancematrix() first")
+        if self.covariance_form == "full":
+            if seed is None:
+                Om = ops.to_dev(legacy_mvn_draw(self.omega_MAP, self.covariance, n))
+            else:
+                Om = ops.rff_sample_omega_full(self._dev["omega_MAP"], self._dev["L"], n, seed=seed)
+            return Om if on_device else Om.cpu().numpy()
         if seed is None:
             Om = ops.rff_sample_omega(self._dev["omega_MAP"], self._dev["hess_diag"], n, Z=ops.to_dev(self._legacy_mvn_normals(n)))
         else:
@@ -202,8 +237,13 @@ class Hsampler:
         rff = _it.RFFFit()
         rff.W, rff.b, rff.sigma_f = self._d("W"), self._d("b"), float(self.theta[2])
         rff.omega_map, rff.hess_diag = self._dev["omega_MAP"], self._dev["hess_diag"]
+        if self.covariance_form == "full":
+            if "L" not in self._dev:
+                raise ValueError("update_covariancematrix() first")
+            rff.L = self._dev["L"]
         PhiT = _it.rff_grid_features(rff.W, rff.b, rff.sigma_f, ops.to_dev(np.asarray(grids, dtype=np.float64)))
-        sums, _, _ = _it.rff_acquisition(rff, PhiT, n_samples, ops.to_dev(np.array([float(mustar)])), shard=shard, seed=seed)
+        sums, _, _ = _it.rff_acquisition(rff, PhiT, n_samples, ops.to_dev(np.array([float(mustar)])), shard=shard, seed=seed,
+                                         covariance=self.covariance_form)
         return sums.cpu().numpy()
 
     # ------------------------------------------------------------------ batched maximiser (north_star piece 3; SURVEY.md 8f rank 4)
