@@ -149,7 +149,8 @@ int ppbo_gemm_nt_lower(const double* A, long long lda, const double* B, long lon
 int ppbo_gemm_nt_cfg(int cfg, const double* A, long long lda, const double* B, long long ldb, double* C, long long ldc,
                      int M, int N, int K, double alpha, double beta, void* stream);
 long long ppbo_potrf_workspace_bytes(int n);
-/* in-place lower Cholesky of the lower triangle of A[n x n] (upper triangle untouched).  info_h: host int,
+/* in-place lower Cholesky of the lower triangle of A[n x n]; the upper triangle is never read, and it is untouched outside the
+ * 128 x 128 diagonal blocks (inside them the trailing updates write whole tiles: scratch there).  info_h: host int,
  * 0 or 1-based index of the first non-positive pivot.  Replaces dpotrf under scipy.linalg.solve(assume_a='pos')
  * (src/misc.py:96-100) and under scipy's trust-exact. */
 int ppbo_potrf_lower(double* A, long long lda, int n, void* workspace, long long workspace_bytes, int* info_h,
