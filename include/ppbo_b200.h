@@ -30,7 +30,13 @@ const char* ppbo_last_error(void);
 int ppbo_device_sm_count(int dev);
 /* number of CUDA kernels this library has launched so far in this process (bench.py: gpu_launches) */
 long long ppbo_launch_count(void);
-/* tuning switches for benchmarking (key 0: tile configuration of the row-max GEMM; 0 = default) */
+/* Switches for reference paths and launch shapes; 0 is the default of every key.  Any other key returns -1.
+ *   4  column-tile groups of the INT8 contraction (> 0: that many)
+ *   8  1: panel and look-ahead GEMMs of the Cholesky through the general GEMM kernel
+ *   9  1: trailing update of the Cholesky through the general GEMM kernel (0 or 1 only)
+ *   11 1: difference-form covariance and posterior-mean kernels instead of the tensor-pipe ones
+ *   14 SMs the INT8 contraction leaves free (> 0: that many; -1: one CTA per work item)
+ *   15 grid of the symmetric mat-vec tile kernel (> 0: that many CTAs) */
 int ppbo_set_tuning(int key, int value);
 /* host-thread role for concurrent fits (no reference counterpart: the reference is single-threaded, ppbo_numerical_main.py:192);
  * background threads get lowest-priority internal streams */

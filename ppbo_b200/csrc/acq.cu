@@ -506,11 +506,11 @@ __global__ void __launch_bounds__(1024) rff_ls_scalars_kernel(const double* __re
 //   hist[2i], hist[2i+1] = (rel, S) of step i
 // scal: output of rff_ls_scalars_kernel for this step; scal[24] the likelihood sum at the current iterate (rff_eval), from which S at
 // the current iterate is recomputed every step (the iterate may have been mixed since the last accepted step).
-// anderson: the steps of this batch are mixed (rff_anderson_kernel); mixed steps are not monotone step by step, so the contraction
-// is judged over three steps (a chord step costs ~1/10 of a refactorisation: three steps must gain a factor 5).
+// The steps are mixed (rff_anderson); mixed steps are not monotone step by step, so the contraction is judged over three steps (a
+// chord step costs ~1/10 of a refactorisation: three steps must gain a factor 5).
 // Returns whether the step was taken (the same value in every thread).
 __device__ __forceinline__ bool rff_chord_decide(double* omega, const double* __restrict__ step, int F, const double* scal, int m,
-                                                 double* state, double* hist, int anderson) {
+                                                 double* state, double* hist) {
     __shared__ int accept_s;
     if (threadIdx.x == 0) {
         const double oo = scal[0], od = scal[1], dd = scal[2], max_step = scal[3], max_om = fmax(scal[4], 1e-300);
@@ -532,8 +532,7 @@ __device__ __forceinline__ bool rff_chord_decide(double* omega, const double* __
             hist[2 * n] = rel;
             hist[2 * n + 1] = S1;
             if (rel <= state[6]) state[4] = 1.0;
-            else if (anderson) { if (rel3 < 1e300 && !(rel <= 0.2 * rel3)) state[4] = 2.0; }
-            else if (!(rel <= 0.5 * prev)) state[4] = 2.0;
+            else if (rel3 < 1e300 && !(rel <= 0.2 * rel3)) state[4] = 2.0;
         }
     }
     __syncthreads();
@@ -661,8 +660,8 @@ __device__ __forceinline__ void rff_anderson(double* omega, const double* __rest
 // part writes the next reads after a barrier, through plain (coherent) loads: only step, setlik and part are read-only here.
 __global__ void __launch_bounds__(1024) rff_chord_tail_kernel(double* omega, const double* __restrict__ step, int F,
                                                               const double* __restrict__ setlik, const double* __restrict__ part,
-                                                              int Q, int m, double* scal, double* state, double* hist, int anderson,
-                                                              double* aa, double* Hh) {
+                                                              int Q, int m, double* scal, double* state, double* hist, double* aa,
+                                                              double* Hh) {
     __shared__ double red[33];
     if (state[4] != 0.0) return;               // queued step behind the one that stopped the batch
     double s = 0.0;
@@ -671,7 +670,7 @@ __global__ void __launch_bounds__(1024) rff_chord_tail_kernel(double* omega, con
     if (threadIdx.x == 0) scal[24] = s;
     rff_ls_scalars(omega, step, F, part, Q, scal);
     __syncthreads();
-    if (!rff_chord_decide(omega, step, F, scal, m, state, hist, anderson) || !anderson) return;
+    if (!rff_chord_decide(omega, step, F, scal, m, state, hist)) return;
     __syncthreads();
     rff_anderson(omega, step, F, state, aa, Hh);
 }
@@ -985,8 +984,6 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
     double* hist_d = ws.scal + 48;
     double prev_rel_h = INFINITY, rel3_h = INFINITY;
     bool first_batch = true;
-    // PPBO_RFF_ANDERSON=0: plain chord steps (diagnostics)
-    const bool anderson = !(getenv("PPBO_RFF_ANDERSON") && atoi(getenv("PPBO_RFF_ANDERSON")) == 0);
     PPBO_CUDA_CHECK(cudaMemsetAsync(ws.aa, 0, sizeof(double) * 8, st));
     for (it = 0; it < max_iter; ++it) {
         if (!refactor) {
@@ -997,7 +994,7 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
                 binv_valid = true;
             }
             double rho = (std::isfinite(prev_rel_h) && last_rel < prev_rel_h) ? last_rel / prev_rel_h : 0.2;
-            rho = std::fmin(std::fmax(rho, 0.02), anderson ? 0.7 : 0.5);
+            rho = std::fmin(std::fmax(rho, 0.02), 0.7);
             int kb = !std::isfinite(last_rel) ? 3 : (last_rel > tol) ? (int)std::ceil(std::log(tol / last_rel) / std::log(rho)) : 1;
             if (first_batch) kb = std::min(kb, 3);
             kb = std::max(1, std::min(kb, std::min(RFF_BATCH_MAX, max_iter - it)));
@@ -1011,7 +1008,7 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
                 launch_rff_fvals(Phi_X, ld, F, N, ws.step, ws.fpart, ws.dfv, ws.fv_count, st, skip);
                 if ((rc = launch_linesearch_lik(ws.fvals, ws.dfv, Q, m, sigma, part, st))) return rc;
                 PPBO_CL rff_chord_tail_kernel<<<1, 1024, 0, st>>>(omega_map, ws.step, F, ws.setlik, part, Q, m, ws.scal, state_d, hist_d,
-                                                                 anderson ? 1 : 0, ws.aa, ws.aaH);
+                                                                 ws.aa, ws.aaH);
             }
             PPBO_LAUNCH_CHECK();
             PPBO_CUDA_CHECK(readback().add(state_h, state_d, sizeof(state_h), st));
@@ -1028,7 +1025,7 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
                 rel3_h = state_h[3];
             }
             // S after the last accepted step; stale once that step's result has been mixed (every accepted step but a converging one)
-            S_cur = (stop == 1 || !anderson) ? (taken > 0 ? state_h[0] : S_cur) : NAN;
+            S_cur = stop == 1 ? (taken > 0 ? state_h[0] : S_cur) : NAN;
             it += taken;
             if (stop == 1) break;
             if (stop == 2 || stop == 3) refactor = true;

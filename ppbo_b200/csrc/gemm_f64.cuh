@@ -134,12 +134,6 @@ struct StoreEpilogue {
 template <class Cfg>
 __global__ void __launch_bounds__(Cfg::THREADS, Cfg::MINB) gemm_nt_store_kernel(GemmOperands g, StoreEpilogue ep) {
     extern __shared__ __align__(16) double smem[];
-#ifdef PPBO_PDL
-    // Programmatic dependent launch (an experiment on the Cholesky critical path, tuning key 7; measured slower and compiled out):
-    // let the next kernel of the stream become resident now and hold this one until its predecessor has completed and flushed.
-    asm volatile("griddepcontrol.launch_dependents;");
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
     int tm, tn;
     if (ep.lower_only) {
         // tiles that touch the lower triangle, row-tile major: row tile ti owns column tiles 0 .. R (ti + 1) - 1, R = BM / BN

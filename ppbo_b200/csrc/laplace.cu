@@ -20,7 +20,6 @@
 
 namespace ppbo {
 
-extern int g_tuning[16];
 int diffspace_gram(const double* S, long long lds, int Q, int m, double* G, long long ldg, cudaStream_t st);
 int newton_matrix(const double* G, long long ldg, int M, const double* sa, double* out, long long ldo, cudaStream_t st);
 
@@ -33,14 +32,14 @@ __device__ __forceinline__ double Phi_tilde(double x) {           // Phi(x / sqr
 
 // One warp per comparison set.  Outputs are optional (nullptr to skip).
 //   set_lik[q] = sum_j Phi~(Delta_qj)        beta[N]        arrow[Qm] (signed a)       sa[Qm] = sqrt(max(a,0))
-//   bvec[N]    = B a+ B^T f + beta           (Newton right-hand side)
-//   ap_fixed  : when given, bvec is built with these (stale) a+ instead of the current ones -- chord steps that reuse a factor
+//   bvec[N]    = B a+ B^T f + beta           (Newton right-hand side)      ap_out[Qm] = a+
+//   ap_fixed  : when given, bvec is built with these a+ instead of the current ones.  No caller passes it, but without the
+//               parameter ptxas spills 32 bytes in this kernel instead of 12.
 __global__ void __launch_bounds__(256) lik_terms_kernel(const double* __restrict__ f, int Q, int m, double sigma,
                                                         double* __restrict__ set_lik, double* __restrict__ beta,
                                                         double* __restrict__ arrow, double* __restrict__ sa,
                                                         double* __restrict__ bvec, const double* __restrict__ ap_fixed = nullptr,
-                                                        double* __restrict__ ap_out = nullptr, const double* __restrict__ skip = nullptr) {
-    if (skip && *skip != 0.0) return;          // queued chord step behind the one that stopped the batch
+                                                        double* __restrict__ ap_out = nullptr) {
     const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (q >= Q) return;
     const long long base = (long long)q * (m + 1);
@@ -95,8 +94,7 @@ __global__ void __launch_bounds__(1024) dot_kernel(const double* __restrict__ x,
 
 // t[u] = sa[u] * (v[r(u)] - v[w(u)])                       (a+^1/2 B^T v)
 __global__ void diff_scale_kernel(const double* __restrict__ v, const double* __restrict__ sa, int Q, int m,
-                                  double* __restrict__ t, const double* __restrict__ skip = nullptr) {
-    if (skip && *skip != 0.0) return;
+                                  double* __restrict__ t) {
     const int u = blockIdx.x * blockDim.x + threadIdx.x;
     if (u >= Q * m) return;
     const int q = u / m, j = u % m;
@@ -107,9 +105,7 @@ __global__ void diff_scale_kernel(const double* __restrict__ v, const double* __
 // alpha_new = b - B (sa .* y);  dalpha = alpha_new - alpha  (one warp per set)
 __global__ void __launch_bounds__(256) alpha_update_kernel(const double* __restrict__ bvec, const double* __restrict__ sa,
                                                            const double* __restrict__ y, const double* __restrict__ alpha,
-                                                           int Q, int m, double* __restrict__ dalpha,
-                                                           const double* __restrict__ skip = nullptr) {
-    if (skip && *skip != 0.0) return;
+                                                           int Q, int m, double* __restrict__ dalpha) {
     const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (q >= Q) return;
     const long long base = (long long)q * (m + 1);
@@ -186,34 +182,6 @@ __global__ void axpy2_kernel(double* __restrict__ alpha, const double* __restric
     if (i < N) {
         alpha[i] += step * dalpha[i];
         f[i] += step * df[i];
-    }
-}
-
-// Likelihood sums of a queued chord step at its step length omega = state[7]:  part[q] = sum_j Phi~(Delta_qj(f + omega df)) and,
-// when part0 is given, the sums at the current iterate f (T there is then recomputed every step instead of being carried)
-__global__ void __launch_bounds__(256) chord_lik_kernel(const double* __restrict__ f, const double* __restrict__ df, int Q, int m,
-                                                        double sigma, const double* __restrict__ state, double* __restrict__ part,
-                                                        double* __restrict__ part0) {
-    if (state[4] != 0.0) return;
-    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (q >= Q) return;
-    const double step = state[7];
-    const long long base = (long long)q * (m + 1);
-    const double fw0 = f[base], fw = fw0 + step * df[base];
-    const double inv_s = 1.0 / sigma;
-    double s = 0.0, s0 = 0.0;
-    for (int j = lane; j < m; j += 32) {
-        const double fj = f[base + 1 + j];
-        s += Phi_tilde((fj + step * df[base + 1 + j] - fw) * inv_s);
-        if (part0) s0 += Phi_tilde((fj - fw0) * inv_s);
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        s += __shfl_xor_sync(0xffffffffu, s, o);
-        s0 += __shfl_xor_sync(0xffffffffu, s0, o);
-    }
-    if (lane == 0) {
-        part[q] = s;
-        if (part0) part0[q] = s0;
     }
 }
 
@@ -1169,7 +1137,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
     // is kept and only the right-hand side is refreshed (chord steps: same fixed point Sigma^-1 f = beta(f), linear
     // convergence at the rate of the relative change of a+; a chord step costs ~1/6 of a factorisation at Qm = 5000, so it
     // is kept as long as it at least halves the step).
-    double CHORD_REL = getenv("PPBO_CHORD_REL") ? atof(getenv("PPBO_CHORD_REL")) : 0.25;   // env override: diagnostics only
+    constexpr double CHORD_REL = 0.25;
     const bool trace = getenv("PPBO_TRACE") != nullptr;
     bool refactor = true, converged = false;
     // Cold start f = 0: every difference is 0, so a = -Delta phi~(Delta) / (2 m sigma^2) = 0 and the Newton matrix
@@ -1179,23 +1147,15 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
     // solves), which makes every later solve with that factor ~3x cheaper than the 40-link chained solve
     bool binv_valid = false;
     bool first_chord_batch = true;
-    // tuning: PPBO_CHORD_EXTRAPOLATE=0 switches the Aitken step lengths off (diagnostics)
-    const bool chord_extrapolate = !(getenv("PPBO_CHORD_EXTRAPOLATE") && atoi(getenv("PPBO_CHORD_EXTRAPOLATE")) == 0);
     double chord_omega = 1.0, chord_ratio = 0.0, chord_wait = 0.0;
-    // tuning key 13: Anderson acceleration of the chord iteration (1 = on, 2 = on and enter the chord phase after the FIRST Newton
-    // factorisation of a cold fit); PPBO_ANDERSON overrides (diagnostics)
-    int anderson_mode = g_tuning[13] == 0 ? 2 : g_tuning[13] - 1;        // key 13: 0 default (= 2), 1 off, 2 after every factor, 3 = 2
-    if (getenv("PPBO_ANDERSON")) anderson_mode = atoi(getenv("PPBO_ANDERSON"));
-    // mode 2 (default): a fit that starts without a usable factor enters the chord phase after its FIRST factorisation (relative
-    // step <= 0.6 instead of 0.25) and mixes the chord steps there; if three mixed steps do not halve the residual the fit pays for
-    // the second factorisation and continues exactly like the unaccelerated iteration.  Warm (bordered) fits are not mixed: the
-    // border's Newton steps change the map from step to step and the Aitken step lengths do better there (measured).
+    // Anderson acceleration of the chord iteration: a fit that starts without a usable factor enters the chord phase after its
+    // FIRST factorisation (relative step <= 0.6 instead of 0.25) and mixes the chord steps there; if three mixed steps do not halve
+    // the residual the fit pays for the second factorisation and continues exactly like the unaccelerated iteration.  Warm
+    // (bordered) fits are not mixed: the border's Newton steps change the map from step to step and the Aitken step lengths do
+    // better there (measured).
     bool aa_failed = false;
     double rel3_h = INFINITY;
-    // PPBO_CHORD_SPACE=alpha: chord steps on (alpha, f) with two Sigma mat-vecs per step (the formulation of the first half of
-    // round 2; diagnostics)
-    const bool diff_space = !(getenv("PPBO_CHORD_SPACE") && getenv("PPBO_CHORD_SPACE")[0] == 'a');
-    auto aa_now = [&]() { return (anderson_mode == 1) || (anderson_mode >= 2 && !warm_factor && n_factor == 1 && !aa_failed); };
+    auto aa_now = [&]() { return !warm_factor && n_factor == 1 && !aa_failed; };
     PPBO_CUDA_CHECK(cudaMemsetAsync(ws.aa, 0, sizeof(double) * 8, st));
     bool factor_current = false;         // Lfac is the factor for the coefficients in ws.sa / ws.ap
     double warm_first_rel = NAN;
@@ -1250,12 +1210,6 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
         refactor = false;
         if (trace) fprintf(stderr, "[ppbo_laplace_fit] warm start: factor of %d rows, border %d, T %.12g\n", M_old, nb, T_cur);
     }
-    // coefficients of the border rows at the current iterate (their own Newton step inside every chord step)
-    auto refresh_border = [&](const double* skip) {
-        const int Qn = nb / m, Qo = M_old / m;
-        PPBO_CL lik_terms_kernel<<<ceil_div(Qn, 8), 256, 0, st>>>(f_map + (long long)Qo * (m + 1), Qn, m, sigma, nullptr, nullptr, nullptr,
-                                                                    ws.sa + M_old, nullptr, nullptr, ws.ap + M_old, skip);
-    };
     // (I + s G s) y = t in place with the factor in Lfac (+ border)
     auto chord_solve = [&](const double* skip) -> int {
         int r_;
@@ -1300,42 +1254,27 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
             double hist_h[2 * CHORD_BATCH_MAX];
             PPBO_CUDA_CHECK(cudaMemcpyAsync(ws.state, state_h, sizeof(state_h), cudaMemcpyHostToDevice, st));
             const double* skip = ws.state + 4;               // non-zero once a step of the batch has stopped it
-            if (diff_space) {
-                // ---- the batch in difference space (see to_diff_kernel): gamma, d, c, dgamma, dd live in the N-vectors of the
-                // alpha-space step, which are idle here
-                double *gam = ws.bvec, *dv = ws.Sb, *cv = ws.dalpha, *dgam = ws.df, *ddv = ws.arrow_tmp;
-                const double thr = 1e-3 * 0.121 / (m * sigma * sigma);       // 1e-3 of the largest possible coefficient
-                if (!in_diff) {              // (consecutive batches stay in difference space: nothing else touches these vectors)
-                    PPBO_CL to_diff_kernel<<<ceil_div(M, 256), 256, 0, st>>>(f_map, alpha, Q, m, dv, gam);
-                    in_diff = true;
-                }
-                for (int i = 0; i < kb; ++i) {
-                    if (bordered)
-                        PPBO_CL dborder_coeff_kernel<<<ceil_div(nb, 64), 64, 0, st>>>(dv + M_old, nb, sigma, m, ws.sa + M_old, ws.ap + M_old, skip);
-                    PPBO_CL dchord_rhs_kernel<<<ceil_div(M, 256), 256, 0, st>>>(dv, ws.ap, M, sigma, m, cv, skip);
-                    if ((rc = symv_lower(G, ldg, M, cv, ws.t, ws.sym, st, skip))) return rc;
-                    PPBO_CL dchord_scale_kernel<<<ceil_div(M, 256), 256, 0, st>>>(ws.t, ws.sa, M, skip);
-                    if ((rc = chord_solve(skip))) return rc;
-                    PPBO_CL dchord_update_kernel<<<ceil_div(M, 256), 256, 0, st>>>(cv, ws.sa, ws.ap, ws.t, gam, dv, M, thr, dgam, ddv, skip);
-                    PPBO_CL dchord_rows_kernel<<<M, 256, 0, st>>>(G, ldg, gam, dgam, ws.ap, dv, M, thr, ddv, skip);
-                    PPBO_CL dchord_lik_kernel<<<set_blocks, 256, 0, st>>>(dv, ddv, Q, m, sigma, ws.state, ws.set_part, anderson ? ws.part0 : nullptr);
-                    PPBO_CL chord_decide_kernel<<<1, 1024, 0, st>>>(gam, dgam, dv, ddv, M, ws.set_part, Q, m, ws.state, ws.hist,
-                                                                      (chord_extrapolate && !anderson) ? 1 : 0, anderson ? ws.part0 : nullptr);
-                    if (anderson && (rc = launch_chord_anderson(gam, dv, ddv, M, ws.state, ws.aa, ws.aaH, st))) return rc;
-                }
-            } else
+            // ---- the batch in difference space (see to_diff_kernel): gamma, d, c, dgamma, dd live in the N-vectors of the
+            // alpha-space Newton step, which are idle here
+            double *gam = ws.bvec, *dv = ws.Sb, *cv = ws.dalpha, *dgam = ws.df, *ddv = ws.arrow_tmp;
+            const double thr = 1e-3 * 0.121 / (m * sigma * sigma);       // 1e-3 of the largest possible coefficient
+            if (!in_diff) {              // (consecutive batches stay in difference space: nothing else touches these vectors)
+                PPBO_CL to_diff_kernel<<<ceil_div(M, 256), 256, 0, st>>>(f_map, alpha, Q, m, dv, gam);
+                in_diff = true;
+            }
             for (int i = 0; i < kb; ++i) {
-                if (bordered) refresh_border(skip);
-                PPBO_CL lik_terms_kernel<<<set_blocks, 256, 0, st>>>(f_map, Q, m, sigma, nullptr, nullptr, nullptr, nullptr, ws.bvec, ws.ap, nullptr, skip);
-                if ((rc = symv_lower(Sigma, lds, N, ws.bvec, ws.Sb, ws.sym, st, skip))) return rc;
-                PPBO_CL diff_scale_kernel<<<ceil_div(M, 256), 256, 0, st>>>(ws.Sb, ws.sa, Q, m, ws.t, skip);
+                if (bordered)
+                    PPBO_CL dborder_coeff_kernel<<<ceil_div(nb, 64), 64, 0, st>>>(dv + M_old, nb, sigma, m, ws.sa + M_old, ws.ap + M_old, skip);
+                PPBO_CL dchord_rhs_kernel<<<ceil_div(M, 256), 256, 0, st>>>(dv, ws.ap, M, sigma, m, cv, skip);
+                if ((rc = symv_lower(G, ldg, M, cv, ws.t, ws.sym, st, skip))) return rc;
+                PPBO_CL dchord_scale_kernel<<<ceil_div(M, 256), 256, 0, st>>>(ws.t, ws.sa, M, skip);
                 if ((rc = chord_solve(skip))) return rc;
-                PPBO_CL alpha_update_kernel<<<set_blocks, 256, 0, st>>>(ws.bvec, ws.sa, ws.t, alpha, Q, m, ws.dalpha, skip);
-                if ((rc = symv_lower(Sigma, lds, N, ws.dalpha, ws.df, ws.sym, st, skip))) return rc;
-                PPBO_CL chord_lik_kernel<<<set_blocks, 256, 0, st>>>(f_map, ws.df, Q, m, sigma, ws.state, ws.set_part, anderson ? ws.part0 : nullptr);
-                PPBO_CL chord_decide_kernel<<<1, 1024, 0, st>>>(alpha, ws.dalpha, f_map, ws.df, N, ws.set_part, Q, m, ws.state, ws.hist,
-                                                                  (chord_extrapolate && !anderson) ? 1 : 0, anderson ? ws.part0 : nullptr);
-                if (anderson && (rc = launch_chord_anderson(alpha, f_map, ws.df, N, ws.state, ws.aa, ws.aaH, st))) return rc;
+                PPBO_CL dchord_update_kernel<<<ceil_div(M, 256), 256, 0, st>>>(cv, ws.sa, ws.ap, ws.t, gam, dv, M, thr, dgam, ddv, skip);
+                PPBO_CL dchord_rows_kernel<<<M, 256, 0, st>>>(G, ldg, gam, dgam, ws.ap, dv, M, thr, ddv, skip);
+                PPBO_CL dchord_lik_kernel<<<set_blocks, 256, 0, st>>>(dv, ddv, Q, m, sigma, ws.state, ws.set_part, anderson ? ws.part0 : nullptr);
+                PPBO_CL chord_decide_kernel<<<1, 1024, 0, st>>>(gam, dgam, dv, ddv, M, ws.set_part, Q, m, ws.state, ws.hist,
+                                                                  !anderson, anderson ? ws.part0 : nullptr);
+                if (anderson && (rc = launch_chord_anderson(gam, dv, ddv, M, ws.state, ws.aa, ws.aaH, st))) return rc;
             }
             PPBO_LAUNCH_CHECK();
             PPBO_CUDA_CHECK(readback().add(state_h, ws.state, sizeof(state_h), st));
@@ -1388,7 +1327,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
             // From the second factorisation on -- and for the first one of a cold fit, which enters the Anderson-mixed chord phase
             // with it -- the factor is very likely reused by chord steps, which need the 1024-block inverses anyway: build them now
             // and let this solve use them too (0.13 ms against 0.48 ms for the chained solve).
-            if ((n_factor >= 2 || (anderson_mode >= 2 && !warm_factor && !aa_failed)) && M >= 2048 && !binv_valid) {
+            if ((n_factor >= 2 || (!warm_factor && !aa_failed)) && M >= 2048 && !binv_valid) {
                 if ((rc = blockinv_build(Lfac, ldl, M, Mdinv, ws.binv, st))) return rc;
                 binv_valid = true;
             }
@@ -1444,7 +1383,7 @@ extern "C" int ppbo_laplace_fit(const double* Sigma, long long lds, int Q, int m
         ++it;
         if (step == 1.0 && last_rel <= tol) { converged = true; break; }
         // chord steps once the Newton iteration is in its contraction region and a factor exists to reuse
-        const double chord_rel = (anderson_mode >= 2 && !warm_factor && n_factor == 1 && !aa_failed && !getenv("PPBO_CHORD_REL")) ? 0.6 : CHORD_REL;
+        const double chord_rel = (!warm_factor && n_factor == 1 && !aa_failed) ? 0.6 : CHORD_REL;
         refactor = !(step == 1.0 && last_rel <= chord_rel) || identity_factor;
     }
     if ((rc = leave_diff())) return rc;

@@ -317,19 +317,15 @@ __device__ __forceinline__ uint64_t umma_desc_advance(uint64_t desc, uint32_t by
     return (desc & 0xFFFFFFFF00000000ull) | (uint64_t)((uint32_t)desc + (bytes >> 4));
 }
 
-// TS: the A digit planes of a stage are copied once from shared memory into TMEM (tcgen05.cp) and every MMA reads A from
-// there; only the (narrow) B planes are re-read from shared memory.  With both operands in shared memory an M=128, N=64, K=32
-// MMA fetches 6 KB per 32 issue cycles = 1.5x the 128 B/clk shared-memory port: the ncu capture of that variant shows the
-// tensor-core shared-memory wavefronts as the top utilisation (61 %) with the tensor pipe at 27 %.
-template <int KS, int BN, bool TS = true>
+// Both operands are read from shared memory.  Copying the A digit planes of a stage into TMEM (tcgen05.cp) so that only the
+// narrow B planes are re-read was measured slower (13.0 ms against 9.8): the copies serialise with the MMAs in the tensor pipe.
+template <int KS, int BN>
 struct Cfg {
     static constexpr int A_PLANE = BM * KB, B_PLANE = BN * KB;
     static constexpr int A_STAGE = KS * A_PLANE, B_STAGE = KS * B_PLANE;
     static constexpr int STAGE_BYTES = A_STAGE + B_STAGE;
     static constexpr int STAGES = (3 * STAGE_BYTES + 256 + MERGE_BYTES <= 232448) ? 3 : 2;
-    static constexpr int A_TMEM_COLS = TS ? KS * (KB / 4) : 0;      // KB bytes per lane and plane, 4 per column
-    static constexpr int TMEM_A0 = KS * BN;                         // first column of the A planes
-    static constexpr int TMEM_USED = KS * BN + A_TMEM_COLS;
+    static constexpr int TMEM_USED = KS * BN;
     static constexpr int TMEM_COLS = TMEM_USED <= 32 ? 32 : TMEM_USED <= 64 ? 64 : TMEM_USED <= 128 ? 128 : TMEM_USED <= 256 ? 256 : 512;
     static constexpr int SMEM = STAGES * STAGE_BYTES + 256 + MERGE_BYTES;
     static constexpr int G1 = KS < 3 ? KS : 3;               // accumulators recombined into the high INT64 word
@@ -350,12 +346,12 @@ struct Params {
     double* fmax; int* arg;                                    // [batch][S] (NG == 1) or partial results [batch][NG][S]
     double* full; long long ld_full, stride_full;              // optional dense output (tests)
     int* err;
-    int diag;      // timing experiments only (tuning key 2): bit 0 = epilogue skips the TMEM reads, bit 1 = producer skips the copies
 };
 // The biased instantiations take the offsets in a derived parameter block: a field added to Params itself changes the code ptxas
 // emits for the unbiased kernels (same arithmetic, other registers and layout).
+// (bias at offset 128 rather than right behind Params at 120: there ptxas spills 12 bytes in the KS = 7 kernel)
 struct BiasParams : Params {
-    const double* bias;                                        // [batch][P] column offsets
+    alignas(16) const double* bias;                            // [batch][P] column offsets
 };
 template <bool BIAS> struct ParamsOf { using T = Params; };
 template <> struct ParamsOf<true> { using T = BiasParams; };
@@ -427,9 +423,9 @@ __device__ __forceinline__ void epi_columns(const uint32_t (&acc)[KS][NC], const
     }
 }
 
-template <int KS, int BN, bool TS, bool BIAS = false>
+template <int KS, int BN, bool BIAS = false>
 __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename ParamsOf<BIAS>::T p) {
-    using C = Cfg<KS, BN, TS>;
+    using C = Cfg<KS, BN>;
     extern __shared__ __align__(1024) uint8_t smem[];
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::STAGES * C::STAGE_BYTES);
     uint64_t* full_bar = bars;
@@ -465,12 +461,6 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
     // CTAs of a row tile and the ntg column tiles of each CTA re-read them.  With NG = 1 every CTA streams its own row tile 16
     // times: 113 MB of live A planes thrash the L2 (ncu: 62 GB of DRAM reads per launch, 12 % L2 hit rate).
     const int items = p.MT * p.batch * p.NG;
-    long long clk0 = 0;
-    unsigned long long ns0 = 0;
-    if ((p.diag & 4) && threadIdx.x == 0) {
-        clk0 = clock64();
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns0));
-    }
 
     if (warp == 0) {
         // ------------------------------------------------------------------------------------- producer
@@ -484,8 +474,7 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
                 const int8_t* Bb = p.B + ((long long)b * p.NT + nt) * p.KBLK * C::B_STAGE;
                 for (int kb = 0; kb < p.KBLK; ++kb) {
                     mbar_wait(empty_bar + stage, phase ^ 1, p.err, 1);
-                    if (lane == 0 && (p.diag & 2)) mbar_arrive(full_bar + stage);
-                    if (lane == 0 && !(p.diag & 2)) {
+                    if (lane == 0) {
                         const uint32_t dst = smem_u32(smem + stage * C::STAGE_BYTES);
                         mbar_expect_tx(full_bar + stage, C::STAGE_BYTES);
                         bulk_g2s(dst, Ab + (long long)kb * C::A_STAGE, C::A_STAGE, full_bar + stage);
@@ -512,14 +501,6 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
                     if (lane == 0) {
                         const uint64_t a_desc0 = umma_desc(smem_u32(smem + stage * C::STAGE_BYTES));
                         const uint64_t b_desc0 = umma_desc_advance(a_desc0, C::A_STAGE);
-                        if (TS) {
-#pragma unroll
-                            for (int i = 0; i < KS; ++i)
-#pragma unroll
-                                for (int kk = 0; kk < KB / UMMA_K; ++kk)
-                                    tc_cp_128x256b(tmem_base + (uint32_t)(C::TMEM_A0 + (i * (KB / UMMA_K) + kk) * (UMMA_K / 4)),
-                                                   umma_desc_advance(a_desc0, i * C::A_PLANE + kk * (UMMA_K / 16) * LBO));
-                        }
                         // Digit plane A_i meets B_0 .. B_{KS-1-i}; those B planes are consecutive 8-row groups of one tall
                         // K-major matrix in shared memory and their accumulators d = i .. KS-1 are consecutive TMEM columns, so
                         // the KS - i products are ONE MMA of N = (KS - i) BN columns (cut into <= 256-column pieces).  A single
@@ -530,7 +511,6 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
 #pragma unroll
                             for (int i = 0; i < KS; ++i) {
                                 const uint64_t adesc = umma_desc_advance(a_desc0, i * C::A_PLANE + kk * (UMMA_K / 16) * LBO);
-                                const uint32_t a_tmem = tmem_base + (uint32_t)(C::TMEM_A0 + (i * (KB / UMMA_K) + kk) * (UMMA_K / 4));
                                 const int ncols = (KS - i) * BN;
                                 const int pieces = (ncols + 255) / 256;
                                 const int width = ((ncols + pieces - 1) / pieces + 15) / 16 * 16;
@@ -541,8 +521,7 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
                                     const uint32_t d_tmem = tmem_base + (uint32_t)(i * BN + c0);
                                     const uint32_t accum = (uint32_t)((kb | kk | i) != 0);
                                     const uint32_t idesc = C::IDESC_BASE | ((uint32_t)(n >> 3) << 17);
-                                    if (TS) tc_mma_i8_ts(d_tmem, a_tmem, bdesc, idesc, accum);
-                                    else tc_mma_i8(d_tmem, adesc, bdesc, idesc, accum);
+                                    tc_mma_i8(d_tmem, adesc, bdesc, idesc, accum);
                                 }
                             }
                         }
@@ -580,21 +559,19 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
                 double* full_row = (p.full && row < p.S) ? p.full + (long long)b * p.stride_full + (long long)row * p.ld_full : nullptr;
                 // 8-column chunks, double-buffered in registers: the TMEM loads of chunk k+1 are in flight while chunk k is
                 // recombined (tcgen05.wait::ld waits for every outstanding load, so the wait sits right before the next issue)
-                if (!(p.diag & 1)) {
-                    uint32_t acc[2][KS][8];
+                uint32_t acc[2][KS][8];
 #pragma unroll
-                    for (int d = 0; d < KS; ++d) tc_ld8(lane_addr + (uint32_t)(d * BN + cbase), acc[0][d]);
+                for (int d = 0; d < KS; ++d) tc_ld8(lane_addr + (uint32_t)(d * BN + cbase), acc[0][d]);
 #pragma unroll
-                    for (int k = 0; k < HC / 8; ++k) {
-                        tc_ld_wait();
-                        if (k + 1 < HC / 8) {
+                for (int k = 0; k < HC / 8; ++k) {
+                    tc_ld_wait();
+                    if (k + 1 < HC / 8) {
 #pragma unroll
-                            for (int d = 0; d < KS; ++d) tc_ld8(lane_addr + (uint32_t)(d * BN + cbase + (k + 1) * 8), acc[(k + 1) & 1][d]);
-                        }
-                        const int col0 = nt * BN + cbase + k * 8;
-                        if (checked) epi_columns<KS, C::G1, true, 8, BIAS>(acc[k & 1], bs + k * 8, col0, p.P, full_row, as2, best, best_arg, brow);
-                        else epi_columns<KS, C::G1, false, 8, BIAS>(acc[k & 1], bs + k * 8, col0, p.P, nullptr, as2, best, best_arg, brow);
+                        for (int d = 0; d < KS; ++d) tc_ld8(lane_addr + (uint32_t)(d * BN + cbase + (k + 1) * 8), acc[(k + 1) & 1][d]);
                     }
+                    const int col0 = nt * BN + cbase + k * 8;
+                    if (checked) epi_columns<KS, C::G1, true, 8, BIAS>(acc[k & 1], bs + k * 8, col0, p.P, full_row, as2, best, best_arg, brow);
+                    else epi_columns<KS, C::G1, false, 8, BIAS>(acc[k & 1], bs + k * 8, col0, p.P, nullptr, as2, best, best_arg, brow);
                 }
                 tc_fence_before();
                 __syncwarp();
@@ -624,12 +601,6 @@ __global__ void __launch_bounds__(THREADS, 1) ozaki_rowmax_kernel(const typename
     __syncthreads();
     if (warp == 1) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)C::TMEM_COLS) : "memory");
-    }
-    if ((p.diag & 4) && threadIdx.x == 0 && blockIdx.x == 0 && p.err) {      // SM clock actually sustained by this launch
-        unsigned long long ns1;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns1));
-        reinterpret_cast<long long*>(p.err)[1] = clock64() - clk0;
-        reinterpret_cast<long long*>(p.err)[2] = (long long)(ns1 - ns0);
     }
 }
 
@@ -688,13 +659,13 @@ static int slice_launch(const double* X, long long ldx, long long strideX, int r
     return PPBO_OK;
 }
 
-template <int KS, int BN, bool TS, bool BIAS = false>
+template <int KS, int BN, bool BIAS = false>
 static int rowmax_launch(const typename ParamsOf<BIAS>::T& p, cudaStream_t st) {
-    using C = Cfg<KS, BN, TS>;
+    using C = Cfg<KS, BN>;
     static std::once_flag once;
     static cudaError_t err = cudaSuccess;
     std::call_once(once, [] {
-        err = cudaFuncSetAttribute(ozaki_rowmax_kernel<KS, BN, TS, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
+        err = cudaFuncSetAttribute(ozaki_rowmax_kernel<KS, BN, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
     });
     PPBO_CUDA_CHECK(err);
     int dev = 0, sms = PPBO_SM_COUNT;
@@ -709,7 +680,7 @@ static int rowmax_launch(const typename ParamsOf<BIAS>::T& p, cudaStream_t st) {
     // collect their SMs one by one as ~120 us work items end and the GP fit stretches from 10.6 to 15.3 ms.
     const int reserve = g_tuning[14];
     const int grid = reserve < 0 ? items : min(items, max(sms - reserve, 1));
-    PPBO_CL ozaki_rowmax_kernel<KS, BN, TS, BIAS><<<grid, THREADS, C::SMEM, st>>>(p);
+    PPBO_CL ozaki_rowmax_kernel<KS, BN, BIAS><<<grid, THREADS, C::SMEM, st>>>(p);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
 }
@@ -906,35 +877,33 @@ static int ozaki_rowmax_impl(const signed char* Aplanes, const double* ascale, i
     p.KBLK = ceil_div(K, oz::KB);
     p.NG = oz::column_groups(p.NT, p.KBLK, slices);
     p.ntg = ceil_div(p.NT, p.NG);
-    // grids per block: as many as keep the block's B planes within ~48 MB of L2 (tuning key 12 overrides; 1 = the earlier order).
-    // Measured on the bench shape under sustained load (scripts/ozaki_order_sweep.py, round-robin): 1 -> 9.79 ms, 2 -> 9.77, 4 -> 9.68,
-    // 7 -> 9.83, 20 -> 10.28: the kernel is bound by the tensor pipe under the power cap, the order only moves DRAM traffic.
+    // grids per block: as many as keep the block's B planes within ~48 MB of L2 (1 = the earlier order, grid outermost).
+    // Measured on the bench shape under sustained load (round-robin): 1 -> 9.79 ms, 2 -> 9.77, 4 -> 9.68, 7 -> 9.83,
+    // 20 -> 10.28: the kernel is bound by the tensor pipe under the power cap, the order only moves DRAM traffic.
     {
         const long long grid_bytes = (long long)p.NT * p.KBLK * slices * oz::BN_DEFAULT * oz::KB;
-        int gbk = g_tuning[12] > 0 ? g_tuning[12] : (int)std::max<long long>(1, (48LL << 20) / std::max<long long>(grid_bytes, 1));
-        p.GB = std::min(std::max(gbk, 1), batch);
+        const int gbk = (int)std::max<long long>(1, (48LL << 20) / std::max<long long>(grid_bytes, 1));
+        p.GB = std::min(gbk, batch);
     }
     PPBO_REQUIRE(workspace_bytes >= ppbo_ozaki_rowmax_workspace_bytes(S, P, batch), "workspace too small");
     PPBO_REQUIRE(p.NG == 1 || workspace != nullptr, "workspace missing");
     double* pmax = reinterpret_cast<double*>(workspace);
     int* parg = reinterpret_cast<int*>(pmax + (long long)batch * p.NG * S);
     p.fmax = p.NG > 1 ? pmax : fmax; p.arg = p.NG > 1 ? parg : arg; p.full = Fs_full; p.ld_full = P; p.stride_full = (long long)S * P; p.err = err_flag;
-    p.diag = g_tuning[2];
     p.bias = bias;
     const oz::Params& p0 = p;                  // the unbiased kernels take the base block
     cudaStream_t st = (cudaStream_t)stream;
-    const bool ts = g_tuning[1] == 1;          // tuning key 1: 1 = A planes staged in TMEM (comparison variant, slower)
     int rc;
-    if (bias) {                                // (no TMEM-staged variant of the biased epilogue)
+    if (bias) {
         switch (slices) {
-            case 5: rc = oz::rowmax_launch<5, oz::BN_DEFAULT, false, true>(p, st); break;
-            case 6: rc = oz::rowmax_launch<6, oz::BN_DEFAULT, false, true>(p, st); break;
-            default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT, false, true>(p, st); break;
+            case 5: rc = oz::rowmax_launch<5, oz::BN_DEFAULT, true>(p, st); break;
+            case 6: rc = oz::rowmax_launch<6, oz::BN_DEFAULT, true>(p, st); break;
+            default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT, true>(p, st); break;
         }
     } else switch (slices) {
-        case 5: rc = ts ? oz::rowmax_launch<5, oz::BN_DEFAULT, true>(p0, st) : oz::rowmax_launch<5, oz::BN_DEFAULT, false>(p0, st); break;
-        case 6: rc = ts ? oz::rowmax_launch<6, oz::BN_DEFAULT, true>(p0, st) : oz::rowmax_launch<6, oz::BN_DEFAULT, false>(p0, st); break;
-        default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT, false>(p0, st); break;   // 7 x 64 + 7 x 16 columns exceed TMEM
+        case 5: rc = oz::rowmax_launch<5, oz::BN_DEFAULT>(p0, st); break;
+        case 6: rc = oz::rowmax_launch<6, oz::BN_DEFAULT>(p0, st); break;
+        default: rc = oz::rowmax_launch<7, oz::BN_DEFAULT>(p0, st); break;
     }
     if (rc) return rc;
     if (p.NG > 1) {

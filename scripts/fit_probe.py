@@ -1,4 +1,4 @@
-"""Laplace fit at the Ackley-20D shape with the iteration trace; PPBO_CHORD_REL / PPBO_TRACE from the environment."""
+"""Laplace fit at the Ackley-20D shape; PPBO_TRACE in the environment prints the iteration trace."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -16,7 +16,7 @@ for _ in range(5):
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record(); fit = ops.laplace_fit(Sigma, Q, m, th[0], tol=tol); b.record(); torch.cuda.synchronize()
     ts.append(a.elapsed_time(b))
-print("%s CHORD_REL=%s tol=%g: %.2f ms %s" % (name, os.environ.get("PPBO_CHORD_REL", "default"), tol, float(np.median(ts)), fit.stats))
+print("%s laplace_fit tol=%g: %.2f ms %s" % (name, tol, float(np.median(ts)), fit.stats))
 W = ops.to_dev(prob["W"]); b = ops.to_dev(prob["b"])
 Phi = ops.rff_features(W, b, X, th[2], feature_major=True)
 for _ in range(2):

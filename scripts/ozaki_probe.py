@@ -38,37 +38,10 @@ def ubench(dev):
                     N, mode, nacc, c, N // 2, 2.0 * 128 * N * 32 / c * 148 * 1.9e9 / 1e12), flush=True)
 
 
-def diag(dev):
-    """where the time of the fused kernel goes: skip the epilogue reads (1), the operand copies (2), both (3)"""
-    lib = _lib.load()
-    S, F, P, B, ks = 32768, 1000, 1024, 20, 6
-    Om = torch.randn(S, F, dtype=torch.float64, device=dev)
-    PhiT = torch.randn(B, P, F, dtype=torch.float64, device=dev)
-    ap, asc = ops.ozaki_slice(Om, 0, ks)
-    bp, bsc = ops.ozaki_slice(PhiT, 1, ks)
-    fmax = torch.empty((B, S), dtype=torch.float64, device=dev)
-    arg = torch.empty((B, S), dtype=torch.int32, device=dev)
-    dbg = torch.zeros(8, dtype=torch.int64, device=dev)
-    for ts in (0,):
-        lib.ppbo_set_tuning(1, ts)
-        for d in (0, 1, 2, 3):
-            lib.ppbo_set_tuning(2, d | 4)
-            t = timeit(lambda: ops.ozaki_rowmax(ap, asc, S, bp, bsc, P, B, F, ks, fmax=fmax, arg=arg, err=dbg), reps=5, warm=2)
-            mmas = (S // 128) * B * (P // 64) * 16 * 42 / 148
-            clk, ns = dbg[1].item(), dbg[2].item()
-            print("smem-A=%d diag=%d: %.3f ms; block 0: %.3f ms at %.0f MHz -> %.1f clk per 128x64x32 MMA (floor 32)" % (
-                ts, d, t, ns * 1e-6, clk / ns * 1e3, clk / mmas), flush=True)
-    lib.ppbo_set_tuning(2, 0)
-    lib.ppbo_set_tuning(1, 0)
-    lib.ppbo_set_tuning(4, 0)
-
-
 def main():
     dev = torch.device("cuda", 0)
     if "--ubench" in sys.argv:
         return ubench(dev)
-    if "--diag" in sys.argv:
-        return diag(dev)
     S, F, P, B = 32768, 1000, 1024, 20
     if len(sys.argv) > 1:
         S = int(sys.argv[1])
@@ -77,8 +50,7 @@ def main():
     PhiT = 0.02 * torch.cos(3 * torch.randn(B, P, F, dtype=torch.float64, device=dev))
     lib = _lib.load()
     ref = ops.rff_eval_argmax(Om, PhiT)
-    for ks, ss, ng in ((6, 0, 1), (6, 0, 2), (6, 0, 4), (6, 0, 8), (6, 0, 16), (5, 0, 4), (7, 0, 4), (6, 1, 4)):
-        lib.ppbo_set_tuning(1, ss)
+    for ks, ng in ((6, 1), (6, 2), (6, 4), (6, 8), (6, 16), (5, 4), (7, 4)):
         lib.ppbo_set_tuning(4, ng)
         ta = timeit(lambda: ops.ozaki_slice(Om, 0, ks))
         tb = timeit(lambda: ops.ozaki_slice(PhiT, 1, ks))
@@ -95,9 +67,8 @@ def main():
         iops = flop * ks * (ks + 1) / 2
         d = (fmax - ref[0]).abs().max().item() / ref[0].abs().max().item()
         same = (arg == ref[1]).double().mean().item()
-        print("slices=%d groups=%d%s: slice A %.3f ms, slice B %.3f ms, gemm+rowmax %.3f ms = %.1f TFLOP/s FP64-equivalent, %.0f TOP/s int8; "
-              "max rel diff vs DMMA %.2e, same argmax %.6f" % (ks, ng, " (A staged in TMEM)" if ss else "", ta, tb, t, flop / t / 1e9, iops / t / 1e9, d, same), flush=True)
-    lib.ppbo_set_tuning(1, 0)
+        print("slices=%d groups=%d: slice A %.3f ms, slice B %.3f ms, gemm+rowmax %.3f ms = %.1f TFLOP/s FP64-equivalent, %.0f TOP/s int8; "
+              "max rel diff vs DMMA %.2e, same argmax %.6f" % (ks, ng, ta, tb, t, flop / t / 1e9, iops / t / 1e9, d, same), flush=True)
     lib.ppbo_set_tuning(4, 0)
 
 

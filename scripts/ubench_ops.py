@@ -29,38 +29,16 @@ def main():
         A = A0 @ A0.T + n * torch.eye(n, dtype=torch.float64, device=dev)
         W = A.clone()
         if n >= 2000:
-            _lib.load().ppbo_set_tuning(3, 1)
-            t1 = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
-            _lib.load().ppbo_set_tuning(3, 0)
-            print("potrf n=%d, critical path on the caller's stream (no priorities): %.3f ms" % (n, t1))
-        if n >= 2000:
-            _lib.load().ppbo_set_tuning(6, 1)
-            t1 = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
-            _lib.load().ppbo_set_tuning(6, 0)
-            print("potrf n=%d, paired rank-256 trailing updates with a two-column look-ahead: %.3f ms" % (n, t1))
-        if n >= 2000:
-            _lib.load().ppbo_set_tuning(7, 1)
-            t1 = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
-            _lib.load().ppbo_set_tuning(7, 0)
-            print("potrf n=%d, programmatic dependent launch on the critical path: %.3f ms" % (n, t1))
-        if n >= 2000:
             _lib.load().ppbo_set_tuning(8, 1)
             t1 = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
             _lib.load().ppbo_set_tuning(8, 0)
             print("potrf n=%d, general GEMM kernel for panel and look-ahead: %.3f ms" % (n, t1))
         if n >= 2000:
-            for key, val, label in ((9, 1, "general GEMM kernel for the trailing update"), (9, 2, "one-tile trailing-update kernel"),
-                                    (10, 4, "strip trailing-update kernel, strips of 4"), (10, 16, "strip trailing-update kernel, strips of 16")):
-                _lib.load().ppbo_set_tuning(key, val)
-                t1 = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
-                _lib.load().ppbo_set_tuning(key, 0)
-                print("potrf n=%d, %s: %.3f ms" % (n, label, t1))
+            _lib.load().ppbo_set_tuning(9, 1)
+            t1 = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
+            _lib.load().ppbo_set_tuning(9, 0)
+            print("potrf n=%d, general GEMM kernel for the trailing update: %.3f ms" % (n, t1))
         t = timeit(lambda: ops.potrf_lower(W), setup=lambda: W.copy_(A))
-        if "--timeline" in sys.argv:
-            W.copy_(A)
-            _lib.load().ppbo_set_tuning(5, 1)
-            ops.potrf_lower(W)
-            _lib.load().ppbo_set_tuning(5, 0)
         W.copy_(A)
         info, ws = ops.potrf_lower(W)
         L = torch.tril(W)
@@ -103,11 +81,9 @@ def main():
             print("  cfg %d %dx%dx%d: %.3f ms (%.2f TFLOP/s) err=%.1e" % (cfg, M, N, K, t, 2.0 * M * N * K / t / 1e9, err))
     Om = torch.randn(32768, 1000, dtype=torch.float64, device=dev)
     PhiT = torch.randn(20, 1024, 1000, dtype=torch.float64, device=dev)
-    for cfg in (() if "--no-rowmax" in sys.argv else (0, 1, 3)):
-        _lib.load().ppbo_set_tuning(0, cfg)
+    if "--no-rowmax" not in sys.argv:
         t = timeit(lambda: ops.rff_eval_argmax(Om, PhiT), reps=3, warm=1)
-        print("rowmax cfg %d S=32768 F=1000 P=1024 B=20: %.2f ms (%.2f TFLOP/s)" % (cfg, t, 2.0 * 32768 * 1000 * 1024 * 20 / t / 1e9))
-    _lib.load().ppbo_set_tuning(0, 0)
+        print("rowmax S=32768 F=1000 P=1024 B=20: %.2f ms (%.2f TFLOP/s)" % (t, 2.0 * 32768 * 1000 * 1024 * 20 / t / 1e9))
     if "--gemm-only" in sys.argv:
         return
     prob = synthetic.make_problem("ackley20d")

@@ -519,28 +519,25 @@ def test_rff_eval_argmax_ties_exact(ops, layout):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("key", [0, 1, 3])
-def test_rowmax_large_configs_and_group_tail(ops, lib, key):
-    """S = 6400, batch 3: ceil(S / 128) * batch >= 148 selects the non-small configurations (tuning key 0: 0 Tall3, 1 Big,
-    3 Sq16); with K = 1024 a row-tile group holds 48 of the 50 row tiles, so the last group is a tail (tiles_m % group_m != 0)
+def test_rowmax_large_configs_and_group_tail(ops):
+    """S = 6400, batch 3: ceil(S / 128) * batch >= 148 selects the non-small configurations (Tall3, and BigU for an odd ld);
+    with K = 1024 a row-tile group holds 48 of the 50 row tiles, so the last group is a tail (tiles_m % group_m != 0)
     whenever the A operand is shared by the batch entries (rff_eval_argmax, and mvn_rowmax with a stride-0 Z)"""
     S, P, K, B = 6400, 257, 1024, 3
     Z, Fac, mu, V = rowmax_case(B, S, P, K, 11, shared=True)
     Zd, Facd, mud = _dev(Z), _dev(Fac), _dev(mu)
-    with tuning(lib, 0, key):
-        fmax, arg = ops.mvn_rowmax(Zd.expand(B, S, K), Facd, mud)                 # group tail
-        assert _check_rowmax(fmax, arg, V)
-        Zb, Facb, mub, Vb = rowmax_case(B, S, P, K, 12)
-        fmax, arg = ops.mvn_rowmax(_dev(Zb), _dev(Facb), _dev(mub))               # per-entry Z: one group
-        assert _check_rowmax(fmax, arg, Vb)
-        Fac0 = Fac.copy()
-        Fac0[:, :, len(tie_pairs(P))] = 0.0                                        # no bias: all-tie rows are 0
-        V0 = np.matmul(Z, Fac0.transpose(0, 2, 1))
-        fmax, arg, _ = ops.rff_eval_argmax(Zd, _dev(Fac0))
-        assert _check_rowmax(fmax, arg, V0)
-        if key == 0:                                                               # odd ld: CfgBigU
-            fmax, arg, _ = ops.rff_eval_argmax(_operand(Z, "odd"), _strided3(Fac0, "odd"))
-            assert _check_rowmax(fmax, arg, V0)
+    fmax, arg = ops.mvn_rowmax(Zd.expand(B, S, K), Facd, mud)                     # group tail
+    assert _check_rowmax(fmax, arg, V)
+    Zb, Facb, mub, Vb = rowmax_case(B, S, P, K, 12)
+    fmax, arg = ops.mvn_rowmax(_dev(Zb), _dev(Facb), _dev(mub))                   # per-entry Z: one group
+    assert _check_rowmax(fmax, arg, Vb)
+    Fac0 = Fac.copy()
+    Fac0[:, :, len(tie_pairs(P))] = 0.0                                            # no bias: all-tie rows are 0
+    V0 = np.matmul(Z, Fac0.transpose(0, 2, 1))
+    fmax, arg, _ = ops.rff_eval_argmax(Zd, _dev(Fac0))
+    assert _check_rowmax(fmax, arg, V0)
+    fmax, arg, _ = ops.rff_eval_argmax(_operand(Z, "odd"), _strided3(Fac0, "odd"))   # odd ld: CfgBigU
+    assert _check_rowmax(fmax, arg, V0)
 
 
 @pytest.mark.gpu
@@ -623,11 +620,11 @@ def test_potrf_exact_factor(ops, n, lda):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("key,value", [(8, 1), (9, 1), (9, 2)])
+@pytest.mark.parametrize("key,value", [(8, 1), (9, 1)])
 @pytest.mark.parametrize("n", [1025, 2049])
 def test_potrf_tuning_paths(ops, lib, n, key, value):
-    """general GEMM kernel instead of the row-panel kernel (8 = 1) or the strip trailing update (9 = 1), one tile per CTA (9 = 2):
-    the same bounds and contract, and close to the default path's factor"""
+    """general GEMM kernel instead of the row-panel kernel (8 = 1) or the strip trailing update (9 = 1): the same bounds and
+    contract, and close to the default path's factor"""
     L0, A = chol_case(n)
     _, _, _, v0 = _factor_on_device(ops, A, n + 2)
     with tuning(lib, key, value):

@@ -139,6 +139,22 @@ def test_c_abi_exports_every_declared_symbol():
     assert lib.ppbo_factor_doubles(256) == 256 * 256 + 2 * 128 * 128
 
 
+def test_set_tuning_rejects_retired_keys():
+    """ppbo_set_tuning accepts the keys that select a reference path or a launch shape (4, 8, 9 = 0 / 1, 11, 14, 15) and
+    rejects the numbers of removed variants, so that a script written for one of them fails instead of timing the default."""
+    from ppbo_b200 import _lib
+    from ppbo_b200 import build as _build
+    _build.build()
+    lib = _lib.load()
+    for key in (0, 1, 2, 3, 5, 6, 7, 10, 12, 13, -1, 16):
+        assert lib.ppbo_set_tuning(key, 1) == -1, key
+        assert b"tuning key" in lib.ppbo_last_error()
+    assert lib.ppbo_set_tuning(9, 2) == -1
+    for key, value in ((4, 2), (8, 1), (9, 1), (11, 1), (14, 12), (15, 3)):
+        assert lib.ppbo_set_tuning(key, value) == 0, key
+        assert lib.ppbo_set_tuning(key, 0) == 0, key
+
+
 def test_no_cpu_fallback_without_gpu():
     import torch
     from ppbo_b200 import ops
