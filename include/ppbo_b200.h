@@ -302,11 +302,6 @@ long long ppbo_rff_factor_cache_doubles(int F);
 int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int m, double sigma, const double* omega0,
                  int max_iter, double tol, double* factor_cache, int warm_factor, double* omega_map, double* hess_diag,
                  void* workspace, long long workspace_bytes, double* stats_h, void* stream);
-/* Hessian factor (and its block inverses) AT omega into factor_cache, asynchronously and without a host synchronisation: what the
- * next ppbo_rff_fit(..., warm_factor = 2) of a grown design starts with.  (The reference's trust-exact run rebuilds its Hessian
- * at every one of its iterations, src/random_fourier_sampler.py:124-132.) */
-int ppbo_rff_refactor(const double* Phi_X, long long ld, int F, int Q, int m, double sigma, const double* omega,
-                      double* factor_cache, void* workspace, long long workspace_bytes, void* stream);
 /* Full Laplace covariance of the weight-space posterior (opt-in; the reference's covariance is diagonal,
  * src/random_fourier_sampler.py:134-137, and so is the default path above).  L[F x ldl] (followed by the inverted 128-blocks the
  * solves read: ppbo_rff_hessian_factor_doubles(F, ldl) doubles in all) receives the Cholesky factor of the EXACT Hessian

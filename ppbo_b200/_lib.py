@@ -85,7 +85,6 @@ _SIGNATURES = {
     "ppbo_rff_objective": (_I, [_P, _L, _I, _I, _I, _D, _P, _PD, _P, _P, _P, _L, _P]),
     "ppbo_rff_factor_cache_doubles": (_L, [_I]),
     "ppbo_rff_fit": (_I, [_P, _L, _I, _I, _I, _D, _P, _I, _D, _P, _I, _P, _P, _P, _L, _PD, _P]),
-    "ppbo_rff_refactor": (_I, [_P, _L, _I, _I, _I, _D, _P, _P, _P, _L, _P]),
     "ppbo_rff_hessian_factor_workspace_bytes": (_L, [_I, _I, _I]),
     "ppbo_rff_hessian_factor_doubles": (_L, [_I, _L]),
     "ppbo_rff_hessian_factor": (_I, [_P, _L, _I, _I, _I, _D, _P, _P, _L, _P, _L, _PI, _P]),

@@ -1101,35 +1101,6 @@ extern "C" int ppbo_rff_fit(const double* Phi_X, long long ld, int F, int Q, int
     return PPBO_OK;
 }
 
-/* Factor of the weight-space Hessian AT omega, asynchronously: H = I + Psi' a+(omega) Psi, its Cholesky factor and the 1024-block
- * inverses go to factor_cache (layout of ppbo_rff_fit); no host synchronisation, nothing is read back.  A model that grows by one
- * comparison set per iteration calls this after each fit, off the critical path (run_iteration: while the sampling contraction
- * runs), so that the next fit starts its chord steps with a factor built at its own starting point instead of one that is an
- * iteration old (13 chord steps and a mid-fit refactorisation every few iterations with the stale factor). */
-extern "C" int ppbo_rff_refactor(const double* Phi_X, long long ld, int F, int Q, int m, double sigma, const double* omega,
-                                 double* factor_cache, void* workspace, long long workspace_bytes, void* stream) {
-    PPBO_REQUIRE(workspace_bytes >= ppbo_rff_workspace_bytes(F, Q, m) && factor_cache != nullptr, "workspace / cache");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int M = Q * m;
-    RffWs ws;
-    ws.carve((double*)workspace, F, Q, m);
-    ws.H = factor_cache;
-    ws.binv = factor_cache + ppbo_factor_doubles(F);
-    double* Hdinv = ws.H + (long long)F * F;
-    int* info_d = reinterpret_cast<int*>(ws.scal + 32);
-    PPBO_CUDA_CHECK(ws.zero_counters(st));
-    int rc;
-    if ((rc = rff_eval(Phi_X, ld, F, Q, m, sigma, omega, ws, nullptr, nullptr, true, ws.scal + 24, st))) return rc;
-    PPBO_CL rff_psi_kernel<<<dim3(ceil_div(M, 256), F), 256, 0, st>>>(Phi_X, ld, Q, m, ws.arrow, ws.PsiT, M);
-    GemmOperands g{ws.PsiT, M, 0, ws.PsiT, M, 0, F, F, M};
-    StoreEpilogue ep{ws.H, F, 0, 1.0, 0.0, 2, 0, 0};                // lower tiles only, as in ppbo_rff_fit
-    if ((rc = launch_gemm_nt(g, ep, 1, st))) return rc;
-    PPBO_CL add_identity_kernel<<<ceil_div(F, 256), 256, 0, st>>>(ws.H, F, F);
-    PPBO_LAUNCH_CHECK();
-    if ((rc = potrf_lower(ws.H, F, F, Hdinv, info_d, st))) return rc;       // I + PSD: always positive definite
-    return blockinv_build(ws.H, F, F, Hdinv, ws.binv, st);
-}
-
 /* The exact weight-space Hessian -grad^2 S(omega) = I + Psi' diag(a) Psi with the SIGNED coefficients a (the fit factors the clamped
  * I + Psi' a+ Psi, which is the right chord matrix but not the Laplace precision), factorised into the caller's L: the full
  * covariance of the weight-space posterior is its inverse.  Nothing of the fit's factor cache is touched. */

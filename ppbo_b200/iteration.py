@@ -26,11 +26,10 @@ from ._lib import PPBOError
 
 F64 = torch.float64
 SHRINKAGE = 1e-6          # GPModel.COVARIANCE_SHRINKAGE, src/gp_model.py:26
-# Sampling contraction Omega . PhiT^T: "i8" = tcgen05 INT8 tensor pipe with error-free splitting into SLICES base-256 digit
-# planes per operand (csrc/ozaki.cu; 6 planes: ~1e-13 relative, i.e. the accuracy of an FP64 GEMM of this depth), "f64" = the
-# FP64 DMMA kernel.  Small contractions (reference-size grids) stay on the FP64 kernel: a 128 x 64 INT8 tile would be mostly
-# padding there.
-SAMPLING_ENGINE = "i8"
+# Sampling contraction Omega . PhiT^T (sampling_engine): "i8" = tcgen05 INT8 tensor pipe with error-free splitting into
+# SAMPLING_SLICES base-256 digit planes per operand (csrc/ozaki.cu; 6 planes: ~1e-13 relative, i.e. the accuracy of an FP64 GEMM
+# of this depth), "f64" = the FP64 DMMA kernel.  Small contractions (reference-size grids) stay on the FP64 kernel: a 128 x 64
+# INT8 tile would be mostly padding there.
 SAMPLING_SLICES = 6
 I8_MIN_WORK = 1 << 24     # S * P * F below which the FP64 kernel is used
 # Covariance of the weight-space Laplace posterior the draws come from: "diag" = the reference's 1 / -hess_diag
@@ -40,34 +39,26 @@ I8_MIN_WORK = 1 << 24     # S * P * F below which the FP64 kernel is used
 WEIGHT_COVARIANCES = ("diag", "full")
 
 
-# The GP fit and the weight-space (RFF) fit only share their input X: both are chains of small, latency-bound launches with one
-# host decision per Newton step, so rank 0 drives them from two host threads on two streams and the shorter one (RFF) hides
-# behind the longer.  The RFF fit then starts from omega = 0 (or the caller's omega0) instead of the projection of the GP mode,
-# which costs one extra Newton step (20 against 19 on the Ackley-20D bench problem).
-CONCURRENT_FITS = True
-# One GPU: the sampling contraction needs the weight-space fit only (mu* enters at the reduction), so the background thread goes
-# on from the weight-space fit to the draws and the INT8 contraction on its lowest-priority stream WHILE the GP fit -- a chain of
-# small, latency-bound kernels that leaves most SMs idle -- runs beside it.  The contraction's persistent grid then leaves
-# OVERLAP_RESERVED_SMS(_COLD) SMs to the fit (tuning key 14); a contraction CTA fills its SM, so the two never share one.
-# PPBO_OVERLAP_SAMPLING=0 restores the sequential order (diagnostics).
-import os as _os
+# One GPU: the sampling contraction needs the weight-space fit only (mu* enters at the reduction), so the weight-space fit, the
+# draws and the INT8 contraction run in the foreground WHILE the GP fit -- a chain of small, latency-bound kernels that leaves most
+# SMs idle -- runs beside them on the background thread.  The contraction's persistent grid then leaves OVERLAP_RESERVED_SMS(_COLD)
+# SMs to the GP fit (tuning key 14); a contraction CTA fills its SM, so the two never share one.  OVERLAP_SAMPLING = False runs the
+# contraction after both fits instead: the same bits, which makes that order the reference of the overlapped one.
+OVERLAP_SAMPLING = True
 # Reserved SMs: an appended iteration's GP chain is short (it still ends before the contraction on 8 SMs); a cold fit has 13
 # chord steps with one 100 MB half-triangle mat-vec of G each plus the factorisation and is the longer chain, so it gets more
 # (sweeps in DESIGN.md 5.1).
-_RESERVE_ENV = _os.environ.get("PPBO_OVERLAP_RESERVE")
-OVERLAP_RESERVED_SMS = int(_RESERVE_ENV) if _RESERVE_ENV else 12            # appended iterations
-OVERLAP_RESERVED_SMS_COLD = int(_RESERVE_ENV) if _RESERVE_ENV else 24       # cold iterations
-# Steady state of the overlapped pipeline, opt-in: refresh the weight-space Hessian factor at each new optimum while the contraction
-# runs (RFFState.refresh_factor).  The next fit then needs 10 chord steps and never a mid-fit refactorisation (7-13 steps and a
-# refactorisation in 6 of 13 iterations with the stale factor, tests/test_steady_state.py), but the refresh (10 GFLOP of Hessian GEMM + a Cholesky) shares
-# the reserved SMs with the GP chain, which then ends AFTER the contraction: 14.05 ms per appended iteration against 13.09 without
-# (measured), so it is off.
-REFRESH_RFF_FACTOR = _os.environ.get("PPBO_RFF_REFRESH", "0") != "0"
-OVERLAP_SAMPLING = _os.environ.get("PPBO_OVERLAP_SAMPLING", "1") != "0"
+OVERLAP_RESERVED_SMS = 12            # appended iterations
+OVERLAP_RESERVED_SMS_COLD = 24       # cold iterations
 
 
 def sampling_engine(S, P, Fdim):
-    return "i8" if (SAMPLING_ENGINE == "i8" and S * P * Fdim >= I8_MIN_WORK) else "f64"
+    return "i8" if S * P * Fdim >= I8_MIN_WORK else "f64"
+
+
+def _fused_draw(Fdim):
+    """whether the draws and their digit planes fit one kernel: it holds 8 rows of F doubles in at most 200 KB of shared memory"""
+    return Fdim * 64 <= 200 * 1024
 
 
 class SlicedGrids:
@@ -325,7 +316,6 @@ class RFFState:
         self.factor_cache = ops.rff_factor_cache(W.shape[0], W.device)
         self.L_buf = None            # exact-Hessian factor of the full covariance: its own buffer, never the fit's factor_cache
         self.fit = None
-        self.pending = None          # stream of an asynchronous refresh of the factor (refresh_factor): the next fit waits for it
 
     def _fit(self, Q, omega0, warm=False):
         r = RFFFit()
@@ -344,23 +334,7 @@ class RFFState:
             self.L_buf = ops.rff_hessian_factor_buffer(self.W.shape[0], self.W.device)
         return rff_full_factor(self.fit, self.Q, self.m, self.theta[0], out=self.L_buf)
 
-    def _wait_refresh(self):
-        if self.pending is not None:
-            torch.cuda.current_stream().wait_stream(self.pending)
-            self.pending = None
-
-    def refresh_factor(self):
-        """Rebuild the Hessian factor (and its block inverses) at the optimum just found, asynchronously on the CURRENT stream: the
-        next append then starts its chord steps from a factor built at its own starting point (ppbo_rff_refactor).  The caller
-        runs this off the critical path and leaves the stream in self.pending."""
-        r = self.fit
-        ops.rff_refactor(r.Phi_X, self.Q, self.m, self.theta[0], r.omega_map, self.factor_cache)
-        r.stats["warm"] = True
-        r.stats["binv_cached"] = True
-        self.pending = torch.cuda.current_stream()
-
     def cold(self, X, omega0=None):
-        self._wait_refresh()
         Q = X.shape[0] // (self.m + 1)
         ops.rff_features(self.W, self.b, X, self.theta[2], True, out=self.Phi_cap[:, :X.shape[0]])
         return self._fit(Q, omega0)
@@ -368,7 +342,6 @@ class RFFState:
     def append(self, X_block):
         if self.Q == 0:
             return self.cold(X_block)
-        self._wait_refresh()
         N_old = self.Q * (self.m + 1)
         ops.rff_features(self.W, self.b, X_block, self.theta[2], True, out=self.Phi_cap[:, N_old:N_old + X_block.shape[0]])
         warm = self.fit.stats.get("factorizations", 0) > 0 or self.fit.stats.get("warm", False)
@@ -425,7 +398,7 @@ def rff_prepare_normals(Fdim, lo, hi, P, dev, Z=None, seed=0, stream_id=0):
     if hi <= lo:
         return None
     i8 = sampling_engine(hi - lo, P, Fdim) == "i8"
-    if Z is None and i8 and Fdim * 64 <= 200 * 1024:
+    if Z is None and i8 and _fused_draw(Fdim):
         return SlicedSamples(drawn=ops.ozaki_normal_slice(hi - lo, Fdim, dev, seed=seed, stream_id=stream_id, sample0=lo,
                                                           slices=SAMPLING_SLICES), count=hi - lo)
     Zloc = Z[lo:hi] if Z is not None else ops.normal_fill(seed, stream_id, lo * Fdim, (hi - lo) * Fdim, dev).view(hi - lo, Fdim)
@@ -455,7 +428,7 @@ def rff_prepare_samples(r, lo, hi, P, Z=None, seed=0, stream_id=0, covariance="d
     Fdim = r.omega_map.shape[0]
     if covariance == "full":
         return rff_prepare_normals(Fdim, lo, hi, P, r.omega_map.device, Z=Z, seed=seed, stream_id=stream_id)
-    if Z is None and sampling_engine(hi - lo, P, Fdim) == "i8" and Fdim * 64 <= 200 * 1024:
+    if Z is None and sampling_engine(hi - lo, P, Fdim) == "i8" and _fused_draw(Fdim):
         # draws and digit planes in one kernel: the S x F matrix of draws never reaches HBM
         return SlicedSamples(drawn=ops.ozaki_sample_slice(r.omega_map, r.hess_diag, hi - lo, seed=seed, stream_id=stream_id, sample0=lo,
                                                           slices=SAMPLING_SLICES), count=hi - lo)
@@ -557,16 +530,15 @@ class IterationInputs:
 
 
 _SIDE_STREAMS = {}
-# The GP fit is the critical path of the iteration: its launches go to a stream one level above the default priority, its
-# Cholesky bulk (library-internal side stream) sits at the same level, and the background weight-space fit keeps the default
-# (lowest) priority for everything (ppbo_set_thread_background), so it only fills the SMs the GP fit leaves idle.
-# None / 0: stay on the caller's stream.
-GP_STREAM_PRIORITY = int(_os.environ.get("PPBO_FG_PRIORITY", "-1"))
+# The foreground chain of the one-GPU schedules goes to a stream one level above the default priority, where this thread's
+# Cholesky bulk (library-internal side stream) sits too; the background thread keeps the default (lowest) priority for everything
+# (ppbo_set_thread_background), so its chain only fills the SMs the foreground leaves idle.
+FOREGROUND_PRIORITY = -1
 _WORKER = None
 
 
 def _background_worker():
-    """One persistent host thread for the concurrent weight-space fit (the library keeps per-thread streams: a fresh thread per
+    """One persistent host thread for the chain beside the foreground one (the library keeps per-thread streams: a fresh thread per
     iteration would create new ones every time).  Marked as background before its first launch."""
     global _WORKER
     if _WORKER is None:
@@ -584,13 +556,46 @@ def _side_stream(dev, priority=0, tag=""):
     return _SIDE_STREAMS[key]
 
 
+def _join(dst, src, tensors):
+    """dst waits for the work queued on src so far; the tensors src made stay allocated until dst's work on them is done"""
+    dst.wait_stream(src)
+    for t in tensors:
+        t.record_stream(dst)
+
+
+def _device_tensors(*parts):
+    """the tensors behind grid features and prepared draws (SlicedGrids, SlicedSamples, a tensor or None)"""
+    out = []
+    for p in parts:
+        if isinstance(p, SlicedGrids):
+            out += [p.PhiT, p.planes, p.scale]
+        elif isinstance(p, SlicedSamples):
+            out += [p.planes, p.scale]
+        elif p is not None:
+            out.append(p)
+    return out
+
+
+def _gp_tensors(gp):
+    return [gp.Sigma, gp.lap.G, gp.lap._Lfac, gp.lap.f_map, gp.lap.alpha, gp.lap.arrow]
+
+
+def _rff_tensors(rff):
+    return [rff.omega_map, rff.hess_diag, rff.Phi_X] + ([rff.L] if rff.L is not None else [])
+
+
+def _weight_space_rank(world):
+    """the rank that runs the weight-space fit: with more than one GPU the two fits run on two of them"""
+    return 1 if world > 1 else 0
+
+
 class IterationState:
     """What persists between the iterations of one PPBO run on this rank: the growing GP model (rank 0) and the growing
     weight-space model (the rank that runs the weight-space fit)."""
 
     def __init__(self, kernel, theta, D, m, Q_cap, dev, W, b, shard=None, fit_iters=100, tol=1e-8):
         shard = shard or Shard()
-        rff_rank = 1 if (CONCURRENT_FITS and shard.world > 1) else 0
+        rff_rank = _weight_space_rank(shard.world)
         self.gp = GPState(kernel, theta, D, m, Q_cap, dev, max_iter=fit_iters, tol=tol) if shard.rank == 0 else None
         self.rff = RFFState(W, b, theta, m, Q_cap, max_iter=fit_iters, tol=tol) if shard.rank == rff_rank else None
         self.Q, self.m = 0, m
@@ -598,6 +603,50 @@ class IterationState:
 
     def design(self, Q):
         return self.X_cap[:Q * (self.m + 1)]
+
+
+class _Iteration:
+    """One call of run_iteration: its arguments and what follows from them, the two fits and the timer marks."""
+
+    def __init__(self, d, kernel, theta, Q, m, S, shard, seed, fit_iters, tol, timers, state, shares, factor_at_mode, shard_mustar,
+                 weight_covariance):
+        self.d, self.kernel, self.theta, self.Q, self.m, self.S, self.seed = d, kernel, theta, Q, m, S, seed
+        self.shard, self.fit_iters, self.tol, self.timers, self.state = shard, fit_iters, tol, timers, state
+        self.factor_at_mode, self.covariance, self.full = factor_at_mode, weight_covariance, weight_covariance == "full"
+        self.W, self.b, self.grids = d["W"], d["b"], d["grids"]
+        self.dev, self.Fdim = self.W.device, self.W.shape[0]
+        self.B, self.P, D = self.grids.shape
+        self.cand = self.grids.reshape(self.B * self.P, D)
+        self.warm = state is not None and state.Q > 0
+        self.X = None if self.warm else d["X"]
+        self.block = d["block"] if self.warm else None
+        self.shard_mustar = (shard.world >= 3 and not self.warm) if shard_mustar is None else shard_mustar
+        self.lo, self.hi = shard.sample_bounds(S, shares)
+        self.i8 = self.hi > self.lo and sampling_engine(self.hi - self.lo, self.P, self.Fdim) == "i8"
+
+    def mark(self, name):
+        """timing event on the current stream"""
+        if self.timers is not None:
+            ev = torch.cuda.Event(enable_timing=True)
+            ev.record()
+            self.timers.append((name, ev))
+
+    def fit_gp(self):
+        if self.state is None:
+            return gp_fit(self.X, self.kernel, self.theta, self.Q, self.m, f_init=self.d.get("f_init"), max_iter=self.fit_iters,
+                          tol=self.tol, factor_at_mode=self.factor_at_mode)
+        if self.warm:
+            return self.state.gp.append(self.block, factor_at_mode=self.factor_at_mode)
+        return self.state.gp.cold(self.X, f_init=self.d.get("f_init"), factor_at_mode=self.factor_at_mode)
+
+    def fit_rff(self):
+        if self.state is None:
+            r = rff_fit(self.X, self.W, self.b, self.theta, self.Q, self.m, omega0=self.d.get("omega0"), max_iter=self.fit_iters,
+                        tol=self.tol)
+            return rff_full_factor(r, self.Q, self.m, self.theta[0]) if self.full else r
+        st = self.state.rff
+        r = st.append(self.block) if self.warm else st.cold(self.X, omega0=self.d.get("omega0"))
+        return st.hessian_factor() if self.full else r
 
 
 def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, tol=1e-8, timers=None, state=None, shares=None,
@@ -616,299 +665,209 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     them inside the collective.
     weight_covariance: "diag" (the reference's) or "full" (WEIGHT_COVARIANCES): the rank that fits the weight space also factors the
     exact Hessian at omega_MAP and sends the factor with (omega_MAP, hess_diag); the draws are standard normals and every sampling
-    rank transforms its grid features once (rff_transform_grids)."""
+    rank transforms its grid features once (rff_transform_grids).
+    timers: a list that receives (name, CUDA event) marks between the stages of the schedule that ran."""
     if weight_covariance not in WEIGHT_COVARIANCES:
         raise PPBOError("weight_covariance must be one of %s" % (WEIGHT_COVARIANCES,))
-    full = weight_covariance == "full"
-    shard = shard or Shard()
-    W, b, grids = d["W"], d["b"], d["grids"]
-    dev = W.device
-    Fdim = W.shape[0]
-    B, P, D = grids.shape
-    warm = state is not None and state.Q > 0
-    if shard_mustar is None:
-        shard_mustar = shard.world >= 3 and not warm
-    X = None if warm else d["X"]
-    block = d["block"] if warm else None
+    it = _Iteration(d, kernel, theta, Q, m, S, shard or Shard(), seed, fit_iters, tol, timers, state, shares, factor_at_mode,
+                    shard_mustar, weight_covariance)
     if state is not None:
-        if warm:
-            state.X_cap[state.Q * (m + 1):Q * (m + 1)].copy_(block)
+        if it.warm:
+            state.X_cap[state.Q * (m + 1):Q * (m + 1)].copy_(it.block)
         else:
-            state.X_cap[:Q * (m + 1)].copy_(X)
-
-    def mark(name):
-        if timers is not None:
-            ev = torch.cuda.Event(enable_timing=True)
-            ev.record()
-            timers.append((name, ev))
-
-    def fit_gp():
-        if state is None:
-            return gp_fit(X, kernel, theta, Q, m, f_init=d.get("f_init"), max_iter=fit_iters, tol=tol, factor_at_mode=factor_at_mode)
-        if warm:
-            return state.gp.append(block, factor_at_mode=factor_at_mode)
-        return state.gp.cold(X, f_init=d.get("f_init"), factor_at_mode=factor_at_mode)
-
-    def fit_rff():
-        if state is None:
-            r = rff_fit(X, W, b, theta, Q, m, omega0=d.get("omega0"), max_iter=fit_iters, tol=tol)
-            return rff_full_factor(r, Q, m, theta[0]) if full else r
-        r = state.rff.append(block) if warm else state.rff.cold(X, omega0=d.get("omega0"))
-        return state.rff.hessian_factor() if full else r
-
-    def mu_star(gp, cand):
-        """max posterior mean over the design rows and the candidate points; with >= 3 ranks every rank takes a slice of the
-        candidates (alpha travels by broadcast) and one all-reduce(max) follows"""
-        if not shard_mustar:
-            return mustar_over_candidates(gp, cand) if shard.rank == 0 else None
-        Qn = Q
-        N = Qn * (m + 1)
-        pack_a = torch.empty(N + 1, dtype=F64, device=dev)          # alpha and max f_MAP
-        if shard.rank == 0:
-            pack_a[:N].copy_(gp.alpha)
-            ops.vec_max(gp.f_map, out=pack_a[N:])
-        shard.broadcast(pack_a, src=0)
-        lo_c, hi_c = shard.bounds(cand.shape[0])
-        out = pack_a[N:].clone()
-        if hi_c > lo_c:
-            Xd = state.design(Q) if state is not None else X
-            mu = ops.posterior_mean(kernel, Xd, theta[1], theta[2], pack_a[:N], cand[lo_c:hi_c])
-            ops.vec_max(mu, out=out, accumulate=True)
-        shard.all_reduce_max(out)
-        return out
-    mark("start")
-    lo, hi = shard.sample_bounds(S, shares)
-    # The grid features (and their digit planes) do not depend on the fit.  On the rank that runs the latency-bound GP fit they
-    # go to the side stream and fill SMs the fit leaves idle; the other ranks compute them while they wait for the broadcast.
+            state.X_cap[:Q * (m + 1)].copy_(it.X)
+    it.mark("start")
     main = torch.cuda.current_stream()
-    grid_stream = _side_stream(dev, tag="grid") if shard.rank == 0 else main
-    if grid_stream is not main:
-        grid_stream.wait_stream(main)
-    PhiT = normals = None
-    i8 = hi > lo and sampling_engine(hi - lo, P, Fdim) == "i8"
-    with torch.cuda.stream(grid_stream):
-        if hi > lo:                                           # a rank without samples (rank 0 of several) needs no grid features
-            PhiT = rff_grid_features(W, b, theta[2], grids)
-            if full:
-                # the draws of the full covariance are plain standard normals: cut into digit planes before any fit ends; the grid
-                # features are sliced after their transform by the Hessian factor
-                normals = rff_prepare_normals(Fdim, lo, hi, P, dev, seed=seed)
-            elif i8:
-                PhiT = SlicedGrids(PhiT)                      # digit planes of the grid features
-    mark("grid_features")
-
-    def grid_tensors():
-        if PhiT is None:
-            return ()
-        out = (PhiT.PhiT, PhiT.planes, PhiT.scale) if isinstance(PhiT, SlicedGrids) else (PhiT,)
-        if isinstance(normals, SlicedSamples):
-            out += (normals.planes, normals.scale)
-        elif normals is not None:
-            out += (normals,)
-        return out
-    pack = torch.empty(2 * Fdim + 1, dtype=F64, device=dev)
-    gp = rff = prepared = None
-    cand = grids.reshape(B * P, D)
-    rff_rank = 1 if (CONCURRENT_FITS and shard.world > 1) else 0      # with more than one GPU the two fits run on two of them
-    if shard.rank == 0 and CONCURRENT_FITS and shard.world == 1 and OVERLAP_SAMPLING and i8:
-        # One GPU, INT8 engine.  Two chains that only share X:
-        #   A  GP fit -> mu*                                   latency-bound, short (8.7 ms cold / 5 ms appended when alone)
-        #   B  weight-space fit -> draws -> contraction        the contraction alone keeps every tensor pipe busy for ~9 ms
-        # B is the longer one and its head (the weight-space fit) is as latency-bound as A, so B runs in the FOREGROUND (this
-        # thread, streams above the default priority) and A on the persistent background thread whose streams all sit at the
-        # lowest priority; the contraction's persistent grid leaves OVERLAP_RESERVED_SMS SMs free, where A finishes while the
-        # tensor pipes of the other SMs are busy.  Only the reduction (3 B sums) needs both chains.
-        bg = _side_stream(dev)
-        bg.wait_stream(main)
-        fg = _side_stream(dev, priority=GP_STREAM_PRIORITY, tag="gp") if GP_STREAM_PRIORITY else main
-        if fg is not main:
-            fg.wait_stream(main)
-
-        def gp_chain():
-            torch.cuda.set_device(dev)
-            with torch.cuda.stream(bg):
-                g = fit_gp()
-                return g, mustar_over_candidates(g, cand)
-        fut = _background_worker().submit(gp_chain)
-        lib = ops._lib.load()
-        fmax = None
-        try:
-            with torch.cuda.stream(fg):
-                rff = fit_rff()
-                mark("rff_fit")
-                fit_done = torch.cuda.Event()
-                fit_done.record(fg)
-                transformed = None
-                if full:
-                    fg.wait_stream(grid_stream)
-                    for t in grid_tensors():
-                        t.record_stream(fg)
-                    prepared = normals
-                    transformed = rff_transform_grids(rff, PhiT, slices=SAMPLING_SLICES)
-                    mark("grid_transform")
-                else:
-                    prepared = rff_prepare_samples(rff, lo, hi, P, seed=seed)
-                    fg.wait_stream(grid_stream)
-                    for t in grid_tensors():
-                        t.record_stream(fg)
-                lib.ppbo_set_tuning(14, OVERLAP_RESERVED_SMS if warm else OVERLAP_RESERVED_SMS_COLD)
-                try:
-                    fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=prepared, covariance=weight_covariance,
-                                                 transformed=transformed)
-                finally:
-                    lib.ppbo_set_tuning(14, 0)
-                mark("sampling")
-            if warm and REFRESH_RFF_FACTOR:
-                # while the contraction runs: the weight-space Hessian factor at the new optimum, for the NEXT iteration's fit
-                # (lowest priority, on the SMs the contraction leaves free; it only waits for this iteration's fit)
-                rf = _side_stream(dev, tag="rff_refresh")
-                rf.wait_event(fit_done)
-                rff.omega_map.record_stream(rf)
-                with torch.cuda.stream(rf):
-                    state.rff.refresh_factor()
-        finally:
-            gp, mustar = fut.result()          # re-raises on this thread
-        main.wait_stream(bg)
-        for t in (gp.Sigma, gp.lap.G, gp.lap._Lfac, gp.lap.f_map, gp.lap.alpha, gp.lap.arrow, mustar):
-            t.record_stream(main)
-        if fg is not main:
-            main.wait_stream(fg)
-            for t in (rff.omega_map, rff.hess_diag, rff.Phi_X, fmax) + ((rff.L,) if full else ()):
-                t.record_stream(main)
-        mark("gp_tail")                        # what is left of the GP fit + mu* after the contraction has finished
-        sums = rff_reduce(fmax, mustar, B, shard)
-        mark("acquisition")
-        if state is not None:
-            state.Q = Q
-        return sums, gp, rff
-    if shard.rank == 0 and CONCURRENT_FITS and shard.world == 1:
-        # (FP64 engine / PPBO_OVERLAP_SAMPLING=0.)  GP fit: foreground, on a stream one priority level above the default;
-        # weight-space fit: a persistent background host thread whose streams all sit at the lowest priority, so it only takes the
-        # SMs the GP fit leaves idle.
-        side = _side_stream(dev)
-        side.wait_stream(main)
-        gp_stream = _side_stream(dev, priority=GP_STREAM_PRIORITY, tag="gp") if GP_STREAM_PRIORITY else main
-        if gp_stream is not main:
-            gp_stream.wait_stream(main)
-
-        def weight_space_fit():
-            torch.cuda.set_device(dev)
-            with torch.cuda.stream(side):
-                fit = fit_rff()
-                # the draws and their digit planes need this fit only: done here, behind the GP fit (the standard normals of the
-                # full covariance are already on the grid stream)
-                return fit, (normals if full else rff_prepare_samples(fit, lo, hi, P, seed=seed))
-        fut = _background_worker().submit(weight_space_fit)
-        try:
-            with torch.cuda.stream(gp_stream):
-                gp = fit_gp()
-                mark("gp_fit")
-                mustar = mustar_over_candidates(gp, cand)
-                mark("mustar")
-        finally:
-            rff, prepared = fut.result()       # re-raises on this thread
-        if gp_stream is not main:
-            main.wait_stream(gp_stream)
-            for t in (gp.Sigma, gp.lap.G, gp.lap._Lfac, gp.lap.f_map, gp.lap.alpha, gp.lap.arrow, mustar):
-                t.record_stream(main)
-        main.wait_stream(side)
-        for t in (rff.omega_map, rff.hess_diag, rff.Phi_X) + ((prepared.planes, prepared.scale) if isinstance(prepared, SlicedSamples)
-                                                              else ((prepared,) if prepared is not None else ())) + \
-                ((rff.L,) if full else ()):
-            t.record_stream(main)
-        mark("rff_fit")                        # what is left of the weight-space fit after the GP fit has finished
-    elif shard.world > 1 and CONCURRENT_FITS:
-        # Several ranks: rank 0 runs the GP fit; rank 1 runs the weight-space fit and broadcasts it; every rank with a sample share
-        # draws and evaluates its samples as soon as the weight-space fit has arrived (the contraction needs that fit only) --
-        # rank 0 after its GP fit; when mu* is known only the reduction and the all-reduce of 3 B doubles are left.
-        pack_rff, mu_t = pack[:2 * Fdim], pack[2 * Fdim:]
-        fmax = None
-        Lbuf = ops.rff_hessian_factor_buffer(Fdim, dev) if full and shard.rank != rff_rank else None
-        if shard.rank == 0:
-            bstream = _side_stream(dev, tag="bcast")     # rank 0 joins the first broadcast off its critical path
-            bstream.wait_stream(main)
-            pack.record_stream(bstream)
-            with torch.cuda.stream(bstream):
-                shard.broadcast(pack_rff, src=rff_rank)
-                if full:
-                    Lbuf.record_stream(bstream)
-                    shard.broadcast(Lbuf, src=rff_rank)
-            gp = fit_gp()
-            mark("gp_fit")
-            main.wait_stream(bstream)
-        else:
-            if shard.rank == rff_rank:
-                rff = fit_rff()
-                mark("rff_fit")
-                pack_rff[:Fdim].copy_(rff.omega_map)
-                pack_rff[Fdim:].copy_(rff.hess_diag)
-                Lbuf = rff.L
-            shard.broadcast(pack_rff, src=rff_rank)
-            if full:
-                shard.broadcast(Lbuf, src=rff_rank)
-            mark("rff_received")
-        if rff is None:
-            rff = RFFFit()
-            rff.W, rff.b, rff.sigma_f, rff.Phi_X, rff.stats = W, b, float(theta[2]), None, None
-        rff.omega_map, rff.hess_diag, rff.L = pack_rff[:Fdim], pack_rff[Fdim:], Lbuf
-        if shard.rank != 0 and hi > lo:
-            fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=normals, covariance=weight_covariance)
-            mark("sampling")
-        if shard_mustar:
-            mustar = mu_star(gp, cand)
-            mu_t.copy_(mustar)
-        else:
-            if shard.rank == 0:
-                mu_t.copy_(mustar_over_candidates(gp, cand))
-            shard.broadcast(mu_t, src=0)
-        mark("mustar")
-        if shard.rank == 0 and hi > lo:
-            if grid_stream is not main:
-                main.wait_stream(grid_stream)
-                for t in grid_tensors():
-                    t.record_stream(main)
-            fmax, _ = rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, prepared=normals, covariance=weight_covariance)
-            mark("sampling")
-        sums = rff_reduce(fmax, mu_t, B, shard)
-        mark("acquisition")
-        if state is not None:
-            state.Q = Q
-        return sums, gp, rff
+    grid = _grid_stage(it, main)
+    it.mark("grid_features")
+    if it.shard.world > 1:
+        sums, gp, rff = _several_ranks(it, main, grid)
+    elif it.i8 and OVERLAP_SAMPLING:
+        sums, gp, rff = _one_gpu_overlapped(it, main, grid)
     else:
-        if shard.rank == 0:
-            gp = fit_gp()
-            mark("gp_fit")
-            mustar = mustar_over_candidates(gp, cand)
-            mark("mustar")
-        if shard.rank == rff_rank:
-            rff = fit_rff()
-            mark("rff_fit")
-    if shard.rank == rff_rank:
-        pack[:Fdim].copy_(rff.omega_map)
-        pack[Fdim:2 * Fdim].copy_(rff.hess_diag)
-    if shard.rank == 0:
-        pack[2 * Fdim:].copy_(mustar)
-    if rff_rank == 0:
-        shard.broadcast(pack, src=0)
-    else:
-        shard.broadcast(pack[:2 * Fdim], src=rff_rank)
-        shard.broadcast(pack[2 * Fdim:], src=0)
-    Lbuf = None
-    if full:
-        Lbuf = rff.L if shard.rank == rff_rank else ops.rff_hessian_factor_buffer(Fdim, dev)
-        shard.broadcast(Lbuf, src=rff_rank)
-        prepared = normals
-    if rff is None:
-        rff = RFFFit()
-        rff.W, rff.b, rff.sigma_f, rff.Phi_X, rff.stats = W, b, float(theta[2]), None, None
-    rff.omega_map, rff.hess_diag, rff.L = pack[:Fdim], pack[Fdim:2 * Fdim], Lbuf
-    if grid_stream is not main:
-        main.wait_stream(grid_stream)
-        for t in grid_tensors():
-            t.record_stream(main)
-    sums, fmax, arg = rff_acquisition(rff, PhiT, S, pack[2 * Fdim:], shard=shard, seed=seed, bounds=(lo, hi), prepared=prepared,
-                                      n_grids=B, covariance=weight_covariance)
-    mark("acquisition")
+        sums, gp, rff = _one_gpu_sequential(it, main, grid)
+    it.mark("acquisition")
     if state is not None:
         state.Q = Q
     return sums, gp, rff
+
+
+def _grid_stage(it, main):
+    """The grid features (and their digit planes, or the standard normals of the full covariance) of this rank's samples: they do
+    not depend on the fit.  On the rank that runs the latency-bound GP fit they go to a side stream and fill SMs the fit leaves
+    idle; the other ranks compute them while they wait for the broadcast.
+    Returns (stream, PhiT, normals, the tensors a stream that reads them must record)."""
+    stream = _side_stream(it.dev, tag="grid") if it.shard.rank == 0 else main
+    if stream is not main:
+        stream.wait_stream(main)
+    PhiT = normals = None
+    with torch.cuda.stream(stream):
+        if it.hi > it.lo:                                     # a rank without samples (rank 0 of several) needs no grid features
+            PhiT = rff_grid_features(it.W, it.b, it.theta[2], it.grids)
+            if it.full:
+                # the draws of the full covariance are plain standard normals: cut into digit planes before any fit ends; the grid
+                # features are sliced after their transform by the Hessian factor
+                normals = rff_prepare_normals(it.Fdim, it.lo, it.hi, it.P, it.dev, seed=it.seed)
+            elif it.i8:
+                PhiT = SlicedGrids(PhiT)                      # digit planes of the grid features
+    return stream, PhiT, normals, _device_tensors(PhiT, normals)
+
+
+def _one_gpu_overlapped(it, main, grid):
+    """One GPU, INT8 engine.  Two chains that only share X:
+      A  GP fit -> mu*                                   latency-bound, short (8.7 ms cold / 5 ms appended when alone)
+      B  weight-space fit -> draws -> contraction        the contraction alone keeps every tensor pipe busy for ~9 ms
+    B is the longer one and its head (the weight-space fit) is as latency-bound as A, so B runs in the FOREGROUND (this thread, on a
+    stream above the default priority) and A on the persistent background thread whose streams all sit at the lowest priority; the
+    contraction's persistent grid leaves OVERLAP_RESERVED_SMS SMs free, where A finishes while the tensor pipes of the other SMs are
+    busy.  Only the reduction (3 B sums) needs both chains."""
+    grid_stream, PhiT, normals, grid_tensors = grid
+    bg = _side_stream(it.dev)
+    bg.wait_stream(main)
+    fg = _side_stream(it.dev, priority=FOREGROUND_PRIORITY, tag="fg")
+    fg.wait_stream(main)
+
+    def gp_chain():
+        torch.cuda.set_device(it.dev)
+        with torch.cuda.stream(bg):
+            g = it.fit_gp()
+            return g, mustar_over_candidates(g, it.cand)
+    fut = _background_worker().submit(gp_chain)
+    lib = ops._lib.load()
+    try:
+        with torch.cuda.stream(fg):
+            rff = it.fit_rff()
+            it.mark("rff_fit")
+            transformed = None
+            if it.full:
+                _join(fg, grid_stream, grid_tensors)
+                prepared = normals
+                transformed = rff_transform_grids(rff, PhiT, slices=SAMPLING_SLICES)
+                it.mark("grid_transform")
+            else:
+                prepared = rff_prepare_samples(rff, it.lo, it.hi, it.P, seed=it.seed)
+                _join(fg, grid_stream, grid_tensors)
+            lib.ppbo_set_tuning(14, OVERLAP_RESERVED_SMS if it.warm else OVERLAP_RESERVED_SMS_COLD)
+            try:
+                fmax, _ = rff_sampled_maxima(rff, PhiT, it.lo, it.hi, seed=it.seed, prepared=prepared, covariance=it.covariance,
+                                             transformed=transformed)
+            finally:
+                lib.ppbo_set_tuning(14, 0)
+            it.mark("sampling")
+    finally:
+        gp, mustar = fut.result()          # re-raises on this thread
+    _join(main, bg, _gp_tensors(gp) + [mustar])
+    _join(main, fg, _rff_tensors(rff) + [fmax])
+    it.mark("gp_tail")                     # what is left of the GP fit + mu* after the contraction has finished
+    return rff_reduce(fmax, mustar, it.B, it.shard), gp, rff
+
+
+def _one_gpu_sequential(it, main, grid):
+    """One GPU, FP64 engine (or OVERLAP_SAMPLING off): the two fits only share X and are both chains of small, latency-bound launches
+    with one host decision per Newton step.  The GP fit runs in the foreground; the weight-space fit and its draws on the
+    background thread, whose streams all sit at the lowest priority, so they only take the SMs the GP fit leaves idle.  The
+    weight-space fit then starts from omega = 0 (or the caller's omega0) instead of the projection of the GP mode, which costs one
+    extra Newton step (20 against 19 on the Ackley-20D bench problem).  The contraction follows both fits."""
+    grid_stream, PhiT, normals, grid_tensors = grid
+    side = _side_stream(it.dev)
+    side.wait_stream(main)
+    fg = _side_stream(it.dev, priority=FOREGROUND_PRIORITY, tag="fg")
+    fg.wait_stream(main)
+
+    def weight_space_fit():
+        torch.cuda.set_device(it.dev)
+        with torch.cuda.stream(side):
+            fit = it.fit_rff()
+            # the draws and their digit planes need this fit only: done here, behind the GP fit (the standard normals of the
+            # full covariance are already on the grid stream)
+            return fit, (normals if it.full else rff_prepare_samples(fit, it.lo, it.hi, it.P, seed=it.seed))
+    fut = _background_worker().submit(weight_space_fit)
+    try:
+        with torch.cuda.stream(fg):
+            gp = it.fit_gp()
+            it.mark("gp_fit")
+            mustar = mustar_over_candidates(gp, it.cand)
+            it.mark("mustar")
+    finally:
+        rff, prepared = fut.result()       # re-raises on this thread
+    _join(main, fg, _gp_tensors(gp) + [mustar])
+    _join(main, side, _rff_tensors(rff) + _device_tensors(prepared))
+    it.mark("rff_fit")                     # what is left of the weight-space fit after the GP fit has finished
+    _join(main, grid_stream, grid_tensors)
+    sums, _, _ = rff_acquisition(rff, PhiT, it.S, mustar, shard=it.shard, seed=it.seed, bounds=(it.lo, it.hi), prepared=prepared,
+                                 n_grids=it.B, covariance=it.covariance)
+    return sums, gp, rff
+
+
+def _several_ranks(it, main, grid):
+    """Several ranks: rank 0 runs the GP fit; rank 1 runs the weight-space fit and broadcasts it; every rank with a sample share
+    draws and evaluates its samples as soon as the weight-space fit has arrived (the contraction needs that fit only) -- rank 0
+    after its GP fit; when mu* is known only the reduction and the all-reduce of 3 B doubles are left."""
+    grid_stream, PhiT, normals, grid_tensors = grid
+    shard, Fdim, full = it.shard, it.Fdim, it.full
+    rff_rank = _weight_space_rank(shard.world)
+    pack = torch.empty(2 * Fdim + 1, dtype=F64, device=it.dev)
+    pack_rff, mu_t = pack[:2 * Fdim], pack[2 * Fdim:]
+    gp = rff = fmax = None
+    Lbuf = ops.rff_hessian_factor_buffer(Fdim, it.dev) if full and shard.rank != rff_rank else None
+    if shard.rank == 0:
+        bstream = _side_stream(it.dev, tag="bcast")     # rank 0 joins the first broadcast off its critical path
+        bstream.wait_stream(main)
+        pack.record_stream(bstream)
+        with torch.cuda.stream(bstream):
+            shard.broadcast(pack_rff, src=rff_rank)
+            if full:
+                Lbuf.record_stream(bstream)
+                shard.broadcast(Lbuf, src=rff_rank)
+        gp = it.fit_gp()
+        it.mark("gp_fit")
+        main.wait_stream(bstream)
+    else:
+        if shard.rank == rff_rank:
+            rff = it.fit_rff()
+            it.mark("rff_fit")
+            pack_rff[:Fdim].copy_(rff.omega_map)
+            pack_rff[Fdim:].copy_(rff.hess_diag)
+            Lbuf = rff.L
+        shard.broadcast(pack_rff, src=rff_rank)
+        if full:
+            shard.broadcast(Lbuf, src=rff_rank)
+        it.mark("rff_received")
+    if rff is None:                                     # the weight-space fit as received: no features of the design, no statistics
+        rff = RFFFit()
+        rff.W, rff.b, rff.sigma_f, rff.Phi_X, rff.stats = it.W, it.b, float(it.theta[2]), None, None
+    rff.omega_map, rff.hess_diag, rff.L = pack_rff[:Fdim], pack_rff[Fdim:], Lbuf
+    if shard.rank != 0 and it.hi > it.lo:
+        fmax, _ = rff_sampled_maxima(rff, PhiT, it.lo, it.hi, seed=it.seed, prepared=normals, covariance=it.covariance)
+        it.mark("sampling")
+    if it.shard_mustar:
+        mu_t.copy_(_sharded_mustar(it, gp))
+    else:
+        if shard.rank == 0:
+            mu_t.copy_(mustar_over_candidates(gp, it.cand))
+        shard.broadcast(mu_t, src=0)
+    it.mark("mustar")
+    if shard.rank == 0 and it.hi > it.lo:
+        _join(main, grid_stream, grid_tensors)
+        fmax, _ = rff_sampled_maxima(rff, PhiT, it.lo, it.hi, seed=it.seed, prepared=normals, covariance=it.covariance)
+        it.mark("sampling")
+    return rff_reduce(fmax, mu_t, it.B, shard), gp, rff
+
+
+def _sharded_mustar(it, gp):
+    """max posterior mean over the design rows and the candidate points, every rank taking a slice of the candidates: alpha and
+    max f_MAP travel by broadcast from rank 0 and one all-reduce(max) follows"""
+    shard, N = it.shard, it.Q * (it.m + 1)
+    pack_a = torch.empty(N + 1, dtype=F64, device=it.dev)          # alpha and max f_MAP
+    if shard.rank == 0:
+        pack_a[:N].copy_(gp.alpha)
+        ops.vec_max(gp.f_map, out=pack_a[N:])
+    shard.broadcast(pack_a, src=0)
+    lo_c, hi_c = shard.bounds(it.cand.shape[0])
+    out = pack_a[N:].clone()
+    if hi_c > lo_c:
+        Xd = it.state.design(it.Q) if it.state is not None else it.X
+        mu = ops.posterior_mean(it.kernel, Xd, it.theta[1], it.theta[2], pack_a[:N], it.cand[lo_c:hi_c])
+        ops.vec_max(mu, out=out, accumulate=True)
+    shard.all_reduce_max(out)
+    return out

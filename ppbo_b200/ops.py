@@ -649,14 +649,6 @@ def rff_fit(Phi_X, Q, m, sigma, omega0=None, max_iter=100, tol=1e-10, factor_cac
                            binv_cached=bool(stats[4]))
 
 
-def rff_refactor(Phi_X, Q, m, sigma, omega, factor_cache):
-    """Hessian factor + block inverses at omega into factor_cache, asynchronously on the current stream (ppbo_rff_refactor)"""
-    F = Phi_X.shape[0]
-    ws, wbytes = _rff_ws(F, Q, m, Phi_X.device)
-    check(_lib.load().ppbo_rff_refactor(_p(Phi_X), Phi_X.stride(0), F, Q, m, float(sigma), _p(omega), _p(factor_cache), _p(ws), wbytes,
-                                        _stream()), "ppbo_rff_refactor")
-
-
 def rff_hessian_factor_buffer(F, dev):
     """flat buffer for rff_hessian_factor: the F x F factor followed by the inverted 128-blocks its solves read"""
     return torch.empty(_lib.load().ppbo_rff_hessian_factor_doubles(F, F), dtype=F64, device=dev)

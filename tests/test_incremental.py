@@ -190,25 +190,3 @@ def test_mu_pred_point(ops, golden):
     assert np.abs(got - ref).max() <= 1e-11 * max(np.abs(ref).max(), 1e-300) + 1e-13 * float(fit.alpha.abs().sum())
     assert pm.calls == len(pts)
 
-
-def test_rff_factor_refresh(ops, golden):
-    """RFFState.refresh_factor (ppbo_rff_refactor): the Hessian factor rebuilt asynchronously at the optimum lets the next appended
-    fit run on chord steps alone and reach the optimum a from-scratch fit finds"""
-    from ppbo_b200 import iteration
-    g = golden
-    if "rff_W" not in g:
-        pytest.skip("no RFF recordings for this kernel")
-    Q, m, theta = g["Q"], g["m"], g["theta"]
-    X = ops.to_dev(g["X"])
-    W, b = ops.to_dev(g["rff_W"]), ops.to_dev(g["rff_b"])
-    n1 = (Q - 1) * (m + 1)
-    st = iteration.RFFState(W, b, theta, m, Q, tol=1e-10)
-    st.cold(X[:n1])
-    st.refresh_factor()
-    r = st.append(X[n1:])
-    torch.cuda.synchronize()
-    # (on these 7-set problems one appended set changes the optimum by O(1): the fit may still refactor; at the bench size the
-    # refreshed factor carries the whole fit -- scripts/timeline.py with PPBO_RFF_REFRESH=1)
-    assert r.stats["info"] == 0 and r.stats["chord_steps"] >= 1
-    ref = iteration.rff_fit(X, W, b, theta, Q, m, tol=1e-10)
-    assert relerr(_np(r.omega_map), _np(ref.omega_map)) < 1e-7

@@ -110,15 +110,6 @@ def check_rff_cache(env, cache, F, what="rff"):
     return L
 
 
-def _rff_hessian(O, PhiX, Q, m, sigma, w):
-    """I + Psi' a+(w) Psi with Psi formed on the host from Phi_X (the clamped Hessian the weight-space factor belongs to)"""
-    F = PhiX.shape[0]
-    D3 = O._rff_diffs(PhiX, Q, m).reshape(F, Q * m)
-    a = O.arrow_coeffs(PhiX.T @ w, Q, m, sigma).ravel()
-    Psi = D3 * np.sqrt(np.maximum(a, 0.0))[None, :]
-    return np.eye(F) + Psi @ Psi.T
-
-
 # ------------------------------------------------------------------------------------------------ references
 def _ref_omega(O, PhiX, Q, m, sigma, w0):
     """weight-space mode next to w0: Newton with the exact Hessian (make_full_fixtures.rff_tight) from w0.  After an append the
@@ -440,26 +431,3 @@ def test_weight_space_fit_below_feature_slices(env):
     r = it.rff_fit(ops.to_dev(Xh), ops.to_dev(Wh), ops.to_dev(bh), theta, Q, m, tol=1e-10)
     _check_rff_mode(env, r, w_ref, PhiX, Q, m, theta[0], "F = 7")
 
-
-# ------------------------------------------------------------------------------------------------ 4. ppbo_rff_refactor
-@pytest.mark.parametrize("F", [333, 1000, 1100])
-def test_rff_refactor_factor_and_block_inverses(env, F):
-    """the weight-space factor rebuilt at a given omega: L L' = I + Psi' a+(omega) Psi (Psi from Phi_X on the host, negative
-    coefficients clamped), its inverted 128-blocks and its 1024-block inverses (two blocks at F = 1100)"""
-    O, ops, syn = env["O"], env["ops"], env["syn"]
-    D, Q, m = 20, 40, 25
-    theta = ACKLEY_THETA
-    Xh, _, _ = syn.make_design(D, Q, m, seed=0)
-    rng = np.random.RandomState(F)
-    W, b = ops.to_dev(rng.randn(F, D) / theta[1]), ops.to_dev(rng.uniform(0, 2 * np.pi, F))
-    PhiX = ops.rff_features(W, b, ops.to_dev(Xh), theta[2], feature_major=True)
-    w = 0.3 * rng.randn(F)
-    cache = ops.rff_factor_cache(F, env["dev"])
-    ops.rff_refactor(PhiX, Q, m, theta[0], ops.to_dev(w), cache)
-    torch.cuda.synchronize()
-    H = _rff_hessian(O, _np(PhiX), Q, m, theta[0], w)
-    a = O.arrow_coeffs(_np(PhiX).T @ w, Q, m, theta[0])
-    assert (a < 0).any() and (a > 0).any()                    # the clamp of a+ is exercised
-    L = check_rff_cache(env, cache, F, "refactor F = %d" % F)
-    Lh = np.tril(_np(L))
-    assert np.abs(Lh @ Lh.T - H).max() <= 1e-12 * np.sqrt(F) * np.abs(H).max()
