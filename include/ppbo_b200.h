@@ -82,7 +82,8 @@ int ppbo_lik_terms(const double* f, int Q, int m, double sigma, double* lik_sum,
 int ppbo_lik_set_sums(const double* f, int Q, int m, double sigma, double* set_sums, void* stream);
 /* dense Lambda[N x N] from the arrow coefficients (public attr GPModel.Lambda_MAP) */
 int ppbo_lambda_dense(const double* arrow, int Q, int m, double* out, long long ld, void* stream);
-/* G[Qm x Qm] = B^T Sigma B, the prior covariance of the latent differences f_j - f_winner */
+/* G[Qm x Qm] = B^T Sigma B, the prior covariance of the latent differences f_j - f_winner.  Qm <= 65535 (one grid row per row of G;
+ * the same limit holds for ppbo_diffspace_gram_append, ppbo_laplace_fit and ppbo_laplace_refactor) */
 int ppbo_diffspace_gram(const double* Sigma, long long lds, int Q, int m, double* G, long long ldg, void* stream);
 
 /* the same for appended comparison sets: entries of G with a row or a column in [Q_old m, Q_new m), in place (bit-identical to
@@ -139,7 +140,7 @@ int ppbo_factor_extend(const double* G, long long ldg, int M_old, int M_new, dou
                        double sigma, double* Lfac, int cap, void* stream);
 
 /* out[N x N] = I + Sigma W (reference_sign = 0) or I - Sigma W = I + Sigma Lambda_MAP (reference_sign = 1: the matrix
- * GPModel.evidence factors, src/gp_model.py:301-302), W = B diag(arrow) B' with the SIGNED coefficients. */
+ * GPModel.evidence factors, src/gp_model.py:301-302), W = B diag(arrow) B' with the SIGNED coefficients.  N = Q (m+1) <= 65535. */
 int ppbo_evidence_matrix(const double* Sigma, long long lds, int Q, int m, const double* arrow, int reference_sign, double* out,
                          long long ldo, void* stream);
 
@@ -198,7 +199,8 @@ long long ppbo_predict_mean_workspace_bytes(int kind, int N, int P, int batch);
 /* Posterior mean and covariance on `batch` grids of P points each (Xp: [batch*P x D]).
  * mu = k*' alpha ; Sigma_p = reg(K**) - k*' (Sigma^-1 - Sigma^-1 Post Sigma^-1) k*  evaluated as
  * reg(K**) - Y'Y (+ low-rank term for negative arrow coefficients), Y = Lfac^-1 a+^1/2 B' k*.
- * Replaces GPModel.mu_Sigma_pred (src/gp_model.py:441-452).  mu: [batch*P], Sigma_p: [batch][P x P] (may be NULL). */
+ * Replaces GPModel.mu_Sigma_pred (src/gp_model.py:441-452).  mu: [batch*P], Sigma_p: [batch][P x P] (may be NULL).
+ * P * batch is not bounded by a launch dimension (the per-point kernels loop over grid rows). */
 /* Negative arrow coefficients at the mode (data that contradict the fit) make W = B a B' indefinite; the factor
  * object only carries a+ = max(a,0).  These three calls build the exact low-rank correction
  * (Woodbury on the r negative columns) that ppbo_predict adds: count (host sync; indices to idx_h), size, build. */

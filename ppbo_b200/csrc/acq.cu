@@ -22,27 +22,34 @@ int kernel_matrix_raw(int kind, const double* X1, int n1, const double* X2, int 
                       double sigma_f, double scale, double diag_add, double* out, long long ld, cudaStream_t st);
 
 // ---------------------------------------------------------------------------------------------- prediction helpers
+// The two kernels below take one grid row per prediction point p < PT = P batch and walk the rows in steps of gridDim.y, which
+// the launch caps at the hardware limit of 65535 (sampled_max_batch predicts P = 70 points for every (xi, x) pair).
+constexpr int PRED_GRID_Y = 65535;
 // Ut[p][u] = sa[u] * (Kc[p][r(u)] - Kc[p][w(u)]),  sa = sqrt(max(arrow,0))          (a+^1/2 B^T k*, one RHS per row)
 __global__ void __launch_bounds__(256) pred_diff_kernel(const double* __restrict__ Kc, long long ldk, int PT, int Q, int m,
                                                         const double* __restrict__ arrow, double* __restrict__ Ut,
                                                         long long ldu) {
-    const int u = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
     if (u >= Q * m) return;
     const int q = u / m, j = u % m;
     const long long w = (long long)q * (m + 1);
     const double a = arrow[u];
-    const double* k = Kc + (long long)p * ldk;
-    Ut[(long long)p * ldu + u] = a > 0.0 ? sqrt(a) * (k[w + 1 + j] - k[w]) : 0.0;
+    for (int p = blockIdx.y; p < PT; p += gridDim.y) {
+        const double* k = Kc + (long long)p * ldk;
+        Ut[(long long)p * ldu + u] = a > 0.0 ? sqrt(a) * (k[w + 1 + j] - k[w]) : 0.0;
+    }
 }
 // Ud[p][i] = Kc[p][r(u_i)] - Kc[p][w(u_i)] for the negative-coefficient indices u_i
 __global__ void pred_negdiff_kernel(const double* __restrict__ Kc, long long ldk, int PT, int m, const int* __restrict__ idx,
                                     int r, double* __restrict__ Ud, long long ldu) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= r) return;
     const int u = idx[i], q = u / m, j = u % m;
     const long long w = (long long)q * (m + 1);
-    const double* k = Kc + (long long)p * ldk;
-    Ud[(long long)p * ldu + i] = k[w + 1 + j] - k[w];
+    for (int p = blockIdx.y; p < PT; p += gridDim.y) {
+        const double* k = Kc + (long long)p * ldk;
+        Ud[(long long)p * ldu + i] = k[w + 1 + j] - k[w];
+    }
 }
 // rows of  a+^1/2 G[:, J-]  (transposed: one row per negative index) and  R0 = diag(1/|a_j|) - G[J-, J-]
 __global__ void neg_rows_kernel(const double* __restrict__ G, long long ldg, int M, const double* __restrict__ arrow,
@@ -767,7 +774,7 @@ extern "C" int ppbo_predict(int kind, const double* X, int N, int D, const doubl
     if ((rc = kernel_matrix_raw(kind, Xp, PT, X, N, D, lengthscales_h, sigma_f, 1.0, 0.0, Kc, N, st))) return rc;
     if (mu && (rc = gemv(Kc, N, PT, N, alpha, mu, st))) return rc;
     if (!Sigma_p) return PPBO_OK;
-    PPBO_CL pred_diff_kernel<<<dim3(ceil_div(M, 256), PT), 256, 0, st>>>(Kc, N, PT, Q, m, arrow, Ut, M);
+    PPBO_CL pred_diff_kernel<<<dim3(ceil_div(M, 256), std::min(PT, PRED_GRID_Y)), 256, 0, st>>>(Kc, N, PT, Q, m, arrow, Ut, M);
     PPBO_LAUNCH_CHECK();
     if ((rc = trsm_right_lower_t(Lfac, cap, M, Lfac + (long long)cap * cap, Ut, M, PT, st))) return rc;   // Yt = Ut L^-T
     for (int b = 0; b < batch; ++b) {     // reg(K**) per grid (diagonal shrinkage needs the square form)
@@ -787,7 +794,7 @@ extern "C" int ppbo_predict(int kind, const double* X, int N, int D, const doubl
         const int* idx = reinterpret_cast<const int*>(neg_corr);
         const double* Ht = neg_corr + (r + 1) / 2;
         const double* R = Ht + (long long)r * M;
-        PPBO_CL pred_negdiff_kernel<<<dim3(ceil_div(r, 128), PT), 128, 0, st>>>(Kc, N, PT, m, idx, r, Ud, r);
+        PPBO_CL pred_negdiff_kernel<<<dim3(ceil_div(r, 128), std::min(PT, PRED_GRID_Y)), 128, 0, st>>>(Kc, N, PT, m, idx, r, Ud, r);
         PPBO_LAUNCH_CHECK();
         GemmOperands g1{Ut, M, 0, Ht, M, 0, PT, r, M};
         StoreEpilogue e1{Ud, r, 0, -1.0, 1.0, 0, 0, 0};                                             // z = Ud - Yt Ht^T

@@ -776,6 +776,7 @@ int set_identity(double* A, long long ld, int n, cudaStream_t st) {
 int diffspace_gram(const double* S, long long lds, int Q, int m, double* G, long long ldg, cudaStream_t st) {
     const int M = Q * m;
     if (M <= 0) return PPBO_OK;
+    PPBO_REQUIRE(M <= 65535, "Q m above 65535 (one grid row per row of G)");
     dim3 grid(ceil_div(M, 256), M);
     PPBO_CL diffspace_gram_kernel<<<grid, 256, 0, st>>>(S, lds, Q, m, G, ldg);
     PPBO_LAUNCH_CHECK();
@@ -807,6 +808,7 @@ __global__ void __launch_bounds__(256) diffspace_gram_append_kernel(const double
 int diffspace_gram_append(const double* S, long long lds, int Q_old, int Q_new, int m, double* G, long long ldg, cudaStream_t st) {
     const int M_old = Q_old * m, M_new = Q_new * m;
     if (M_new <= M_old) return PPBO_OK;
+    PPBO_REQUIRE(M_new <= 65535, "Q m above 65535 (one grid row per row of G)");
     PPBO_CL diffspace_gram_append_kernel<<<dim3(ceil_div(M_new, 256), M_new), 256, 0, st>>>(S, lds, M_old, M_new, m, G, ldg);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
@@ -824,6 +826,7 @@ __global__ void __launch_bounds__(256) gram_mirror_kernel(double* __restrict__ o
 
 int newton_matrix(const double* G, long long ldg, int M, const double* sa, double* out, long long ldo, cudaStream_t st) {
     if (M <= 0) return PPBO_OK;
+    PPBO_REQUIRE(M <= 65535, "Q m above 65535 (one grid row per row of the Newton matrix)");
     dim3 grid(ceil_div(M, 256), M);
     PPBO_CL newton_matrix_kernel<<<grid, 256, 0, st>>>(G, ldg, M, sa, out, ldo);
     PPBO_LAUNCH_CHECK();

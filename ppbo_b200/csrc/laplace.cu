@@ -1013,6 +1013,7 @@ extern "C" int ppbo_lambda_dense(const double* arrow, int Q, int m, double* out,
 extern "C" int ppbo_evidence_matrix(const double* Sigma, long long lds, int Q, int m, const double* arrow, int reference_sign,
                                     double* out, long long ldo, void* stream) {
     PPBO_REQUIRE(Q >= 1 && m >= 1 && ldo >= (long long)Q * (m + 1), "shape");
+    PPBO_REQUIRE((long long)Q * (m + 1) <= 65535, "Q (m+1) above 65535 (one grid row per row of the output)");
     const int N = Q * (m + 1);
     PPBO_CL evidence_matrix_kernel<<<dim3(ceil_div(N, 256), N), 256, 0, (cudaStream_t)stream>>>(Sigma, lds, Q, m, arrow,
                                                                                                 reference_sign ? -1.0 : 1.0, out, ldo);

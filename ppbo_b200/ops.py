@@ -399,6 +399,9 @@ def predict(kernel, X, lengthscales, sigma_f, shrinkage, fit, Xp, P, batch, want
               lib.ppbo_predict_mean_workspace_bytes(_kind(kernel), N, P, batch))
     ws = _scratch("predict" if want_cov else "predict_mean", wbytes, dev)
     neg_corr = fit.neg_corr if want_cov else None            # the mean needs alpha only (no factor, no Woodbury term)
+    if want_cov and fit.info > 0:
+        # the Woodbury block of the negative coefficients has no Cholesky factor: there is no covariance to return
+        raise PPBOError("posterior precision not positive definite (info %d): no predictive covariance" % fit.info)
     Lfac = fit.Lfac if want_cov else None
     check(lib.ppbo_predict(_kind(kernel), _p(X), N, D, _ls(lengthscales, D), float(sigma_f), float(shrinkage), fit.Q, fit.m,
                            _p(fit.alpha), _p(fit.arrow), _p(Lfac), fit.cap, _p(neg_corr), fit.n_neg if want_cov else 0, _p(Xp), P,
