@@ -261,6 +261,21 @@ int ppbo_mvn_rowmax(const double* Z, long long ldz, long long strideZ, const dou
 int ppbo_acq_reduce(const double* fmax, int S, int batch, double mustar, double* out, void* stream);
 /* same with mu* read from device memory (no host round trip between the mu* search and the reduction) */
 int ppbo_acq_reduce_dev(const double* fmax, int S, int batch, const double* mustar_dev, double* out, void* stream);
+/* Greedy batch selection by joint expected improvement (q-EI) over the SAME draws behind fmax[batch][S]: the maxima of grid b and
+ * grid b' in sample s are values of one sampled function, so q-EI(A) = E_s[max(max_{b in A} fmax[b][s] - mu*, 0)].  Step k of q
+ * (no addition to the reference, which proposes one query; no host synchronisation between the steps):
+ *   ppbo_acq_batch_gain : gain[b] = sum_s max(max(cur[s], fmax[b][s]) - mu*, 0) for every candidate (mu* in device memory; cur is
+ *                         not read at k = 0), in the order of ppbo_acq_reduce_dev (step 0: its column 0, bit for bit);
+ *                         gain[batch] = S.  gain: batch + 1 doubles, which several ranks sum (one all-reduce) before the pick.
+ *   ppbo_acq_batch_pick : w = arg-max of gain[0..batch) over the candidates not in idx[0..k), lowest index on ties; idx[k] = w,
+ *                         val[k] = gain[w] / gain[batch] (the joint EI of the first k+1 picks), cur[s] = max(cur[s], fmax[w][s])
+ *                         (k = 0: cur = fmax[w]).  S = 0 (a rank without samples) picks without touching cur or fmax.
+ * Both: argument error unless 0 <= k < q <= batch <= PPBO_ACQ_BATCH_MAX; ppbo_acq_batch_gain also needs S >= 1 and mu*. */
+#define PPBO_ACQ_BATCH_MAX 65535
+int ppbo_acq_batch_gain(const double* fmax, int S, int batch, const double* mustar_dev, const double* cur, int k, int q,
+                        double* gain, void* stream);
+int ppbo_acq_batch_pick(const double* gain, int batch, const double* fmax, int S, int k, int q, int* idx, double* val, double* cur,
+                        void* stream);
 /* out[0] = max_i x[i] (accumulate != 0: also over the previous out[0]).  Batched candidate form of the max the reference's
  * GPModel.mu_star looks for (src/gp_model.py:415-437): mu* over a set of candidate points. */
 int ppbo_vec_max(const double* x, long long n, int accumulate, double* out, void* stream);

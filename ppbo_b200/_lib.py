@@ -76,6 +76,8 @@ _SIGNATURES = {
     "ppbo_mvn_rowmax": (_I, [_P, _L, _L, _P, _L, _L, _P, _L, _I, _I, _I, _I, _P, _P, _P]),
     "ppbo_acq_reduce": (_I, [_P, _I, _I, _D, _P, _P]),
     "ppbo_acq_reduce_dev": (_I, [_P, _I, _I, _P, _P, _P]),
+    "ppbo_acq_batch_gain": (_I, [_P, _I, _I, _P, _P, _I, _I, _P, _P]),
+    "ppbo_acq_batch_pick": (_I, [_P, _I, _P, _I, _I, _I, _P, _P, _P, _P]),
     "ppbo_vec_max": (_I, [_P, _L, _I, _P, _P]),
     "ppbo_rff_features": (_I, [_P, _P, _I, _I, _P, _I, _D, _P, _L, _I, _P]),
     "ppbo_rff_jacobian": (_I, [_P, _P, _I, _I, _P, _D, _P, _P]),

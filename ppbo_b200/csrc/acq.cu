@@ -94,6 +94,83 @@ __global__ void __launch_bounds__(1024) acq_reduce_kernel(const double* __restri
     }
 }
 
+// ---- greedy batch selection (q-EI over the shared draws) ----------------------------------------------------------------------
+// gain[b] = sum_s max(max(cur[s], fm[b][s]) - mu*, 0) with cur = the per-sample max of the lines chosen so far (k == 0: none, cur
+// is not read).  The strided order and block_sum of acq_reduce_kernel, so that step 0 equals its column 0 bit for bit.
+// gain[batch] = S: the number of samples the gains sum over (summed with them over the ranks; the pick divides by it).
+__global__ void __launch_bounds__(1024) acq_batch_gain_kernel(const double* __restrict__ fm, int S, int batch,
+                                                              const double* __restrict__ mustar_dev, const double* __restrict__ cur,
+                                                              int k, double* __restrict__ gain) {
+    __shared__ double red[33];
+    const double mustar = mustar_dev[0];
+    const double* x = fm + (long long)blockIdx.x * S;
+    double s0 = 0;
+    for (int i = threadIdx.x; i < S; i += 1024) {
+        double v = x[i];
+        if (k > 0) v = fmax(cur[i], v);
+        s0 += fmax(v - mustar, 0.0);
+    }
+    s0 = block_sum(s0, red);
+    if (threadIdx.x == 0) {
+        gain[blockIdx.x] = s0;
+        if (blockIdx.x == 0) gain[batch] = (double)S;
+    }
+}
+
+// Step k of the greedy selection: w = arg-max of gain over the candidates not in idx[0..k) (lowest index on ties), idx[k] = w,
+// val[k] = gain[w] / gain[batch], cur[s] = max(cur[s], fm[w][s]) (k == 0: cur = fm[w]).  Every CTA recomputes the same arg-max
+// over the B gains with its own chosen mask in shared memory, built from idx[0..k) (written by earlier launches: CTA 0 writing
+// idx[k] races with nobody), and updates its own slice of cur.
+constexpr int PICK_THREADS = 256;
+__global__ void __launch_bounds__(PICK_THREADS) acq_batch_pick_kernel(const double* __restrict__ gain, int batch,
+                                                                      const double* __restrict__ fm, int S, int k,
+                                                                      int* __restrict__ idx, double* __restrict__ val,
+                                                                      double* __restrict__ cur) {
+    __shared__ unsigned chosen[(PPBO_ACQ_BATCH_MAX + 31) / 32];
+    __shared__ double wv[PICK_THREADS / 32];
+    __shared__ int wi[PICK_THREADS / 32];
+    __shared__ int win_s;
+    const int nwords = (batch + 31) >> 5, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int i = threadIdx.x; i < nwords; i += PICK_THREADS) chosen[i] = 0u;
+    __syncthreads();
+    for (int j = threadIdx.x; j < k; j += PICK_THREADS) {
+        const int c = idx[j];
+        atomicOr(&chosen[c >> 5], 1u << (c & 31));
+    }
+    __syncthreads();
+    // bi < 0: nothing seen yet (the first unchosen candidate is taken whatever its gain, so a NaN cannot leave the pick empty)
+    double bv = -INFINITY;
+    int bi = -1;
+    for (int c = threadIdx.x; c < batch; c += PICK_THREADS) {
+        if ((chosen[c >> 5] >> (c & 31)) & 1u) continue;
+        const double g = gain[c];
+        if (bi < 0 || g > bv) { bv = g; bi = c; }           // increasing c: a tie keeps the lower index
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (oi >= 0 && (bi < 0 || ov > bv || (ov == bv && oi < bi))) { bv = ov; bi = oi; }
+    }
+    if (lane == 0) { wv[warp] = bv; wi[warp] = bi; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < PICK_THREADS / 32; ++w)
+            if (wi[w] >= 0 && (bi < 0 || wv[w] > bv || (wv[w] == bv && wi[w] < bi))) { bv = wv[w]; bi = wi[w]; }
+        win_s = bi;
+        if (blockIdx.x == 0) {
+            idx[k] = bi;
+            val[k] = bv / gain[batch];
+        }
+    }
+    __syncthreads();
+    const int w = win_s;
+    const int s = blockIdx.x * PICK_THREADS + threadIdx.x;
+    if (s < S) {
+        const double v = fm[(long long)w * S + s];
+        cur[s] = k > 0 ? fmax(cur[s], v) : v;
+    }
+}
+
 // out[0] = max(init, max_i x[i]) with init = out[0] if `accumulate` (single CTA; used for mu* over candidate points)
 __global__ void __launch_bounds__(1024) vec_max_kernel(const double* __restrict__ x, long long n, int accumulate,
                                                        double* __restrict__ out) {
@@ -826,6 +903,28 @@ extern "C" int ppbo_acq_reduce(const double* fmax, int S, int batch, double must
 extern "C" int ppbo_acq_reduce_dev(const double* fmax, int S, int batch, const double* mustar_dev, double* out, void* stream) {
     PPBO_REQUIRE(S >= 1 && batch >= 1 && mustar_dev != nullptr, "shape");
     PPBO_CL acq_reduce_kernel<<<batch, 1024, 0, (cudaStream_t)stream>>>(fmax, S, 0.0, mustar_dev, out);
+    PPBO_LAUNCH_CHECK();
+    return PPBO_OK;
+}
+
+extern "C" int ppbo_acq_batch_gain(const double* fmax, int S, int batch, const double* mustar_dev, const double* cur, int k, int q,
+                                   double* gain, void* stream) {
+    PPBO_REQUIRE(S >= 1 && batch >= 1 && mustar_dev != nullptr, "shape");
+    PPBO_REQUIRE(batch <= PPBO_ACQ_BATCH_MAX, "more candidates than one selection takes");
+    PPBO_REQUIRE(q >= 1 && q <= batch && k >= 0 && k < q, "need 0 <= k < q <= batch");
+    PPBO_REQUIRE(k == 0 || cur != nullptr, "cur missing");
+    PPBO_CL acq_batch_gain_kernel<<<batch, 1024, 0, (cudaStream_t)stream>>>(fmax, S, batch, mustar_dev, cur, k, gain);
+    PPBO_LAUNCH_CHECK();
+    return PPBO_OK;
+}
+
+extern "C" int ppbo_acq_batch_pick(const double* gain, int batch, const double* fmax, int S, int k, int q, int* idx, double* val,
+                                   double* cur, void* stream) {
+    PPBO_REQUIRE(S >= 0 && batch >= 1 && (S == 0 || (fmax != nullptr && cur != nullptr)), "shape");
+    PPBO_REQUIRE(batch <= PPBO_ACQ_BATCH_MAX, "more candidates than one selection takes");
+    PPBO_REQUIRE(q >= 1 && q <= batch && k >= 0 && k < q, "need 0 <= k < q <= batch");
+    PPBO_CL acq_batch_pick_kernel<<<std::max(1, ceil_div(S, PICK_THREADS)), PICK_THREADS, 0, (cudaStream_t)stream>>>(
+        gain, batch, fmax, S, k, idx, val, cur);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;
 }

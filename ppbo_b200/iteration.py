@@ -501,6 +501,31 @@ def rff_acquisition(r, PhiT, S, mustar_dev, shard=None, Z=None, seed=0, stream_i
     return rff_reduce(fmax, mustar_dev, n_grids, shard), fmax, arg
 
 
+def select_batch(fmax, mustar_dev, q, n_grids, shard=None):
+    """q query lines by greedy joint expected improvement over the draws behind fmax [B, S_loc] (this rank's samples; None on a
+    rank without samples): step k adds the line that raises E_s[max(max_{b in chosen} fmax[b][s] - mu*, 0)] most, lowest index on
+    ties.  The maxima of all lines in one sample come from the same sampled function, so a line that reaches the same peak as a
+    chosen one adds nothing.  Returns (idx [q] int32, qei [q]) on the device, qei[k] = the joint EI of the first k+1 picks.
+    With several ranks every step's gains go through one all-reduce of B + 1 doubles (the last one counts the samples), so all
+    ranks pick the same lines; every rank joins every collective."""
+    shard = shard or Shard()
+    if not 1 <= q <= n_grids:
+        raise PPBOError("batch size q must be in [1, %d], not %r" % (n_grids, q))
+    dev = mustar_dev.device
+    idx = torch.empty(q, dtype=torch.int32, device=dev)
+    qei = torch.empty(q, dtype=F64, device=dev)
+    gain = torch.zeros(n_grids + 1, dtype=F64, device=dev)
+    cur = None if fmax is None else torch.empty(fmax.shape[1], dtype=F64, device=dev)
+    for k in range(q):
+        if fmax is not None:
+            ops.acq_batch_gain(fmax, mustar_dev, cur, k, q, out=gain)
+        shard.all_reduce_sum(gain)
+        ops.acq_batch_pick(gain, fmax, k, q, idx, qei, cur)
+        if fmax is None:
+            gain.zero_()                 # this rank's share of the next step's sums
+    return idx, qei
+
+
 def acquisition_values(sums, S):
     """host: EI and variance-of-max per grid from the reduced sums (src/acquisition.py:81,178)."""
     s = np.asarray(sums, dtype=float)
@@ -650,8 +675,9 @@ class _Iteration:
 
 
 def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, tol=1e-8, timers=None, state=None, shares=None,
-                  factor_at_mode=False, shard_mustar=None, weight_covariance="diag"):
-    """d: dict of device tensors (IterationInputs.to_device).  Returns (sums [B,3] device, gp, rff).
+                  factor_at_mode=False, shard_mustar=None, weight_covariance="diag", batch=None):
+    """d: dict of device tensors (IterationInputs.to_device).  Returns (sums [B,3] device, gp, rff); with batch=q also the q query
+    lines chosen by greedy joint expected improvement over the same draws (select_batch): (sums, gp, rff, (idx [q], qei [q])).
     Rank 0 fits; the others receive (omega_MAP, hess_diag, mu*) by broadcast while they compute the grid features.
     tol: both Newton iterations stop when the last full step is below tol relative to the iterate.  The chord steps contract
     by ~5x per step, so the distance to the mode is ~tol/4 = 2.5e-9 at the default: 400x inside the 1e-6 parity bound of
@@ -666,9 +692,13 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     weight_covariance: "diag" (the reference's) or "full" (WEIGHT_COVARIANCES): the rank that fits the weight space also factors the
     exact Hessian at omega_MAP and sends the factor with (omega_MAP, hess_diag); the draws are standard normals and every sampling
     rank transforms its grid features once (rff_transform_grids).
-    timers: a list that receives (name, CUDA event) marks between the stages of the schedule that ran."""
+    timers: a list that receives (name, CUDA event) marks between the stages of the schedule that ran.
+    batch: q >= 1 keeps this rank's per-sample maxima and runs the greedy selection after the reduction on every rank (inside the
+    "acquisition" stage); without it nothing of the result changes."""
     if weight_covariance not in WEIGHT_COVARIANCES:
         raise PPBOError("weight_covariance must be one of %s" % (WEIGHT_COVARIANCES,))
+    if batch is not None and not 1 <= batch <= d["grids"].shape[0]:
+        raise PPBOError("batch must be in [1, %d], not %r" % (d["grids"].shape[0], batch))
     it = _Iteration(d, kernel, theta, Q, m, S, shard or Shard(), seed, fit_iters, tol, timers, state, shares, factor_at_mode,
                     shard_mustar, weight_covariance)
     if state is not None:
@@ -681,15 +711,16 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     grid = _grid_stage(it, main)
     it.mark("grid_features")
     if it.shard.world > 1:
-        sums, gp, rff = _several_ranks(it, main, grid)
+        sums, gp, rff, fmax, mustar = _several_ranks(it, main, grid)
     elif it.i8 and OVERLAP_SAMPLING:
-        sums, gp, rff = _one_gpu_overlapped(it, main, grid)
+        sums, gp, rff, fmax, mustar = _one_gpu_overlapped(it, main, grid)
     else:
-        sums, gp, rff = _one_gpu_sequential(it, main, grid)
+        sums, gp, rff, fmax, mustar = _one_gpu_sequential(it, main, grid)
+    picks = select_batch(fmax, mustar, batch, it.B, it.shard) if batch is not None else None
     it.mark("acquisition")
     if state is not None:
         state.Q = Q
-    return sums, gp, rff
+    return (sums, gp, rff) if batch is None else (sums, gp, rff, picks)
 
 
 def _grid_stage(it, main):
@@ -759,7 +790,7 @@ def _one_gpu_overlapped(it, main, grid):
     _join(main, bg, _gp_tensors(gp) + [mustar])
     _join(main, fg, _rff_tensors(rff) + [fmax])
     it.mark("gp_tail")                     # what is left of the GP fit + mu* after the contraction has finished
-    return rff_reduce(fmax, mustar, it.B, it.shard), gp, rff
+    return rff_reduce(fmax, mustar, it.B, it.shard), gp, rff, fmax, mustar
 
 
 def _one_gpu_sequential(it, main, grid):
@@ -794,9 +825,9 @@ def _one_gpu_sequential(it, main, grid):
     _join(main, side, _rff_tensors(rff) + _device_tensors(prepared))
     it.mark("rff_fit")                     # what is left of the weight-space fit after the GP fit has finished
     _join(main, grid_stream, grid_tensors)
-    sums, _, _ = rff_acquisition(rff, PhiT, it.S, mustar, shard=it.shard, seed=it.seed, bounds=(it.lo, it.hi), prepared=prepared,
-                                 n_grids=it.B, covariance=it.covariance)
-    return sums, gp, rff
+    sums, fmax, _ = rff_acquisition(rff, PhiT, it.S, mustar, shard=it.shard, seed=it.seed, bounds=(it.lo, it.hi), prepared=prepared,
+                                    n_grids=it.B, covariance=it.covariance)
+    return sums, gp, rff, fmax, mustar
 
 
 def _several_ranks(it, main, grid):
@@ -851,7 +882,7 @@ def _several_ranks(it, main, grid):
         _join(main, grid_stream, grid_tensors)
         fmax, _ = rff_sampled_maxima(rff, PhiT, it.lo, it.hi, seed=it.seed, prepared=normals, covariance=it.covariance)
         it.mark("sampling")
-    return rff_reduce(fmax, mu_t, it.B, shard), gp, rff
+    return rff_reduce(fmax, mu_t, it.B, shard), gp, rff, fmax, mu_t
 
 
 def _sharded_mustar(it, gp):

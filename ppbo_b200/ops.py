@@ -798,6 +798,24 @@ def acq_reduce_dev(fmax, mustar_dev):
     return out
 
 
+def acq_batch_gain(fmax, mustar_dev, cur, k, q, out=None):
+    """gains [B + 1] of greedy step k over this rank's samples: gain[b] = sum_s max(max(cur[s], fmax[b][s]) - mu*, 0), gain[B] = S"""
+    B, S = fmax.shape
+    out = torch.empty(B + 1, dtype=F64, device=fmax.device) if out is None else out
+    check(_lib.load().ppbo_acq_batch_gain(_p(fmax), S, B, _p(mustar_dev), _p(cur), int(k), int(q), _p(out), _stream()),
+          "ppbo_acq_batch_gain")
+    return out
+
+
+def acq_batch_pick(gain, fmax, k, q, idx, val, cur):
+    """step k: idx[k] = best candidate not in idx[:k] (lowest index on ties), val[k] = gain[idx[k]] / gain[B], cur updated with its
+    maxima.  fmax None: a rank without samples (picks only)."""
+    B = gain.shape[0] - 1
+    S = 0 if fmax is None else fmax.shape[1]
+    check(_lib.load().ppbo_acq_batch_pick(_p(gain), B, _p(fmax), S, int(k), int(q), _p(idx), _p(val), _p(cur), _stream()),
+          "ppbo_acq_batch_pick")
+
+
 def vec_max(x, out=None, accumulate=False):
     out = torch.empty(1, dtype=F64, device=x.device) if out is None else out
     check(_lib.load().ppbo_vec_max(_p(x), x.numel(), 1 if accumulate else 0, _p(out), _stream()), "ppbo_vec_max")

@@ -153,6 +153,58 @@ def next_query(PPBO_settings, GP_model, unscale=True):
     return (xi_next, x_next)
 
 
+BATCH_STRATEGIES = ('EI-EXT-FAST', 'EI-VARMAX-FAST')
+
+
+def sampled_max_joint(pairs, GP_model, mc_samples):
+    """f_max on the 70-point grid of every (xi, x) in `pairs` from JOINT posterior draws over all B grids: one prediction of the
+    B*70 points with their cross-covariance, one device Cholesky factor L (jitter retry: lines through x* nearly share points),
+    f = mu + L z with z = np.random.standard_normal((S, B*70)) in one call.  RNG: the B grid jitters in order, then the S x B*70
+    normals.  Returns fmax [B, S] and, for checking, the grids [B, 70, D], Z [S, B*70], mu [B*70] and L (device)."""
+    B, S, P = len(pairs), int(mc_samples), GRID_POINTS
+    grids = np.empty((B, P, GP_model.D))
+    for b, (xi, x) in enumerate(pairs):
+        grids[b] = GP_model.FP.xi_grid(xi=xi, x=x, alpha_grid_distribution='equispaced', alpha_star=None, m=P, is_scaled=True)
+    Z = np.random.standard_normal((S, B * P))
+    mu, Sp = GP_model._predict_dev(ops.to_dev(grids.reshape(B * P, -1)), B * P, 1)
+    L = _device_factor(Sp)[0]
+    Zd = ops.to_dev(Z)
+    # grid b's rows of L are its points' coefficients on the B*70 joint normals: one row-max per grid over the shared draws
+    fmax, _arg = ops.mvn_rowmax(Zd.unsqueeze(0).expand(B, -1, -1), L.view(B, P, B * P), mu.view(B, P))
+    return fmax, grids, Z, mu.view(-1), L
+
+
+def next_query_batch(PPBO_settings, GP_model, q, unscale=True):
+    """q queries for evaluators who answer in parallel (no counterpart in the reference, which proposes one).  For the strategies
+    whose xi is a coordinate direction through x* ('EI-EXT-FAST', 'EI-VARMAX-FAST'): the D lines of EId_xstar, joint posterior
+    draws on all of them (sampled_max_joint), and q lines chosen greedily by joint expected improvement over those draws
+    (ppbo_b200.iteration.select_batch): a line that reaches the same peak as a chosen one adds nothing, where the top q by marginal
+    EI would take both.  Each chosen xi then gets its x from next_x_given_xi, in pick order.  Returns a list of q (xi, x) pairs,
+    normalised and unscaled as next_query does.
+    RNG consumption: the D grid jitters (reference order of _coordinate_pairs), one standard_normal((mc_samples, D*70)) call, then
+    whatever next_x_given_xi draws for each pick in turn (nothing for x_acquisition_function 'exploit')."""
+    from ppbo_b200 import iteration
+    name = PPBO_settings.xi_acquisition_function
+    if name not in BATCH_STRATEGIES:
+        raise ValueError("next_query_batch serves %s, not %r" % (BATCH_STRATEGIES, name))
+    xis, pairs = _coordinate_pairs(GP_model)
+    if not 1 <= q <= len(pairs):
+        raise ValueError("q must be in [1, %d], not %r" % (len(pairs), q))
+    fmax = sampled_max_joint(pairs, GP_model, PPBO_settings.mc_samples)[0]
+    mustar = ops.to_dev(np.array([float(GP_model.mustar)]))
+    idx, _qei = iteration.select_batch(fmax, mustar, q, len(pairs))
+    out = []
+    for b in idx.cpu().numpy():
+        xi_next = xis[int(b)].copy()
+        x_next = next_x_given_xi(xi_next, GP_model, PPBO_settings)
+        xi_next = np.abs(xi_next) / np.max(np.abs(xi_next))
+        if unscale:
+            xi_next = GP_model.FP.unscale(xi_next, retain_0_values=True)
+            x_next = GP_model.FP.unscale(x_next, retain_0_values=True)
+        out.append((xi_next, x_next))
+    return out
+
+
 def EI(xi, x, GP_model, mc_samples):
     """expected improvement of the projective query (xi, x) (src/acquisition.py:72-81)"""
     return float(_ei_values([(xi, x)], GP_model, mc_samples)[0])

@@ -231,9 +231,8 @@ class Hsampler:
         fmax, arg, _ = ops.rff_eval_argmax(Om, PhiT)
         return fmax.cpu().numpy(), arg.cpu().numpy()
 
-    def sample_max_over_grids(self, grids, n_samples, mustar, seed=0, shard=None):
-        """EI / varmax ingredients from RFF posterior draws: sums over the samples of max(fmax - mu*, 0), fmax, fmax^2 per grid
-        (reduced over all ranks of `shard`)."""
+    def _rff_fit(self):
+        """this sampler's fit as the iteration module's RFFFit (device tensors)"""
         rff = _it.RFFFit()
         rff.W, rff.b, rff.sigma_f = self._d("W"), self._d("b"), float(self.theta[2])
         rff.omega_map, rff.hess_diag = self._dev["omega_MAP"], self._dev["hess_diag"]
@@ -241,10 +240,27 @@ class Hsampler:
             if "L" not in self._dev:
                 raise ValueError("update_covariancematrix() first")
             rff.L = self._dev["L"]
+        return rff
+
+    def sample_max_over_grids(self, grids, n_samples, mustar, seed=0, shard=None):
+        """EI / varmax ingredients from RFF posterior draws: sums over the samples of max(fmax - mu*, 0), fmax, fmax^2 per grid
+        (reduced over all ranks of `shard`)."""
+        rff = self._rff_fit()
         PhiT = _it.rff_grid_features(rff.W, rff.b, rff.sigma_f, ops.to_dev(np.asarray(grids, dtype=np.float64)))
         sums, _, _ = _it.rff_acquisition(rff, PhiT, n_samples, ops.to_dev(np.array([float(mustar)])), shard=shard, seed=seed,
                                          covariance=self.covariance_form)
         return sums.cpu().numpy()
+
+    def select_batch_over_grids(self, grids, n_samples, mustar, q, seed=0, shard=None):
+        """q of the grids (query lines) by greedy joint expected improvement over the same RFF posterior draws
+        (iteration.select_batch): host arrays (idx [q], qei [q]), qei[k] = the joint EI of the first k+1 picks; the same on every
+        rank of `shard`."""
+        rff = self._rff_fit()
+        PhiT = _it.rff_grid_features(rff.W, rff.b, rff.sigma_f, ops.to_dev(np.asarray(grids, dtype=np.float64)))
+        lo, hi = (shard or _it.Shard()).bounds(n_samples)
+        fmax, _ = _it.rff_sampled_maxima(rff, PhiT, lo, hi, seed=seed, covariance=self.covariance_form)
+        idx, qei = _it.select_batch(fmax, ops.to_dev(np.array([float(mustar)])), q, PhiT.shape[0], shard=shard)
+        return idx.cpu().numpy(), qei.cpu().numpy()
 
     # ------------------------------------------------------------------ batched maximiser (north_star piece 3; SURVEY.md 8f rank 4)
     def return_xstar_batch(self, omegas, n_restarts=16, max_iter=500, gtol=1e-9):
