@@ -194,7 +194,8 @@ int ppbo_symv_lower(const double* A, long long lda, int n, const double* x, doub
 
 /* ---- K4: prediction and exact-GP acquisition ----------------------------------------------------- */
 long long ppbo_predict_workspace_bytes(int N, int Q, int m, int P, int batch);
-/* workspace of a mean-only call (Sigma_p == NULL): the SE / RQ tensor-pipe path never materialises the cross-covariance */
+/* workspace of a mean-only call (Sigma_p == NULL): the mat-vec mode of the SE / RQ / Matern / camphor kernels (camphor as an SE
+ * kernel on lifted coordinates) never materialises the cross-covariance */
 long long ppbo_predict_mean_workspace_bytes(int kind, int N, int P, int batch);
 /* Posterior mean and covariance on `batch` grids of P points each (Xp: [batch*P x D]).
  * mu = k*' alpha ; Sigma_p = reg(K**) - k*' (Sigma^-1 - Sigma^-1 Post Sigma^-1) k*  evaluated as
@@ -296,9 +297,12 @@ int ppbo_rff_value_grad(const double* W, const double* b, int F, int D, const do
 /* Maximisers of S sampled functions g_s(x) = phi(x)' Omega[s] over [0,1]^D, R restarts each from X0[S][R][D]: one CTA per
  * (sample, restart) runs projected gradient ascent (Barzilai-Borwein steps, Armijo backtracking) until the projected gradient is
  * below gtol or max_iter; xbest[S][D], fbest[S] = the best restart per sample.  work: S R (D + 1) doubles.  Batched form of
- * Hsampler.return_xstar / sample_xstar (src/random_fourier_sampler.py:143-178,215-220: sequential scipy L-BFGS-B restarts). */
+ * Hsampler.return_xstar / sample_xstar (src/random_fourier_sampler.py:143-178,215-220: sequential scipy L-BFGS-B restarts).
+ * periodic_mask: bit d set = coordinate d has period 1 (the camphor kernel's basis: 0b111011); such a coordinate is reduced modulo
+ * 1 after every step instead of being projected, and its whole gradient counts in the stationarity test.  0: the box [0,1]^D. */
 int ppbo_rff_maximize(const double* W, const double* b, int F, int D, double sigma_f, const double* Omega, long long ldo, int S,
-                      const double* X0, int R, int max_iter, double gtol, double* xbest, double* fbest, double* work, void* stream);
+                      const double* X0, int R, int max_iter, double gtol, int periodic_mask, double* xbest, double* fbest,
+                      double* work, void* stream);
 /* weight-space objective pieces (Hsampler.S / S_grad / S_hessian, src/random_fourier_sampler.py:106-122):
  * f = Phi_X' omega (Phi_X feature-major [F x N]); S = -1/2|omega|^2 - lik_sum/m (host double); grad[F];
  * hess_diag[F] (the reference Hessian is diagonal).  Any output may be NULL. */

@@ -82,7 +82,7 @@ _SIGNATURES = {
     "ppbo_rff_features": (_I, [_P, _P, _I, _I, _P, _I, _D, _P, _L, _I, _P]),
     "ppbo_rff_jacobian": (_I, [_P, _P, _I, _I, _P, _D, _P, _P]),
     "ppbo_rff_value_grad": (_I, [_P, _P, _I, _I, _P, _P, _D, _P, _P]),
-    "ppbo_rff_maximize": (_I, [_P, _P, _I, _I, _D, _P, _L, _I, _P, _I, _I, _D, _P, _P, _P, _P]),
+    "ppbo_rff_maximize": (_I, [_P, _P, _I, _I, _D, _P, _L, _I, _P, _I, _I, _D, _I, _P, _P, _P, _P]),
     "ppbo_rff_workspace_bytes": (_L, [_I, _I, _I]),
     "ppbo_rff_objective": (_I, [_P, _L, _I, _I, _I, _D, _P, _PD, _P, _P, _P, _L, _P]),
     "ppbo_rff_factor_cache_doubles": (_L, [_I]),

@@ -18,6 +18,7 @@ namespace ppbo {
 extern int g_tuning[16];
 int kernel_matvec(int kind, const double* X1, int n1, const double* X2, int n2, int D, const double* ls_h, double sigma_f,
                   const double* alpha, double* mu, double* partial, cudaStream_t st);
+bool km_has_matvec(int kind);
 int kernel_matrix_raw(int kind, const double* X1, int n1, const double* X2, int n2, int D, const double* ls_h,
                       double sigma_f, double scale, double diag_add, double* out, long long ld, cudaStream_t st);
 
@@ -257,13 +258,16 @@ __global__ void __launch_bounds__(256) rff_value_grad_kernel(const double* __res
 // pair is one CTA: projected gradient ascent with Barzilai-Borwein step lengths and Armijo backtracking on the box, the objective and
 // its gradient evaluated together (each thread owns F / 128 features; one block reduction of D + 1 numbers per evaluation).
 // Stationarity is measured by the projected gradient |clip(x + grad) - x|_inf.  A second kernel keeps the best restart per sample.
+// Coordinates with their bit set in `periodic` have period 1 (the sampled functions of a periodic kernel's basis are exactly
+// periodic there): a step reduces them modulo 1 instead of projecting them, the Armijo slope and the Barzilai-Borwein pair use the
+// unwrapped step, and their full gradient counts in the stationarity measure.  periodic = 0 is plain projected ascent on the box.
 constexpr int RM_THREADS = 128, RM_MAX_D = 32;
 __global__ void __launch_bounds__(RM_THREADS) rff_maximize_kernel(const double* __restrict__ W, const double* __restrict__ b, int F, int D,
                                                                   double amp, const double* __restrict__ Omega, long long ldo,
                                                                   const double* __restrict__ X0, int R, int max_iter, double gtol,
-                                                                  double* __restrict__ xout, double* __restrict__ fout,
-                                                                  int* __restrict__ iters_out) {
-    __shared__ double x[RM_MAX_D], g[RM_MAX_D], xt[RM_MAX_D], gt[RM_MAX_D];
+                                                                  unsigned periodic, double* __restrict__ xout,
+                                                                  double* __restrict__ fout, int* __restrict__ iters_out) {
+    __shared__ double x[RM_MAX_D], g[RM_MAX_D], xt[RM_MAX_D], gt[RM_MAX_D], sx[RM_MAX_D];
     __shared__ double red[RM_THREADS / 32][RM_MAX_D + 1];
     __shared__ double fval_s;
     const int s = blockIdx.x / R, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -306,7 +310,8 @@ __global__ void __launch_bounds__(RM_THREADS) rff_maximize_kernel(const double* 
         }
         __syncthreads();
     };
-    if (tid < D) x[tid] = fmin(fmax(x0[tid], 0.0), 1.0);
+    const bool wrap = (periodic >> (tid & 31)) & 1u;    // this thread's coordinate (tid < D) is periodic
+    if (tid < D) x[tid] = wrap ? x0[tid] - floor(x0[tid]) : fmin(fmax(x0[tid], 0.0), 1.0);
     __syncthreads();
     eval(x, g);
     double f = fval_s;
@@ -316,16 +321,25 @@ __global__ void __launch_bounds__(RM_THREADS) rff_maximize_kernel(const double* 
     int it = 0;
     for (; it < max_iter; ++it) {
         double pg = 0.0;                                // projected-gradient stationarity measure
-        for (int d = 0; d < D; ++d) pg = fmax(pg, fabs(fmin(fmax(x[d] + g[d], 0.0), 1.0) - x[d]));
+        for (int d = 0; d < D; ++d) pg = fmax(pg, ((periodic >> d) & 1u) ? fabs(g[d]) : fabs(fmin(fmax(x[d] + g[d], 0.0), 1.0) - x[d]));
         if (pg <= gtol) break;
         double ft = f, slope = 0.0;
         int tries = 0;
         for (;; ++tries) {
             __syncthreads();
-            if (tid < D) xt[tid] = fmin(fmax(x[tid] + t * g[tid], 0.0), 1.0);
+            if (tid < D) {
+                const double v = x[tid] + t * g[tid];
+                if (wrap) {
+                    xt[tid] = v - floor(v);
+                    sx[tid] = v - x[tid];
+                } else {
+                    xt[tid] = fmin(fmax(v, 0.0), 1.0);
+                    sx[tid] = xt[tid] - x[tid];
+                }
+            }
             __syncthreads();
             slope = 0.0;
-            for (int d = 0; d < D; ++d) slope = fma(g[d], xt[d] - x[d], slope);
+            for (int d = 0; d < D; ++d) slope = fma(g[d], sx[d], slope);
             eval(xt, gt);
             ft = fval_s;
             if (ft >= f + 1e-4 * slope || tries >= 30) break;
@@ -334,7 +348,7 @@ __global__ void __launch_bounds__(RM_THREADS) rff_maximize_kernel(const double* 
         if (!(ft >= f)) break;                          // no ascent possible at this resolution
         double ss = 0.0, sy = 0.0;
         for (int d = 0; d < D; ++d) {
-            const double sd = xt[d] - x[d], yd = gt[d] - g[d];
+            const double sd = sx[d], yd = gt[d] - g[d];
             ss = fma(sd, sd, ss);
             sy = fma(sd, yd, sy);
         }
@@ -818,12 +832,11 @@ extern "C" long long ppbo_predict_workspace_bytes(int N, int Q, int m, int P, in
     return (PT * N + PT * M + PT * M + 64) * 8;     // Kc, Ut, (Ud | Zs up to r <= M columns)
 }
 
-/* workspace of a mean-only call (Sigma_p == NULL): the tensor-pipe kernels never materialise the cross-covariance */
+/* workspace of a mean-only call (Sigma_p == NULL): the mat-vec mode of the SE / RQ / Matern / camphor kernels never materialises
+   the cross-covariance */
+static long long predict_mean_bytes(bool streams, int N, long long PT) { return (PT * (streams ? (N + 63) / 64 : N) + 64) * 8; }
 extern "C" long long ppbo_predict_mean_workspace_bytes(int kind, int N, int P, int batch) {
-    const long long PT = (long long)P * batch;
-    if (kind == PPBO_KERNEL_SE || kind == PPBO_KERNEL_RQ || kind == PPBO_KERNEL_MATERN32 || kind == PPBO_KERNEL_MATERN52)
-        return (PT * ((N + 63) / 64) + 64) * 8;
-    return (PT * N + 64) * 8;
+    return predict_mean_bytes(km_has_matvec(kind), N, (long long)P * batch);
 }
 
 extern "C" int ppbo_predict(int kind, const double* X, int N, int D, const double* lengthscales_h, double sigma_f,
@@ -833,8 +846,10 @@ extern "C" int ppbo_predict(int kind, const double* X, int N, int D, const doubl
     PPBO_REQUIRE(N == Q * (m + 1), "N must equal Q (m+1)");
     PPBO_REQUIRE(Sigma_p == nullptr || cap >= Q * m, "factor capacity below Q m");
     PPBO_REQUIRE(P >= 1 && batch >= 1, "empty grid");
+    // the mean alone streams through kernel_matvec unless tuning key 11 selects the materialising path (cross-covariance + GEMV)
+    const bool streams = g_tuning[11] == 0 && km_has_matvec(kind);
     PPBO_REQUIRE(workspace_bytes >= (Sigma_p ? ppbo_predict_workspace_bytes(N, Q, m, P, batch)
-                                             : ppbo_predict_mean_workspace_bytes(g_tuning[11] ? PPBO_KERNEL_CAMPHOR : kind, N, P, batch)),
+                                             : predict_mean_bytes(streams, N, (long long)P * batch)),
                  "workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
     const int PT = P * batch, M = Q * m;
@@ -967,16 +982,18 @@ extern "C" int ppbo_rff_value_grad(const double* W, const double* b, int F, int 
 }
 
 extern "C" int ppbo_rff_maximize(const double* W, const double* b, int F, int D, double sigma_f, const double* Omega, long long ldo,
-                                 int S, const double* X0, int R, int max_iter, double gtol, double* xbest, double* fbest,
-                                 double* work, void* stream) {
+                                 int S, const double* X0, int R, int max_iter, double gtol, int periodic_mask, double* xbest,
+                                 double* fbest, double* work, void* stream) {
     PPBO_REQUIRE(F >= 1 && D >= 1 && D <= RM_MAX_D, "D must be in [1, 32]");
     PPBO_REQUIRE(S >= 0 && R >= 1 && max_iter >= 0 && gtol >= 0 && work != nullptr, "arguments");
+    PPBO_REQUIRE(periodic_mask >= 0 && (D == 32 || (periodic_mask >> D) == 0), "periodic_mask names a coordinate beyond D");
     if (S == 0) return PPBO_OK;
     cudaStream_t st = (cudaStream_t)stream;
     const double amp = sqrt(2.0 * sigma_f * sigma_f / F);
     double* xall = work;                                  // [S][R][D]
     double* fall = work + (long long)S * R * D;          // [S][R]
-    PPBO_CL rff_maximize_kernel<<<S * R, RM_THREADS, 0, st>>>(W, b, F, D, amp, Omega, ldo, X0, R, max_iter, gtol, xall, fall, nullptr);
+    PPBO_CL rff_maximize_kernel<<<S * R, RM_THREADS, 0, st>>>(W, b, F, D, amp, Omega, ldo, X0, R, max_iter, gtol, (unsigned)periodic_mask, xall, fall,
+                                                                  nullptr);
     PPBO_CL rff_maximize_select_kernel<<<ceil_div(S, 128), 128, 0, st>>>(xall, fall, S, R, D, xbest, fbest);
     PPBO_LAUNCH_CHECK();
     return PPBO_OK;

@@ -199,7 +199,7 @@ __global__ void __launch_bounds__(KT_THREADS, 2) kernel_matrix_tiled_kernel(cons
 constexpr int KM_B = 128, KM_BN = 64, KM_THREADS = 512;        // 128 x 64 tiles, 16 warps of 32 x 16, two CTAs per SM (32 warps
                                                                   // hide the 13-deep Horner chains of the entry function)
 enum { KM_STORE = 0, KM_SYMMETRIC = 1, KM_MATVEC = 2 };
-__host__ __device__ inline int km_ldx(int D) { const int Dp = (D + 3) / 4 * 4; return (Dp % 8 == 4) ? Dp : Dp + 4; }
+__host__ __device__ constexpr int km_ldx(int D) { const int Dp = (D + 3) / 4 * 4; return (Dp % 8 == 4) ? Dp : Dp + 4; }
 
 // ---- streaming tensor-pipe kernel -------------------------------------------------------------------------------------------
 // profiles/r01_ncu_gram.txt: the one-tile-per-CTA kernel of round 1 executed ~109 instructions per matrix entry, 22 of them FP64:
@@ -289,6 +289,51 @@ __global__ void __launch_bounds__(128) km_prepare_kernel(const double* __restric
         const double v = (r < n && d < D) ? (X[(long long)r * D + d] - shift[d]) * p.inv_ls[d] : 0.0;
         row[d] = v;
         if (d < Dp) s = fma(v, v, s);
+    }
+    blk[(long long)TR * LDX + (r % TR)] = s;
+    blk[(long long)TR * LDX + TR + (r % TR)] = (alpha != nullptr && r < n) ? alpha[r] : 0.0;
+}
+
+// camphor_copper_kernel is an SE kernel in lifted coordinates: for each periodic d (0, 1, 3, 4, 5) u = (cos 2 pi x_d, sin 2 pi x_d) / l_0,
+// so that |u(x) - u(y)|^2 / 2 = 2 sin^2(pi (x_d - y_d)) / l_0^2, and x_2 / (l_2 + 0.05) for coordinate 2: D' = 11 coordinates, on
+// which the SE instantiation of the stream kernel computes the camphor mean (mat-vec mode only; Sigma and its appends keep the
+// difference form and their bits).  The shift s (the first point of X2) is subtracted in product form,
+//   cos a - cos b = -2 sin((a+b)/2) sin((a-b)/2),  sin a - sin b = 2 cos((a+b)/2) sin((a-b)/2),
+// so a lifted coordinate of a point close to s is exact to a few ulp relative instead of 2.2e-16 absolute.
+constexpr int KM_CAMPHOR_LIFTED_D = 11;
+__global__ void __launch_bounds__(128) km_prepare_camphor_kernel(const double* __restrict__ X, int n, int TR, KernelParams p,
+                                                                 const double* __restrict__ shift, const double* __restrict__ alpha,
+                                                                 double* __restrict__ out) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    constexpr int LDX = km_ldx(KM_CAMPHOR_LIFTED_D);
+    const int tiles = (n + TR - 1) / TR;
+    if (r >= tiles * TR) return;
+    double u[LDX];
+#pragma unroll
+    for (int j = 0; j < LDX; ++j) u[j] = 0.0;
+    if (r < n) {
+        int j = 0;
+#pragma unroll
+        for (int d = 0; d < 6; ++d) {
+            const double x = X[(long long)r * 6 + d], c = shift[d];
+            if (d == 2) {
+                u[j++] = (x - c) * p.inv_ls[2];
+            } else {
+                double sp, cp;
+                sincospi(x + c, &sp, &cp);
+                const double h = 2.0 * sinpi(x - c) * p.inv_ls[0];
+                u[j++] = -sp * h;
+                u[j++] = cp * h;
+            }
+        }
+    }
+    double* blk = out + (long long)(r / TR) * km_block_doubles(TR, LDX);
+    double* row = blk + (long long)(r % TR) * LDX;
+    double s = 0.0;
+#pragma unroll
+    for (int j = 0; j < LDX; ++j) {
+        row[j] = u[j];
+        s = fma(u[j], u[j], s);
     }
     blk[(long long)TR * LDX + (r % TR)] = s;
     blk[(long long)TR * LDX + TR + (r % TR)] = (alpha != nullptr && r < n) ? alpha[r] : 0.0;
@@ -477,10 +522,13 @@ static int km_column_groups(int tm, int tn) {
     return G < 1 ? 1 : G;
 }
 
+// p.kind == PPBO_KERNEL_CAMPHOR (mat-vec mode, KIND = SE): the points enter in the lifted operand form of km_prepare_camphor_kernel
 template <int KIND>
 static int launch_kernel_matrix_mma(const KernelParams& p, const double* X1, int n1, const double* X2, int n2, double* out,
                                     long long ld, int mode, const double* alpha, cudaStream_t st, int* groups_out = nullptr) {
-    const int LDX = km_ldx(p.D);
+    const bool lifted = p.kind == PPBO_KERNEL_CAMPHOR;
+    const int D = lifted ? KM_CAMPHOR_LIFTED_D : p.D;
+    const int LDX = km_ldx(D);
     const long long blk1 = km_block_doubles(KM_B, LDX), blk2 = km_block_doubles(KM_BN, LDX);
     const size_t smem = (size_t)(blk1 + 2 * blk2) * sizeof(double) + 32;
     static bool attr_done = false;
@@ -497,17 +545,22 @@ static int launch_kernel_matrix_mma(const KernelParams& p, const double* X1, int
     double* P1 = nullptr;
     PPBO_CUDA_CHECK(malloc_async((void**)reinterpret_cast<void**>(&P1), sizeof(double) * (tm * blk1 + tn * blk2), st));
     double* P2 = P1 + tm * blk1;
-    PPBO_CL km_prepare_kernel<<<ceil_div(tm * KM_B, 128), 128, 0, st>>>(X1, n1, KM_B, p, X2, nullptr, P1);
-    PPBO_CL km_prepare_kernel<<<ceil_div(tn * KM_BN, 128), 128, 0, st>>>(X2, n2, KM_BN, p, X2, alpha, P2);
+    if (lifted) {
+        PPBO_CL km_prepare_camphor_kernel<<<ceil_div(tm * KM_B, 128), 128, 0, st>>>(X1, n1, KM_B, p, X2, nullptr, P1);
+        PPBO_CL km_prepare_camphor_kernel<<<ceil_div(tn * KM_BN, 128), 128, 0, st>>>(X2, n2, KM_BN, p, X2, alpha, P2);
+    } else {
+        PPBO_CL km_prepare_kernel<<<ceil_div(tm * KM_B, 128), 128, 0, st>>>(X1, n1, KM_B, p, X2, nullptr, P1);
+        PPBO_CL km_prepare_kernel<<<ceil_div(tn * KM_BN, 128), 128, 0, st>>>(X2, n2, KM_BN, p, X2, alpha, P2);
+    }
     const int G = km_column_groups(tm, tn);
     if (groups_out) *groups_out = G;
     const dim3 grid(G, tm);
     if (mode == KM_SYMMETRIC)
-        PPBO_CL kernel_matrix_stream_kernel<KIND, KM_SYMMETRIC><<<grid, KM_THREADS, smem, st>>>(P1, n1, P2, n2, p.D, p.sf2, p.diag_scale, p.diag_add, out, ld, tn);
+        PPBO_CL kernel_matrix_stream_kernel<KIND, KM_SYMMETRIC><<<grid, KM_THREADS, smem, st>>>(P1, n1, P2, n2, D, p.sf2, p.diag_scale, p.diag_add, out, ld, tn);
     else if (mode == KM_MATVEC)
-        PPBO_CL kernel_matrix_stream_kernel<KIND, KM_MATVEC><<<grid, KM_THREADS, smem, st>>>(P1, n1, P2, n2, p.D, p.sf2, p.diag_scale, p.diag_add, out, G, tn);
+        PPBO_CL kernel_matrix_stream_kernel<KIND, KM_MATVEC><<<grid, KM_THREADS, smem, st>>>(P1, n1, P2, n2, D, p.sf2, p.diag_scale, p.diag_add, out, G, tn);
     else
-        PPBO_CL kernel_matrix_stream_kernel<KIND, KM_STORE><<<grid, KM_THREADS, smem, st>>>(P1, n1, P2, n2, p.D, p.sf2, p.diag_scale, p.diag_add, out, ld, tn);
+        PPBO_CL kernel_matrix_stream_kernel<KIND, KM_STORE><<<grid, KM_THREADS, smem, st>>>(P1, n1, P2, n2, D, p.sf2, p.diag_scale, p.diag_add, out, ld, tn);
     PPBO_LAUNCH_CHECK();
     PPBO_CUDA_CHECK(cudaFreeAsync(P1, st));
     return PPBO_OK;
@@ -516,6 +569,8 @@ static int launch_kernel_matrix_mma(const KernelParams& p, const double* X1, int
 static bool km_has_mma(int kind) {
     return kind == PPBO_KERNEL_SE || kind == PPBO_KERNEL_RQ || kind == PPBO_KERNEL_MATERN32 || kind == PPBO_KERNEL_MATERN52;
 }
+// kinds whose posterior mean streams through the mat-vec mode: the tensor-pipe kinds and camphor in its lifted SE form
+bool km_has_matvec(int kind) { return km_has_mma(kind) || kind == PPBO_KERNEL_CAMPHOR; }
 static int launch_kernel_matrix_mma_kind(const KernelParams& p, const double* X1, int n1, const double* X2, int n2, double* out,
                                          long long ld, int mode, const double* alpha, cudaStream_t st, int* groups_out = nullptr) {
     switch (p.kind) {
@@ -525,6 +580,9 @@ static int launch_kernel_matrix_mma_kind(const KernelParams& p, const double* X1
             return launch_kernel_matrix_mma<PPBO_KERNEL_MATERN32>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
         case PPBO_KERNEL_MATERN52:
             return launch_kernel_matrix_mma<PPBO_KERNEL_MATERN52>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
+        case PPBO_KERNEL_CAMPHOR:
+            PPBO_REQUIRE(mode == KM_MATVEC, "camphor runs on the tensor pipe in mat-vec mode only");
+            return launch_kernel_matrix_mma<PPBO_KERNEL_SE>(p, X1, n1, X2, n2, out, ld, mode, alpha, st, groups_out);
     }
     PPBO_REQUIRE(false, "kernel kind has no tensor-pipe version");
 }
@@ -618,10 +676,11 @@ int kernel_matrix_raw(int kind, const double* X1, int n1, const double* X2, int 
 }
 
 // mu[i] = sum_j k(X1_i, X2_j) alpha_j without materialising the n1 x n2 matrix (GPModel.mu_pred batched, src/gp_model.py:454-458);
-// partial: n1 * ceil(n2 / 64) doubles of scratch.  Returns 1 when done, 0 when the kernel kind has no tensor-pipe version.
+// partial: n1 * ceil(n2 / 64) doubles of scratch.  Returns 1 when done, 0 when the kernel kind has no mat-vec mode or tuning key 11
+// selects the materialising difference-form path.
 int kernel_matvec(int kind, const double* X1, int n1, const double* X2, int n2, int D, const double* ls_h, double sigma_f,
                   const double* alpha, double* mu, double* partial, cudaStream_t st) {
-    if (g_tuning[11] != 0 || !km_has_mma(kind)) return 0;
+    if (g_tuning[11] != 0 || !km_has_matvec(kind)) return 0;
     KernelParams p;
     int rc = fill_params(p, kind, D, ls_h, sigma_f);
     if (rc) return rc;

@@ -602,8 +602,10 @@ def rff_jacobian(W, b, x, sigma_f):
     return J
 
 
-def rff_maximize(W, b, sigma_f, Omega, X0, max_iter=500, gtol=1e-9):
-    """Omega [S,F], starts X0 [S,R,D] -> (xbest [S,D], fbest [S]): maximisers of the sampled functions phi(x)' Omega[s] on [0,1]^D"""
+def rff_maximize(W, b, sigma_f, Omega, X0, max_iter=500, gtol=1e-9, periodic_mask=0):
+    """Omega [S,F], starts X0 [S,R,D] -> (xbest [S,D], fbest [S]): maximisers of the sampled functions phi(x)' Omega[s] on [0,1]^D.
+    Coordinates whose bit is set in `periodic_mask` (spectral.periodic_mask of the basis' kernel) wrap modulo 1 instead of being
+    projected onto [0, 1]."""
     Fdim, D = W.shape
     S, R, _ = X0.shape
     dev = W.device
@@ -611,7 +613,8 @@ def rff_maximize(W, b, sigma_f, Omega, X0, max_iter=500, gtol=1e-9):
     fbest = torch.empty(S, dtype=F64, device=dev)
     work = _scratch("rff_maximize", S * R * (D + 1) * 8, dev)
     check(_lib.load().ppbo_rff_maximize(_p(W), _p(b), Fdim, D, float(sigma_f), _p(Omega), Omega.stride(0), S, _p(X0.contiguous()), R,
-                                        int(max_iter), float(gtol), _p(xbest), _p(fbest), _p(work), _stream()), "ppbo_rff_maximize")
+                                        int(max_iter), float(gtol), int(periodic_mask), _p(xbest), _p(fbest), _p(work), _stream()),
+          "ppbo_rff_maximize")
     return xbest, fbest
 
 

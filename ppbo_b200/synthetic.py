@@ -84,7 +84,7 @@ def make_problem(name, seed=0, Q=None, S=None, P=None, F=None, kernel=None):
     if cfg["F"]:
         W, b = draw_rff_basis(cfg["kernel"], cfg["F"], D, cfg["theta"][1], rng)       # src/random_fourier_sampler.py:42-43
         if W is None:
-            raise ValueError("random Fourier basis exists for the SE and Matern kernels only, not %s (use F=0)" % cfg["kernel"])
+            raise ValueError("random Fourier basis exists for the SE, Matern and camphor kernels only, not %s (use F=0)" % cfg["kernel"])
         prob["W"], prob["b"] = W, b
         prob["omega0"] = np.zeros(cfg["F"])
     return prob

@@ -7,7 +7,8 @@ evaluated on B projected xi-grids as one dense contraction Omega[S x F] . Phi_gr
 max / arg-max, optionally sharded over the GPUs of a box.
 
 Random numbers: every draw comes from the global legacy numpy RNG on the host, in the reference's order (generate_basis:
-W then b -- for the Matern kernels, an addition, W's normals, its chi-square draws, then b; update_omega_MAP: omega0; sample_omega: F normals through numpy's SVD-factor rule, which for the diagonal Laplace
+W then b -- for the Matern kernels, an addition, W's normals, its chi-square draws, then b; for the camphor kernel, an addition,
+the uniforms of its integer frequencies, the normals of its SE column, then b (ppbo_b200/spectral.py); update_omega_MAP: omega0; sample_omega: F normals through numpy's SVD-factor rule, which for the diagonal Laplace
 covariance is a permutation by decreasing variance).
 """
 import os
@@ -24,7 +25,7 @@ if _ROOT not in sys.path:
 from misc import pd_inverse, var2_normal_pdf  # noqa: E402,F401
 from ppbo_b200 import ops  # noqa: E402
 from ppbo_b200 import iteration as _it  # noqa: E402
-from ppbo_b200.spectral import draw_rff_basis  # noqa: E402
+from ppbo_b200.spectral import draw_rff_basis, periodic_mask  # noqa: E402
 
 
 def legacy_mvn_draw(mean, cov, n, rng=np.random):
@@ -66,7 +67,7 @@ class Hsampler:
 
     # ------------------------------------------------------------------ basis and feature maps (:38-58)
     def generate_basis(self):
-        # SE: the reference's draws; Matern: z, u, b (ppbo_b200/spectral.py); RQ / camphor: b only, no W
+        # SE: the reference's draws; Matern: z, u, b; camphor: u, z, b (ppbo_b200/spectral.py); RQ: b only, no W
         self.W, b = draw_rff_basis(self.kernel, self.nFeatures, self.D, self.theta[1], np.random)
         self.b = b[:, None]
         self._dev.clear()
@@ -75,7 +76,7 @@ class Hsampler:
         if name not in self._dev:
             if name == "W":
                 if self.W is None:
-                    raise ValueError("random Fourier basis exists for the SE kernel only (generate_basis)")
+                    raise ValueError("random Fourier basis exists for the SE, Matern and camphor kernels only (generate_basis)")
                 self._dev[name] = ops.to_dev(self.W)
             elif name == "b":
                 self._dev[name] = ops.to_dev(np.asarray(self.b).reshape(-1))
@@ -268,7 +269,8 @@ class Hsampler:
         the global RNG, sample by sample): a quarter like return_xstar -- a random GP local maximiser + 0.01 U(0,1) jitter; a quarter
         on the diagonal, (c, ..., c) + jitter with c a random coordinate of a local maximiser (what the reference's return_xstar
         actually starts from: its mu_star leaves xstars_local one-dimensional, src/gp_model.py:425-435, so indexing it yields a
-        scalar); the rest uniform in the box.  Every (sample, restart) is one CTA of ppbo_rff_maximize."""
+        scalar); the rest uniform in the box.  Every (sample, restart) is one CTA of ppbo_rff_maximize; the kernel's periodic
+        coordinates (spectral.periodic_mask) wrap around instead of being projected onto the box."""
         omegas = np.atleast_2d(np.asarray(omegas, dtype=np.float64))
         S, D = omegas.shape[0], self.D
         n_local = max(1, n_restarts // 4)
@@ -282,7 +284,8 @@ class Hsampler:
                     X0[s, r] = np.clip(loc.ravel()[np.random.randint(loc.size)] + 0.01 * np.random.uniform(0, 1, size=D), 0, 1)
                 else:
                     X0[s, r] = np.random.uniform(0, 1, size=D)
-        xb, fb = ops.rff_maximize(self._d("W"), self._d("b"), self.theta[2], ops.to_dev(omegas), ops.to_dev(X0), max_iter=max_iter, gtol=gtol)
+        xb, fb = ops.rff_maximize(self._d("W"), self._d("b"), self.theta[2], ops.to_dev(omegas), ops.to_dev(X0), max_iter=max_iter, gtol=gtol,
+                                  periodic_mask=periodic_mask(self.kernel))
         return xb.cpu().numpy(), fb.cpu().numpy()
 
     def sample_xstars(self, n, n_restarts=16):
