@@ -251,6 +251,16 @@ int ppbo_mu_star_de(int kind, const double* X, int N, int D, const double* lengt
  * arithmetic of ppbo_mu_pred_point (same bits).  GPModel.mu_pred (src/gp_model.py:454-458) for the windows above. */
 int ppbo_mu_pred_points(int kind, const double* X, int N, int D, const double* lengthscales_h, double sigma_f, const double* alpha,
                         const double* x_h, int B, double* mu_h, void* stream);
+/* Multi-start ascent of the posterior mean mu(x) = sum_i alpha_i k(x, X_i) over [0,1]^D (X [N][D], alpha [N], X0 [R][D]: DEVICE),
+ * one CTA per start: the projected gradient ascent of ppbo_rff_maximize with the value and the analytic gradient of mu fused in
+ * one pass over the design.  Stops when the projected gradient is below gtol * sigma_f^2 * sum_i |alpha_i| (relative to the bound
+ * on |mu|) or after max_iter steps; periodic_mask as for ppbo_rff_maximize (camphor: 0b111011).  Per start (DEVICE): the end point
+ * xout[R][D], mu there fout[R], the gradient there gout[R][D] and the steps taken iters[R]; xbest[D], fbest[1] = the best start
+ * (the lowest index on ties).  max_iter = 0: mu and its gradient at the starts (projected onto the box / wrapped).
+ * D <= 32; every kernel kind but PPBO_KERNEL_SQDIST. */
+int ppbo_mu_maximize(int kind, const double* X, int N, int D, const double* lengthscales_h, double sigma_f, const double* alpha,
+                     const double* X0, int R, int max_iter, double gtol, int periodic_mask, double* xout, double* fout, double* gout,
+                     int* iters, double* xbest, double* fbest, void* stream);
 /* fmax[b][s] = max_p ( mu[b][p] + sum_k Z[b][s][k] Fac[b][p][k] ), arg[b][s] = first arg-max.
  * Replaces the S calls of np.random.multivariate_normal + np.max in acquisition.EI / varmax
  * (src/acquisition.py:78-80, 175-177); Fac is the (P x P) sampling factor (row p = coefficients of point p). */

@@ -73,6 +73,7 @@ _SIGNATURES = {
     "ppbo_mu_star_de": (_I, [_I, _P, _I, _I, _PD, _D, _P, _PD, _PD, _I, _I, _D, _D, _D, _D, _D, _I, POINTER(c_uint), _PI, _PD, _PD,
                              _PI, _P]),
     "ppbo_mu_pred_points": (_I, [_I, _P, _I, _I, _PD, _D, _P, _PD, _I, _PD, _P]),
+    "ppbo_mu_maximize": (_I, [_I, _P, _I, _I, _PD, _D, _P, _P, _I, _I, _D, _I, _P, _P, _P, _P, _P, _P, _P]),
     "ppbo_mvn_rowmax": (_I, [_P, _L, _L, _P, _L, _L, _P, _L, _I, _I, _I, _I, _P, _P, _P]),
     "ppbo_acq_reduce": (_I, [_P, _I, _I, _D, _P, _P]),
     "ppbo_acq_reduce_dev": (_I, [_P, _I, _I, _P, _P, _P]),

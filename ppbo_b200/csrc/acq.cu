@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "../../include/ppbo_b200.h"
+#include "ascent.cuh"
 #include "common.cuh"
 #include "gemm_f64.cuh"
 #include "linalg.cuh"
@@ -255,13 +256,9 @@ __global__ void __launch_bounds__(256) rff_value_grad_kernel(const double* __res
 // ---- batched maximiser of sampled functions --------------------------------------------------------------------------------
 // Hsampler.return_xstar (src/random_fourier_sampler.py:143-178) maximises ONE sampled function g(x) = phi(x)' omega over [0,1]^D with
 // 5-30 sequential scipy L-BFGS-B restarts, every objective / gradient evaluation a Python call.  Here every (sample s, restart r)
-// pair is one CTA: projected gradient ascent with Barzilai-Borwein step lengths and Armijo backtracking on the box, the objective and
-// its gradient evaluated together (each thread owns F / 128 features; one block reduction of D + 1 numbers per evaluation).
-// Stationarity is measured by the projected gradient |clip(x + grad) - x|_inf.  A second kernel keeps the best restart per sample.
-// Coordinates with their bit set in `periodic` have period 1 (the sampled functions of a periodic kernel's basis are exactly
-// periodic there): a step reduces them modulo 1 instead of projecting them, the Armijo slope and the Barzilai-Borwein pair use the
-// unwrapped step, and their full gradient counts in the stationarity measure.  periodic = 0 is plain projected ascent on the box.
-constexpr int RM_THREADS = 128, RM_MAX_D = 32;
+// pair is one CTA running ascent_loop (ascent.cuh), the objective and its gradient evaluated together (each thread owns F / 128
+// features; one block reduction of D + 1 numbers per evaluation).  A second kernel keeps the best restart per sample.  The sampled
+// functions of a periodic kernel's basis are exactly periodic on its periodic coordinates, which `periodic` names.
 __global__ void __launch_bounds__(RM_THREADS) rff_maximize_kernel(const double* __restrict__ W, const double* __restrict__ b, int F, int D,
                                                                   double amp, const double* __restrict__ Omega, long long ldo,
                                                                   const double* __restrict__ X0, int R, int max_iter, double gtol,
@@ -310,55 +307,8 @@ __global__ void __launch_bounds__(RM_THREADS) rff_maximize_kernel(const double* 
         }
         __syncthreads();
     };
-    const bool wrap = (periodic >> (tid & 31)) & 1u;    // this thread's coordinate (tid < D) is periodic
-    if (tid < D) x[tid] = wrap ? x0[tid] - floor(x0[tid]) : fmin(fmax(x0[tid], 0.0), 1.0);
-    __syncthreads();
-    eval(x, g);
-    double f = fval_s;
-    double gmax = 0.0;
-    for (int d = 0; d < D; ++d) gmax = fmax(gmax, fabs(g[d]));
-    double t = 0.05 / fmax(gmax, 1e-12);               // first step: at most 5 % of the box
-    int it = 0;
-    for (; it < max_iter; ++it) {
-        double pg = 0.0;                                // projected-gradient stationarity measure
-        for (int d = 0; d < D; ++d) pg = fmax(pg, ((periodic >> d) & 1u) ? fabs(g[d]) : fabs(fmin(fmax(x[d] + g[d], 0.0), 1.0) - x[d]));
-        if (pg <= gtol) break;
-        double ft = f, slope = 0.0;
-        int tries = 0;
-        for (;; ++tries) {
-            __syncthreads();
-            if (tid < D) {
-                const double v = x[tid] + t * g[tid];
-                if (wrap) {
-                    xt[tid] = v - floor(v);
-                    sx[tid] = v - x[tid];
-                } else {
-                    xt[tid] = fmin(fmax(v, 0.0), 1.0);
-                    sx[tid] = xt[tid] - x[tid];
-                }
-            }
-            __syncthreads();
-            slope = 0.0;
-            for (int d = 0; d < D; ++d) slope = fma(g[d], sx[d], slope);
-            eval(xt, gt);
-            ft = fval_s;
-            if (ft >= f + 1e-4 * slope || tries >= 30) break;
-            t *= 0.5;
-        }
-        if (!(ft >= f)) break;                          // no ascent possible at this resolution
-        double ss = 0.0, sy = 0.0;
-        for (int d = 0; d < D; ++d) {
-            const double sd = sx[d], yd = gt[d] - g[d];
-            ss = fma(sd, sd, ss);
-            sy = fma(sd, yd, sy);
-        }
-        __syncthreads();
-        if (tid < D) { x[tid] = xt[tid]; g[tid] = gt[tid]; }
-        __syncthreads();
-        f = ft;
-        t = (sy < 0.0) ? fmin(fmax(-ss / sy, 1e-8), 1e4) : 2.0 * t;       // Barzilai-Borwein (concave along s), else expand
-        if (ss == 0.0) break;
-    }
+    double f;
+    const int it = ascent_loop(eval, D, x0, max_iter, gtol, periodic, x, g, xt, gt, sx, fval_s, f);
     if (tid < D) xout[(long long)blockIdx.x * D + tid] = x[tid];
     if (tid == 0) {
         fout[blockIdx.x] = f;
@@ -378,6 +328,12 @@ __global__ void rff_maximize_select_kernel(const double* __restrict__ xall, cons
     }
     fbest[s] = bf;
     for (int d = 0; d < D; ++d) xbest[(long long)s * D + d] = xall[((long long)s * R + br) * D + d];
+}
+// also the pick of the posterior-mean search (gram.cu, S = 1)
+int maximize_select(const double* xall, const double* fall, int S, int R, int D, double* xbest, double* fbest, cudaStream_t st) {
+    PPBO_CL rff_maximize_select_kernel<<<ceil_div(S, 128), 128, 0, st>>>(xall, fall, S, R, D, xbest, fbest);
+    PPBO_LAUNCH_CHECK();
+    return PPBO_OK;
 }
 
 // y[i] = sum_f Phi[f][i] omega[f]   (feature-major Phi: coalesced over i).  HBM-bound (8 F N bytes): the feature range is cut
@@ -994,9 +950,7 @@ extern "C" int ppbo_rff_maximize(const double* W, const double* b, int F, int D,
     double* fall = work + (long long)S * R * D;          // [S][R]
     PPBO_CL rff_maximize_kernel<<<S * R, RM_THREADS, 0, st>>>(W, b, F, D, amp, Omega, ldo, X0, R, max_iter, gtol, (unsigned)periodic_mask, xall, fall,
                                                                   nullptr);
-    PPBO_CL rff_maximize_select_kernel<<<ceil_div(S, 128), 128, 0, st>>>(xall, fall, S, R, D, xbest, fbest);
-    PPBO_LAUNCH_CHECK();
-    return PPBO_OK;
+    return maximize_select(xall, fall, S, R, D, xbest, fbest, st);
 }
 
 extern "C" long long ppbo_rff_workspace_bytes(int F, int Q, int m) {

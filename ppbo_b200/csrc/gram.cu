@@ -7,7 +7,10 @@
 // (2 D + exp) is within ~2x of the HBM floor (DESIGN.md K1).  Layout: CTA tile 64 rows x 128 columns, the two
 // point tiles staged in shared memory pre-scaled by 1/l_d; thread = 2 adjacent columns x 16 rows, 16-byte
 // coalesced stores.
+#include <cmath>
+
 #include "../../include/ppbo_b200.h"
+#include "ascent.cuh"
 #include "common.cuh"
 #include "gemm_f64.cuh"
 
@@ -733,6 +736,131 @@ __global__ void __launch_bounds__(1024) mu_pred_point_kernel(const double* __res
     if (threadIdx.x == 0) out[blockIdx.x] = s;
 }
 
+// ---- multi-start ascent of the posterior mean ---------------------------------------------------------------------------------
+// k(r2) and 2 dk/dr2 of the stationary kernels (r2 = |(x - y) / l|^2), both finite at r2 = 0
+constexpr double M_PI_D = 3.141592653589793;
+template <int KIND>
+__device__ __forceinline__ void kernel_value_slope(double r2, double sf2, double& k, double& dk2) {
+    if (KIND == PPBO_KERNEL_SE) {
+        k = sf2 * exp(-0.5 * r2);
+        dk2 = -k;
+    } else if (KIND == PPBO_KERNEL_RQ) {                                    // alpha = 2
+        const double it = 1.0 / (1.0 + 0.25 * r2);
+        k = sf2 * it * it;
+        dk2 = -k * it;
+    } else if (KIND == PPBO_KERNEL_MATERN32) {
+        const double a = sqrt(3.0 * r2), e = sf2 * exp(-a);
+        k = (1.0 + a) * e;
+        dk2 = -3.0 * e;
+    } else {                                                                // Matern-5/2
+        const double a = sqrt(5.0 * r2), e = sf2 * exp(-a);
+        k = (1.0 + a + 5.0 * r2 / 3.0) * e;
+        dk2 = -(5.0 / 3.0) * (1.0 + a) * e;
+    }
+}
+
+// One CTA per start runs ascent_loop (ascent.cuh) on mu(x) = sum_i alpha_i k(x, X_i).  An evaluation is one pass over the N design
+// rows: each thread takes rows tid, tid + 128, ... and keeps its D partial gradients in registers; the D + 1 sums are reduced in a
+// fixed order (warp shuffle tree, then the four warps in index order), so the result does not depend on timing.
+//   d mu / d x_d = sum_i alpha_i 2 k'(r2_i) (x_d - X_id) / l_d^2                  (k' = dk / dr2)
+//   camphor, k = sf2 exp(-E) (E of mu_pred_point_kernel):  d mu / d x_d = -sum_i alpha_i k_i dE_i/dx_d,  dE/dx_d = (2 pi / l0^2) sin(2 pi Delta_d) on the
+//   periodic coordinates and Delta_2 / (l2 + 0.05)^2 on coordinate 2
+// The stopping tolerance is gtol * sf2 * sum_i |alpha_i| (a bound on |mu|): relative to the problem's scale.
+template <int KIND>
+__global__ void __launch_bounds__(RM_THREADS) mu_ascent_kernel(const double* __restrict__ X, int N, KernelParams p,
+                                                               const double* __restrict__ alpha, const double* __restrict__ X0,
+                                                               int max_iter, double gtol, unsigned periodic, double* __restrict__ xout,
+                                                               double* __restrict__ fout, double* __restrict__ gout,
+                                                               int* __restrict__ iters) {
+    __shared__ double x[RM_MAX_D], g[RM_MAX_D], xt[RM_MAX_D], gt[RM_MAX_D], sx[RM_MAX_D];
+    __shared__ double red[RM_THREADS / 32][RM_MAX_D + 1];
+    __shared__ double red33[33];
+    __shared__ double fval_s;
+    const int D = p.D, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const double sf2 = p.sf2;
+    double scale = 0.0;
+    for (int i = tid; i < N; i += RM_THREADS) scale += fabs(alpha[i]);
+    scale = sf2 * block_sum(scale, red33);
+    // the factor every gradient sum is multiplied by once at the end
+    double gfac = 0.0;
+    if (tid < D) {
+        if (KIND == PPBO_KERNEL_CAMPHOR) gfac = tid == 2 ? p.inv_ls[2] * p.inv_ls[2] : 4.0 * M_PI_D * p.inv_ls[0] * p.inv_ls[0];
+        else gfac = p.inv_ls[tid];
+    }
+    auto eval = [&](const double* xv, double* gv) {
+        double val = 0.0, gl[RM_MAX_D];
+#pragma unroll
+        for (int d = 0; d < RM_MAX_D; ++d) gl[d] = 0.0;
+        for (int i = tid; i < N; i += RM_THREADS) {
+            const double* xi = X + (long long)i * D;
+            const double ai = alpha[i];
+            if (KIND == PPBO_KERNEL_CAMPHOR) {
+                const double il = p.inv_ls[0], il2 = il * il, ilz = p.inv_ls[2];
+                double dE[6], E = 0.0;          // dE[d] = dE/dx_d without its constant factor gfac
+#pragma unroll
+                for (int d = 0; d < 6; ++d) {
+                    const double dl = xv[d] - xi[d];
+                    if (d == 2) {
+                        E += 0.5 * dl * dl * ilz * ilz;
+                        dE[d] = dl;
+                    } else {
+                        double sn, cs;
+                        sincospi(dl, &sn, &cs);
+                        E += 2.0 * sn * sn * il2;
+                        dE[d] = sn * cs;                // sin(2 pi dl) / 2
+                    }
+                }
+                const double k = sf2 * exp(-E), c = -ai * k;
+                val = fma(k, ai, val);
+#pragma unroll
+                for (int d = 0; d < 6; ++d) gl[d] = fma(c, dE[d], gl[d]);
+            } else {
+                double r2 = 0.0;
+                for (int d = 0; d < D; ++d) {
+                    const double t = (xv[d] - xi[d]) * p.inv_ls[d];
+                    r2 = fma(t, t, r2);
+                }
+                double k, dk2;
+                kernel_value_slope<KIND>(r2, sf2, k, dk2);
+                val = fma(k, ai, val);
+                const double c = ai * dk2;
+#pragma unroll
+                for (int d = 0; d < RM_MAX_D; ++d)
+                    if (d < D) gl[d] = fma(c, (xv[d] - xi[d]) * p.inv_ls[d], gl[d]);
+            }
+        }
+        for (int o = 16; o > 0; o >>= 1) val += __shfl_xor_sync(0xffffffffu, val, o);
+        if (lane == 0) red[warp][RM_MAX_D] = val;
+#pragma unroll
+        for (int d = 0; d < RM_MAX_D; ++d) {
+            if (d < D) {
+                double v = gl[d];
+                for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+                if (lane == 0) red[warp][d] = v;
+            }
+        }
+        __syncthreads();
+        if (tid <= D) {
+            const int k = (tid == D) ? RM_MAX_D : tid;
+            const double v = (red[0][k] + red[1][k]) + (red[2][k] + red[3][k]);
+            if (tid == D) fval_s = v;
+            else gv[tid] = gfac * v;
+        }
+        __syncthreads();
+    };
+    const double* x0 = X0 + (long long)blockIdx.x * D;
+    double f;
+    const int it = ascent_loop(eval, D, x0, max_iter, gtol * scale, periodic, x, g, xt, gt, sx, fval_s, f);
+    if (tid < D) {
+        xout[(long long)blockIdx.x * D + tid] = x[tid];
+        gout[(long long)blockIdx.x * D + tid] = g[tid];
+    }
+    if (tid == 0) {
+        fout[blockIdx.x] = f;
+        iters[blockIdx.x] = it;
+    }
+}
+
 struct PinnedPoint {
     double* host = nullptr;
     double* dev = nullptr;
@@ -996,6 +1124,47 @@ extern "C" int ppbo_mu_pred_points(int kind, const double* X, int N, int D, cons
     PPBO_CUDA_CHECK(cudaStreamSynchronize(st));
     memcpy(mu_h, out_h, sizeof(double) * (size_t)B);
     return PPBO_OK;
+}
+
+namespace ppbo {
+int maximize_select(const double* xall, const double* fall, int S, int R, int D, double* xbest, double* fbest, cudaStream_t st);
+}
+
+extern "C" int ppbo_mu_maximize(int kind, const double* X, int N, int D, const double* lengthscales_h, double sigma_f,
+                                const double* alpha, const double* X0, int R, int max_iter, double gtol, int periodic_mask,
+                                double* xout, double* fout, double* gout, int* iters, double* xbest, double* fbest, void* stream) {
+    PPBO_REQUIRE(kind != PPBO_KERNEL_SQDIST, "the squared distance is not a covariance function");
+    PPBO_REQUIRE(D >= 1 && D <= RM_MAX_D, "D must be in [1, 32]");
+    KernelParams p;
+    int rc = fill_params(p, kind, D, lengthscales_h, sigma_f);
+    if (rc) return rc;
+    PPBO_REQUIRE(R >= 1 && N >= 0 && max_iter >= 0, "R >= 1, N >= 0 and max_iter >= 0");
+    PPBO_REQUIRE(gtol >= 0.0 && std::isfinite(gtol), "gtol must be finite and non-negative");
+    PPBO_REQUIRE(periodic_mask >= 0 && (D == 32 || (periodic_mask >> D) == 0), "periodic_mask names a coordinate beyond D");
+    PPBO_REQUIRE(X0 && xout && fout && gout && iters && xbest && fbest && (N == 0 || (X && alpha)), "arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned mask = (unsigned)periodic_mask;
+    switch (kind) {
+        case PPBO_KERNEL_SE:
+            PPBO_CL mu_ascent_kernel<PPBO_KERNEL_SE><<<R, RM_THREADS, 0, st>>>(X, N, p, alpha, X0, max_iter, gtol, mask, xout, fout, gout, iters);
+            break;
+        case PPBO_KERNEL_RQ:
+            PPBO_CL mu_ascent_kernel<PPBO_KERNEL_RQ><<<R, RM_THREADS, 0, st>>>(X, N, p, alpha, X0, max_iter, gtol, mask, xout, fout, gout, iters);
+            break;
+        case PPBO_KERNEL_CAMPHOR:
+            PPBO_CL mu_ascent_kernel<PPBO_KERNEL_CAMPHOR><<<R, RM_THREADS, 0, st>>>(X, N, p, alpha, X0, max_iter, gtol, mask, xout, fout, gout,
+                                                                                   iters);
+            break;
+        case PPBO_KERNEL_MATERN32:
+            PPBO_CL mu_ascent_kernel<PPBO_KERNEL_MATERN32><<<R, RM_THREADS, 0, st>>>(X, N, p, alpha, X0, max_iter, gtol, mask, xout, fout, gout,
+                                                                                    iters);
+            break;
+        default:
+            PPBO_CL mu_ascent_kernel<PPBO_KERNEL_MATERN52><<<R, RM_THREADS, 0, st>>>(X, N, p, alpha, X0, max_iter, gtol, mask, xout, fout, gout,
+                                                                                    iters);
+    }
+    PPBO_LAUNCH_CHECK();
+    return maximize_select(xout, fout, 1, R, D, xbest, fbest, st);
 }
 
 extern "C" int ppbo_kernel_se_grad(const double* X1, int n1, const double* X2, int n2, int D,

@@ -13,7 +13,7 @@ Host side is Python/torch for memory, streams and torch.distributed only; all ar
     fmax,arg [B][S_loc]   per-sample max / first arg-max over the grid (the S x P product never reaches HBM)
 
 Multi-GPU (SURVEY.md 8e): only the Monte-Carlo samples are partitioned.  Rank 0 fits and broadcasts the small fit
-products (omega_MAP, hess_diag, mu*: 8(2F+1) bytes); every rank draws its own slice of the counter-based normal stream,
+products (omega_MAP, hess_diag, mu*: 8(2F+1) bytes, 8(2F+D+1) with the x* of an incumbent); every rank draws its own slice of the counter-based normal stream,
 evaluates its S/R samples on all B grids and one all-reduce(sum) of the 3B partial sums follows.
 """
 import threading
@@ -23,6 +23,7 @@ import torch
 
 from . import ops
 from ._lib import PPBOError
+from .spectral import periodic_mask
 
 F64 = torch.float64
 SHRINKAGE = 1e-6          # GPModel.COVARIANCE_SHRINKAGE, src/gp_model.py:26
@@ -270,6 +271,35 @@ def mustar_over_candidates(g, candidates=None):
     if candidates is not None and candidates.shape[0] > 0:
         ops.vec_max(posterior_mean(g, candidates), out=out, accumulate=True)
     return out
+
+
+# Starts of the continuous mu* search: the MUSTAR_STARTS design rows with the largest f_MAP (DESIGN.md 7 item 16 and
+# profiles/r04_mustar_ascent_probe.txt for the choice), plus the best candidate of this iteration's lines and the previous x*.
+MUSTAR_STARTS = 128
+
+
+def mustar_starts(f_map, X, cand_mu=None, candidates=None, n_starts=MUSTAR_STARTS, prev=None):
+    """Starts [R, D] of mustar_ascent: the n_starts rows of X with the largest f_map (stable descending sort: the lowest index
+    first among equal values), the candidate with the largest posterior mean cand_mu (the first one on ties) and prev (the last
+    x*), in this order.  Device or host tensors alike."""
+    order = torch.sort(f_map, descending=True, stable=True).indices[:min(n_starts, X.shape[0])]
+    parts = [X[order]]
+    if candidates is not None and candidates.shape[0] > 0:
+        parts.append(candidates[torch.argmax(cand_mu)].view(1, -1))
+    if prev is not None:
+        parts.append(prev.reshape(1, -1).to(X.dtype))
+    return torch.cat(parts)
+
+
+def mustar_ascent(g, candidates=None, n_starts=MUSTAR_STARTS, prev=None, max_iter=ops.MU_MAXIMIZE_MAX_ITER, gtol=ops.MU_MAXIMIZE_GTOL):
+    """Continuous mu* and x* of the GP fit g on the device: multi-start ascent of the posterior mean (ops.mu_maximize) from
+    mustar_starts.  Returns (mu* [1], x* [D], the end point of every start [R, D]); mu* = mu(x*) as the ascent kernel evaluates
+    it (the reference's GPModel.mu_star returns mu_pred(xstar) as well).  No synchronisation."""
+    cand_mu = posterior_mean(g, candidates) if candidates is not None and candidates.shape[0] > 0 else None
+    X0 = mustar_starts(g.f_map, g.X, cand_mu, candidates, n_starts, prev)
+    xbest, fbest, xout, _, _, _ = ops.mu_maximize(g.kernel, g.X, g.lengthscales, g.theta[2], g.alpha, X0, max_iter=max_iter, gtol=gtol,
+                                                  periodic_mask=periodic_mask(g.kernel))
+    return fbest, xbest, xout
 
 
 class RFFFit:
@@ -625,6 +655,7 @@ class IterationState:
         self.rff = RFFState(W, b, theta, m, Q_cap, max_iter=fit_iters, tol=tol) if shard.rank == rff_rank else None
         self.Q, self.m = 0, m
         self.X_cap = torch.empty((Q_cap * (m + 1), D), dtype=F64, device=dev)       # the design, on every rank (mu* slices)
+        self.xstar = None            # x* of the last iteration run with an incumbent: one more start of the next search
 
     def design(self, Q):
         return self.X_cap[:Q * (self.m + 1)]
@@ -634,7 +665,7 @@ class _Iteration:
     """One call of run_iteration: its arguments and what follows from them, the two fits and the timer marks."""
 
     def __init__(self, d, kernel, theta, Q, m, S, shard, seed, fit_iters, tol, timers, state, shares, factor_at_mode, shard_mustar,
-                 weight_covariance):
+                 weight_covariance, incumbent):
         self.d, self.kernel, self.theta, self.Q, self.m, self.S, self.seed = d, kernel, theta, Q, m, S, seed
         self.shard, self.fit_iters, self.tol, self.timers, self.state = shard, fit_iters, tol, timers, state
         self.factor_at_mode, self.covariance, self.full = factor_at_mode, weight_covariance, weight_covariance == "full"
@@ -645,7 +676,10 @@ class _Iteration:
         self.warm = state is not None and state.Q > 0
         self.X = None if self.warm else d["X"]
         self.block = d["block"] if self.warm else None
-        self.shard_mustar = (shard.world >= 3 and not self.warm) if shard_mustar is None else shard_mustar
+        self.incumbent = incumbent
+        if shard_mustar is None:
+            shard_mustar = shard.world >= 3 and not self.warm and incumbent is None
+        self.shard_mustar = shard_mustar
         self.lo, self.hi = shard.sample_bounds(S, shares)
         self.i8 = self.hi > self.lo and sampling_engine(self.hi - self.lo, self.P, self.Fdim) == "i8"
 
@@ -664,6 +698,17 @@ class _Iteration:
             return self.state.gp.append(self.block, factor_at_mode=self.factor_at_mode)
         return self.state.gp.cold(self.X, f_init=self.d.get("f_init"), factor_at_mode=self.factor_at_mode)
 
+    def mustar(self, g):
+        """mu* of the GP fit g on the device: the discrete stand-in (1 double), or with an incumbent the continuous search, written
+        into the incumbent (mu*, x*: 1 + D doubles, which the reductions read as mu* through its first element)"""
+        if self.incumbent is None:
+            return mustar_over_candidates(g, self.cand)
+        prev = self.state.xstar if self.warm else None
+        mu, x, _ = mustar_ascent(g, self.cand, prev=prev)
+        self.incumbent[:1].copy_(mu)
+        self.incumbent[1:].copy_(x)
+        return self.incumbent
+
     def fit_rff(self):
         if self.state is None:
             r = rff_fit(self.X, self.W, self.b, self.theta, self.Q, self.m, omega0=self.d.get("omega0"), max_iter=self.fit_iters,
@@ -675,7 +720,7 @@ class _Iteration:
 
 
 def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, tol=1e-8, timers=None, state=None, shares=None,
-                  factor_at_mode=False, shard_mustar=None, weight_covariance="diag", batch=None):
+                  factor_at_mode=False, shard_mustar=None, weight_covariance="diag", batch=None, incumbent=None):
     """d: dict of device tensors (IterationInputs.to_device).  Returns (sums [B,3] device, gp, rff); with batch=q also the q query
     lines chosen by greedy joint expected improvement over the same draws (select_batch): (sums, gp, rff, (idx [q], qei [q])).
     Rank 0 fits; the others receive (omega_MAP, hess_diag, mu*) by broadcast while they compute the grid features.
@@ -694,13 +739,24 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     rank transforms its grid features once (rff_transform_grids).
     timers: a list that receives (name, CUDA event) marks between the stages of the schedule that ran.
     batch: q >= 1 keeps this rank's per-sample maxima and runs the greedy selection after the reduction on every rank (inside the
-    "acquisition" stage); without it nothing of the result changes."""
+    "acquisition" stage); without it nothing of the result changes.
+    incumbent: a float64 device tensor of D + 1 elements turns on the continuous mu* search (mustar_ascent, on rank 0 right after
+    the GP fit) in place of the discrete stand-in mustar_over_candidates: the EI sums and the batch selection use its mu*, and
+    every rank's incumbent receives (mu*, x*).  With a state, x* is kept there and starts the next appended iteration's search.
+    Not with shard_mustar=True.  incumbent=None changes nothing."""
     if weight_covariance not in WEIGHT_COVARIANCES:
         raise PPBOError("weight_covariance must be one of %s" % (WEIGHT_COVARIANCES,))
     if batch is not None and not 1 <= batch <= d["grids"].shape[0]:
         raise PPBOError("batch must be in [1, %d], not %r" % (d["grids"].shape[0], batch))
+    if incumbent is not None:
+        D = d["grids"].shape[2]
+        if not (isinstance(incumbent, torch.Tensor) and incumbent.dtype == F64 and incumbent.is_cuda and incumbent.is_contiguous()
+                and incumbent.numel() == D + 1):
+            raise PPBOError("incumbent must be a contiguous float64 device tensor of D + 1 = %d elements" % (D + 1))
+        if shard_mustar:
+            raise PPBOError("the continuous mu* search runs on rank 0: shard_mustar=True cannot be combined with an incumbent")
     it = _Iteration(d, kernel, theta, Q, m, S, shard or Shard(), seed, fit_iters, tol, timers, state, shares, factor_at_mode,
-                    shard_mustar, weight_covariance)
+                    shard_mustar, weight_covariance, incumbent)
     if state is not None:
         if it.warm:
             state.X_cap[state.Q * (m + 1):Q * (m + 1)].copy_(it.block)
@@ -720,6 +776,8 @@ def run_iteration(d, kernel, theta, Q, m, S, shard=None, seed=0, fit_iters=100, 
     it.mark("acquisition")
     if state is not None:
         state.Q = Q
+        if incumbent is not None:
+            state.xstar = incumbent[1:].clone()
     return (sums, gp, rff) if batch is None else (sums, gp, rff, picks)
 
 
@@ -762,7 +820,7 @@ def _one_gpu_overlapped(it, main, grid):
         torch.cuda.set_device(it.dev)
         with torch.cuda.stream(bg):
             g = it.fit_gp()
-            return g, mustar_over_candidates(g, it.cand)
+            return g, it.mustar(g)
     fut = _background_worker().submit(gp_chain)
     lib = ops._lib.load()
     try:
@@ -817,7 +875,7 @@ def _one_gpu_sequential(it, main, grid):
         with torch.cuda.stream(fg):
             gp = it.fit_gp()
             it.mark("gp_fit")
-            mustar = mustar_over_candidates(gp, it.cand)
+            mustar = it.mustar(gp)
             it.mark("mustar")
     finally:
         rff, prepared = fut.result()       # re-raises on this thread
@@ -837,7 +895,7 @@ def _several_ranks(it, main, grid):
     grid_stream, PhiT, normals, grid_tensors = grid
     shard, Fdim, full = it.shard, it.Fdim, it.full
     rff_rank = _weight_space_rank(shard.world)
-    pack = torch.empty(2 * Fdim + 1, dtype=F64, device=it.dev)
+    pack = torch.empty(2 * Fdim + (1 if it.incumbent is None else it.incumbent.numel()), dtype=F64, device=it.dev)
     pack_rff, mu_t = pack[:2 * Fdim], pack[2 * Fdim:]
     gp = rff = fmax = None
     Lbuf = ops.rff_hessian_factor_buffer(Fdim, it.dev) if full and shard.rank != rff_rank else None
@@ -875,8 +933,10 @@ def _several_ranks(it, main, grid):
         mu_t.copy_(_sharded_mustar(it, gp))
     else:
         if shard.rank == 0:
-            mu_t.copy_(mustar_over_candidates(gp, it.cand))
+            mu_t.copy_(it.mustar(gp))
         shard.broadcast(mu_t, src=0)
+        if it.incumbent is not None and shard.rank != 0:
+            it.incumbent.copy_(mu_t)
     it.mark("mustar")
     if shard.rank == 0 and it.hi > it.lo:
         _join(main, grid_stream, grid_tensors)

@@ -566,6 +566,29 @@ def mu_pred_points(kernel, X, lengthscales, sigma_f, alpha, points):
     return out
 
 
+MU_MAXIMIZE_MAX_ITER = 100      # step cap of the posterior-mean ascent (DESIGN.md 7 item 16)
+MU_MAXIMIZE_GTOL = 1e-10        # its stationarity tolerance, relative to sigma_f^2 sum |alpha| (the bound on |mu|)
+
+
+def mu_maximize(kernel, X, lengthscales, sigma_f, alpha, X0, max_iter=MU_MAXIMIZE_MAX_ITER, gtol=MU_MAXIMIZE_GTOL, periodic_mask=0):
+    """Multi-start ascent of mu(x) = k(x, X) alpha over [0,1]^D from the starts X0 [R, D] (ppbo_mu_maximize, one CTA per start).
+    Device tensors, no synchronisation: (xbest [D], fbest [1], xout [R, D], fout [R], gout [R, D], iters [R] int32) -- the best end
+    point (lowest start index on ties) and its mean, then per start the end point, the mean and its gradient there and the steps
+    taken.  max_iter = 0: the mean and its gradient at the starts.  periodic_mask: spectral.periodic_mask of the kernel."""
+    R, D = X0.shape
+    dev = X0.device
+    xout = torch.empty((R, D), dtype=F64, device=dev)
+    gout = torch.empty((R, D), dtype=F64, device=dev)
+    fout = torch.empty(R, dtype=F64, device=dev)
+    iters = torch.empty(R, dtype=torch.int32, device=dev)
+    xbest = torch.empty(D, dtype=F64, device=dev)
+    fbest = torch.empty(1, dtype=F64, device=dev)
+    check(_lib.load().ppbo_mu_maximize(_kind(kernel), _p(X), X.shape[0], D, _ls(lengthscales, D), float(sigma_f), _p(alpha),
+                                       _p(X0.contiguous()), R, int(max_iter), float(gtol), int(periodic_mask), _p(xout), _p(fout),
+                                       _p(gout), _p(iters), _p(xbest), _p(fbest), _stream()), "ppbo_mu_maximize")
+    return xbest, fbest, xout, fout, gout, iters
+
+
 def mvn_rowmax(Z, Fac, mu):
     """Z: [B,S,K], Fac: [B,P,K], mu: [B,P] -> fmax [B,S], arg [B,S] (int32)"""
     B, S, K = Z.shape
